@@ -7,7 +7,7 @@ advances every chain of every rank by one mcmc_step; `value` = chain-steps per s
 whole job.  Chains are independent (weak scaling: a fixed number of chains per GPU, no data-path
 collective; one NCCL all_gather of the per-chain log-posteriors at the end).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--chains C]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--chains C] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -21,6 +21,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree untouched (it may be read-only)
+DUMP_LIMIT_BYTES = 64 << 20
 
 M, Q, PU = 512, 8, 10
 D = Q + 1
@@ -558,6 +560,19 @@ def cfg4_full_bench(torch, model, rank, world):
             'checksum_finite': bool(torch.isfinite(msum).all().item())}
 
 
+def dump_outputs(dirname, arrays):
+    """arrays: name -> array with one row per chain.  Writes dirname/<name>.npy; when all rows together exceed
+    DUMP_LIMIT_BYTES, the same seeded sample of chains is kept in every array."""
+    os.makedirs(dirname, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    keep = np.arange(n)
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), np.ascontiguousarray(a[keep]))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -624,6 +639,9 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     dev_ms = e0.elapsed_time(e1)
     lp_last = out['lp'][-1].clone()
+    if args.dump_outputs and rank == 0:
+        # what the timed run returns for its last step: every chain's parameter vector and log-posterior (float64)
+        dump_outputs(args.dump_outputs, {'draws': out['draws'][-1].cpu().numpy(), 'lp': lp_last.cpu().numpy()})
     # same K steps again from the same state with per-kernel CUDA-event timers and evaluation counters
     # (instrumented pass: feeds `roofline` only)
     eng.theta.copy_(theta0); eng.sigwl.copy_(sig0)
@@ -754,6 +772,9 @@ def main():
     ap.add_argument('--cfg5-steps', type=int, default=2)
     ap.add_argument('--cfg4-full', action='store_true', help='run cfg4 at full size (1000 x 100 000) also with fewer than 8 GPUs')
     ap.add_argument('--no-extras', action='store_true', help='skip the rsvd / cfg5 / cfg4 / single-chain blocks')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the last step of the timed run as DIR/draws.npy (chains, P) and '
+                         'DIR/lp.npy (chains,), float64 (rank 0\'s chains; a seeded sample of chains above 64 MB in all)')
     if len(sys.argv) > 1 and sys.argv[1] == '--ref-worker':
         return _ref_worker_main(sys.argv[2:])
     args = ap.parse_args()

@@ -2,7 +2,6 @@
 import ctypes
 import os
 import re
-import sys
 import numpy as np
 import pytest
 
@@ -182,25 +181,10 @@ def test_normal_proposals_are_rejected_loudly():
     assert "if b.mcmc.stepType not in PROP_KIND:" in src and 'raise NotImplementedError' in src
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/src'), reason='reference tree not present (GPU box)')
-def test_reference_modules_resolve_against_the_shim():
-    """`import src.model` from the reference tree binds every sepia name it uses to this repository's mirror, and the
-    functions the reference calls exist with the argument names it passes (src/model.py:13-15,57-106,225-238;
+def test_sepia_mirror_takes_the_reference_call_arguments():
+    """The functions GladsGP's drivers call exist with the argument names they pass (src/model.py:57-106,225-238;
     assess_all_models.py:468-492)."""
-    import importlib
     import inspect
-    import subprocess
-    code = (
-        "import sys; sys.path.insert(0, %r); sys.path.insert(1, '/root/reference');"
-        "import src.model as rm; import sepia, inspect;"
-        "assert rm.SepiaModel.__module__.startswith('gladsgp_b200.sepia');"
-        "assert rm.SepiaData.__module__.startswith('gladsgp_b200.sepia');"
-        "assert callable(rm.SepiaParam);"
-        "print(sorted(n for n in dir(rm) if not n.startswith('_'))[:40])" % ROOT)
-    r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-3000:]
-    for name in ('init_model', 'fit_models', 'load_model'):
-        assert name in r.stdout
     from sepia.SepiaModel import SepiaModel
     from sepia.SepiaData import SepiaData
     from sepia.SepiaPredict import SepiaEmulatorPrediction
