@@ -22,7 +22,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from gladsgp_b200 import model as gmodel, synthetic          # noqa: E402
-from sepia.SepiaPredict import SepiaEmulatorPrediction        # noqa: E402
+from sepia.SepiaPredict import SepiaEmulatorPrediction, SepiaXvalEmulatorPrediction   # noqa: E402
 
 
 def make_config(workdir, m, q, n_x, n_t, tag, seed):
@@ -77,6 +77,13 @@ def main():
     rmse = np.sqrt(np.mean((ypred_mean - y_test) ** 2))
     cover = np.mean((y_test >= lq) & (y_test <= uq))
     print('test RMSE %.4f (field sd %.3f), 95%% interval coverage %.3f' % (rmse, y_test.std(), cover))
+    # leave-one-out cross-validation on the training set: no test ensemble needed, same samples (cached factors)
+    t0 = time.perf_counter()
+    xv = SepiaXvalEmulatorPrediction(samples=samples, model=model)
+    xv.w = xv.w.astype(np.float32)
+    err = xv.get_y_error_stats(y_test=y_train.astype(np.float32))
+    print('leave-one-out over %d simulations: %.2f s, RMSE %.4f, 95%% interval coverage %.3f'
+          % (args.m, time.perf_counter() - t0, float(np.sqrt(np.mean(err['rmse'] ** 2))), float(np.mean(err['frac_covered']))))
     print('artefacts in', os.path.join(workdir, 'data', 'models'), sorted(os.listdir(os.path.join(workdir, 'data', 'models'))))
     return rmse, cover
 

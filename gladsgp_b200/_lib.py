@@ -59,6 +59,8 @@ SIGNATURES = {
     'ggp_pred_cov_f64': (_I, [_P, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P]),
     'ggp_chol_draw_workspace_bytes': (_LL, [_I, _I]),
     'ggp_chol_draw_f64': (_I, [_P, _I, _I, _P, _P, _P, _P, _LL, _P]),
+    'ggp_xval_workspace_bytes': (_LL, [_I, _I, _I]),
+    'ggp_xval_solve_f64': (_I, [_P, _P, _I, _I, _P, _I, _P, _P, _P, _P, _LL, _P]),
     'ggp_reconstruct_f32': (_I, [_P, _P, _P, _I, _P, _I, _I, _I, _LL, _P, _P]),
     'ggp_reconstruct_stats_f32': (_I, [_P, _P, _P, _I, _P, _I, _P, _I, _I, _I, _LL, _D, _P, _P, _P, _P]),
     'ggp_errstats_workspace_bytes': (_LL, [_I, _LL]),

@@ -294,10 +294,12 @@ class Predictor:
         self.B = self.beta.shape[0]
         self.lamz = _f64(lamz, torch, dev).reshape(-1)
         self.s11 = _f64(s11_diag, torch, dev).reshape(-1)
-        out = loglik_batched(self.X, W, self.beta, self.lamz, diag_add, want_factor=True, want_u=True)
+        self.W = _f64(W, torch, dev).reshape(self.B, self.m)          # training weights: the means of cross-validation
+        out = loglik_batched(self.X, self.W, self.beta, self.lamz, diag_add, want_factor=True, want_u=True)
         self.factor, self.u, self.loglik, self.info = out['factor'], out['u'], out['loglik'], out['info']
         self.Mp = self.u.shape[1]
         self._ws = None
+        self._xws = None
 
     def predict(self, Xp, want_V=False):
         """Xp (n,d) -> mean (B,n), var (B,n)[, V (B,n,Mp)]."""
@@ -325,8 +327,92 @@ class Predictor:
                                    self.m, self.B, ptr(Sig), stream_ptr()), 'ggp_pred_cov_f64')
         return Sig
 
+    def xval_solve(self, idx, want_Z=False, b0=0, nb=None):
+        """ggp_xval_solve_f64 on blocks [b0, b0+nb): training rows idx (n,) -> alpha (nb,n) = z.u, p (nb,n) = z.z
+        [, Z (nb,n,Mp)] with z = L^-1 e_idx."""
+        torch, lib, dev = self.torch, self.lib, 'cuda'
+        nb = self.B - b0 if nb is None else nb
+        idx = torch.as_tensor(np.asarray(idx) if not torch.is_tensor(idx) else idx, device=dev).to(torch.int32).contiguous()
+        n = idx.numel()
+        need = lib.ggp_xval_workspace_bytes(self.m, n, nb)
+        if self._xws is None or self._xws.numel() < need:
+            self._xws = torch.empty(need, dtype=torch.uint8, device=dev)
+        alpha = torch.empty((nb, n), dtype=torch.float64, device=dev)
+        p = torch.empty((nb, n), dtype=torch.float64, device=dev)
+        Z = torch.empty((nb, n, self.Mp), dtype=torch.float64, device=dev) if want_Z else None
+        check(lib.ggp_xval_solve_f64(ptr(self.factor[b0:]), ptr(self.u[b0:]), self.m, nb, ptr(idx), n, ptr(alpha), ptr(p),
+                                     ptr(Z), ptr(self._xws), self._xws.numel(), stream_ptr()), 'ggp_xval_solve_f64')
+        return (alpha, p, Z) if want_Z else (alpha, p)
+
+    def xval(self, folds, sub_diag):
+        """Cross-validated moments of held-out training rows from the factors of the full S22 (SEPIA refits a sub-model
+        per fold; the Schur complement gives the same moments): for a fold F, with G = (S22^-1)_FF and a = (S22^-1 w)_F,
+          mu_F = w_F - G^-1 a,   Sig_F = G^-1 - sub_diag I.
+        folds: sequence of 1-D arrays of distinct rows in [0, m) (checked by the caller).  sub_diag (B,): the part of the
+        S22 nugget a prediction leaves out (1 / (LamSim lamWOs), or 0 with addResidVar).
+        Returns (mu, var, Sig): mu, var (B, N), N = sum |F|, fold-major and in the given order within a fold; Sig has one
+        entry per fold, (B, |F|, |F|) for |F| > 1 and None for a one-row fold (its variance is var)."""
+        torch, dev = self.torch, 'cuda'
+        folds = [np.asarray(f, dtype=np.int64).reshape(-1) for f in folds]
+        sizes = np.array([f.size for f in folds])
+        offs = np.concatenate([[0], np.cumsum(sizes)])
+        flat = np.concatenate(folds)
+        idx = np.unique(flat)                                  # ascending: each row skips the panels above it
+        pos = np.searchsorted(idx, flat)                       # flat[k] = idx[pos[k]]
+        N, n = flat.size, idx.size
+        sub = _f64(sub_diag, torch, dev).reshape(self.B, 1)
+        w = self.W[:, torch.as_tensor(idx, device=dev)]
+        mu = torch.empty((self.B, N), dtype=torch.float64, device=dev)
+        var = torch.empty((self.B, N), dtype=torch.float64, device=dev)
+        Sig = [None] * len(folds)
+        groups = {}                                            # fold size > 1 -> fold numbers
+        for k, s in enumerate(sizes):
+            if s > 1:
+                groups.setdefault(int(s), []).append(k)
+        if groups:
+            # the rows z_i go through the Gram products in chunks of blocks, at most XVAL_Z_BYTES of them at a time
+            per = n * self.Mp * 8
+            chunk = max(1, min(self.B, XVAL_Z_BYTES // per))
+            alpha = torch.empty((self.B, n), dtype=torch.float64, device=dev)
+            p = torch.empty((self.B, n), dtype=torch.float64, device=dev)
+            gsig = {s: torch.empty((self.B, len(ks), s, s), dtype=torch.float64, device=dev) for s, ks in groups.items()}
+            for b0 in range(0, self.B, chunk):
+                nb = min(chunk, self.B - b0)
+                a_c, p_c, Z = self.xval_solve(idx, want_Z=True, b0=b0, nb=nb)
+                alpha[b0:b0 + nb] = a_c
+                p[b0:b0 + nb] = p_c
+                for s, ks in groups.items():
+                    rows = torch.as_tensor(np.concatenate([pos[offs[k]:offs[k + 1]] for k in ks]), device=dev)
+                    cols = torch.as_tensor(np.concatenate([np.arange(offs[k], offs[k + 1]) for k in ks]), device=dev)
+                    Zg = Z[:, rows].reshape(nb, len(ks), s, self.Mp)
+                    L, info = torch.linalg.cholesky_ex(Zg @ Zg.transpose(-1, -2))
+                    if bool(info.any()):
+                        raise np.linalg.LinAlgError('cross-validation: a held-out block of S22^-1 is not positive definite')
+                    Gi = torch.cholesky_inverse(L)
+                    a = a_c[:, rows].reshape(nb, len(ks), s, 1)
+                    mu[b0:b0 + nb, cols] = (w[b0:b0 + nb, rows].reshape(nb, len(ks), s) -
+                                            (Gi @ a).squeeze(-1)).reshape(nb, -1)
+                    Sg = Gi - sub[b0:b0 + nb, :, None, None] * torch.eye(s, dtype=torch.float64, device=dev)
+                    gsig[s][b0:b0 + nb] = Sg
+                    var[b0:b0 + nb, cols] = torch.diagonal(Sg, dim1=-2, dim2=-1).reshape(nb, -1)
+                del Z
+            for s, ks in groups.items():
+                for t, k in enumerate(ks):
+                    Sig[k] = gsig[s][:, t]
+        else:
+            alpha, p = self.xval_solve(idx)
+        one = np.nonzero(sizes == 1)[0]
+        if one.size:
+            cols = torch.as_tensor(offs[one], device=dev)
+            r = torch.as_tensor(pos[offs[one]], device=dev)
+            pr = p[:, r]
+            mu[:, cols] = w[:, r] - alpha[:, r] / pr
+            var[:, cols] = 1.0 / pr - sub
+        return mu, var, Sig
+
 
 CHOL_DRAW_WS_BYTES = 1 << 30         # scratch factors of chol_draw: at most 1 GiB, more blocks go in several launches
+XVAL_Z_BYTES = 1 << 30               # rows z_i of Predictor.xval's multi-row folds: at most 1 GiB, more blocks in several launches
 
 
 def chol_draw(Sigma, z):

@@ -120,11 +120,10 @@ class SepiaEmulatorPrediction(SepiaPrediction):
         W = np.broadcast_to(self.model._w_pcs[None], (ns, pu, m)).reshape(ns * pu, m)
         return ns, beta, lamz, dadd, s11.reshape(-1), np.ascontiguousarray(W)
 
-    def _w_pred(self):
-        torch = _lib.require_cuda()
+    def _predictor(self):
+        """self._pred: the factored (sample, PC) blocks of these samples, from the model's cache or built and cached.
+        Returns the number of samples."""
         num = self.model.num
-        pu = num.pu
-        npred = self.xpredt.shape[0]
         key = _samples_key(self.samples, self.model, self.addResidVar)
         cached = getattr(self.model, '_pred_cache', None)
         if cached is not None and cached[0] == key:
@@ -135,8 +134,16 @@ class SepiaEmulatorPrediction(SepiaPrediction):
             bad = int((self._pred.info != 0).sum().item())
             if bad:
                 raise np.linalg.LinAlgError('%d of %d (sample, PC) covariance matrices are not positive definite' %
-                                            (bad, ns * pu))
+                                            (bad, ns * num.pu))
             self.model._pred_cache = (key, self._pred, ns)
+        return ns
+
+    def _w_pred(self):
+        torch = _lib.require_cuda()
+        num = self.model.num
+        pu = num.pu
+        npred = self.xpredt.shape[0]
+        ns = self._predictor()
         if self.joint is None and npred > MAX_JOINT:
             # SEPIA draws one joint realisation over all designs of a call; above MAX_JOINT designs the npred x npred blocks
             # (nsamp*pu of them) are not formed unless asked for: say so instead of changing the distribution silently
@@ -292,8 +299,117 @@ class SepiaEmulatorPrediction(SepiaPrediction):
         return out
 
 
-class SepiaXvalEmulatorPrediction:
-    """Imported, never called, by the reference (assess_all_models.py:31-32)."""
+def _check_folds(folds, m):
+    """leave_out_inds -> list of int64 index arrays; ValueError for anything SEPIA's per-fold refit could not run."""
+    try:
+        folds = list(folds)
+    except TypeError:
+        raise ValueError('leave_out_inds must be a list of arrays of training-row indices') from None
+    if not folds:
+        raise ValueError('leave_out_inds has no folds')
+    out = []
+    for k, f in enumerate(folds):
+        a = np.atleast_1d(np.asarray(f))
+        if a.ndim != 1 or a.size == 0:
+            raise ValueError('fold %d of leave_out_inds is empty or not one-dimensional' % k)
+        if a.dtype.kind not in 'iu':
+            raise ValueError('fold %d of leave_out_inds: indices must be integers, got %s' % (k, a.dtype))
+        if a.min() < 0 or a.max() >= m:
+            raise ValueError('fold %d of leave_out_inds: index out of range [0, %d)' % (k, m))
+        if np.unique(a).size != a.size:
+            raise ValueError('fold %d of leave_out_inds holds a row twice' % k)
+        if a.size == m:
+            raise ValueError('fold %d of leave_out_inds holds all %d training rows: nothing is left to predict from' % (k, m))
+        out.append(a.astype(np.int64))
+    return out
 
-    def __init__(self, *args, **kwargs):
-        raise NotImplementedError('cross-validation prediction is not exercised by GladsGP and is out of scope')
+
+class SepiaXvalEmulatorPrediction(SepiaEmulatorPrediction):
+    """Cross-validated emulator predictions (SEPIA's emulator check; imported by assess_all_models.py:31-32): the training
+    rows of every fold are predicted from the other simulations with the same posterior samples, so an emulator can be
+    validated without a test ensemble.
+
+    SEPIA builds a sub-model per fold and runs wPred at its held-out rows.  Here the factors of the full S22 -- shared with
+    SepiaEmulatorPrediction through the model's cache -- give the same moments in closed form (ops.Predictor.xval).
+    leave_out_inds: list of folds (arrays of training-row indices; folds may overlap); default leave-one-out
+    [[0], [1], ..., [m-1]].  Outputs:
+    * .w (nsamp, sum |F|, pu): fold-major, in the given order within a fold; get_y / get_y_stats / get_y_error_stats work
+      on it as on any prediction (y_test = the held-out rows of y_sim);
+    * .xpred / .t_pred: the held-out rows of x_trans / t_trans; .leave_out_inds: the folds (int64 arrays);
+    * storeMuSigma: .mu / .sigma are lists with one entry per fold, (nsamp, pu |F|) / (nsamp, pu |F|, pu |F|), PC-major.
+    Realisations consume one np.random.normal value per (fold, sample, PC, row), in that order, as SEPIA's per-fold wPred
+    calls do; a one-row fold is drawn as sqrt(var) z, a larger one through a Cholesky factor of each per-PC block."""
+
+    def __init__(self, samples=None, model=None, leave_out_inds=None, addResidVar=False, storeRlz=True,
+                 storeMuSigma=False):
+        if samples is None or model is None:
+            raise TypeError('samples and model are required')
+        m = model.num.m
+        self.leave_out_inds = _check_folds([[i] for i in range(m)] if leave_out_inds is None else leave_out_inds, m)
+        rows = np.concatenate(self.leave_out_inds)
+        sd = model.data.sim_data
+        self.model = model
+        self.samples = samples
+        self.addResidVar = addResidVar
+        self.storeRlz = storeRlz
+        self.storeMuSigma = storeMuSigma
+        self.joint = None
+        self.xpred = np.asarray(sd.x_trans)[rows]
+        self.t_pred = None if sd.t_trans is None else np.asarray(sd.t_trans)[rows]
+        self.xpredt = model.num.zt[rows]
+        self.w = None
+        self.mu = None
+        self.sigma = None
+        self._xval()
+
+    def _xval(self):
+        torch = _lib.require_cuda()
+        num = self.model.num
+        pu = num.pu
+        ns = self._predictor()
+        folds = self.leave_out_inds
+        sizes = np.array([f.size for f in folds])
+        offs = np.concatenate([[0], np.cumsum(sizes)])
+        N = int(offs[-1])
+        lamWOs = np.asarray(self.samples['lamWOs'], dtype=np.float64).reshape(-1, 1)
+        # SEPIA's predictive variance of a held-out row leaves out the 1/(LamSim lamWOs) part of S22's nugget unless
+        # addResidVar (then it is S22's own diagonal, as the s11 of SepiaEmulatorPrediction)
+        sub = np.zeros((ns, pu)) if self.addResidVar else 1.0 / (num.LamSim[None, :] * lamWOs)
+        mu, var, Sig = self._pred.xval(folds, sub.reshape(-1))
+        mu = mu.reshape(ns, pu, N)
+        var = var.reshape(ns, pu, N)
+        if self.storeMuSigma:
+            muh, varh = mu.cpu().numpy(), var.cpu().numpy()
+            self.mu, self.sigma = [], []
+            for k, s in enumerate(sizes):
+                sl = slice(offs[k], offs[k + 1])
+                self.mu.append(muh[:, :, sl].reshape(ns, pu * s))
+                blk = Sig[k].reshape(ns, pu, s, s).cpu().numpy() if s > 1 else varh[:, :, sl, None]
+                sig = np.zeros((ns, pu * s, pu * s))
+                for j in range(pu):
+                    sig[:, j * s:(j + 1) * s, j * s:(j + 1) * s] = blk[:, j]
+                self.sigma.append(sig)
+        if self.storeRlz:
+            # fold k takes the ns * pu * |F_k| values from ns * pu * offs[k] on, ordered (sample, PC, row)
+            zd = torch.as_tensor(np.random.normal(size=ns * pu * N), device='cuda')
+            B = ns * pu
+            dev = torch.empty((ns, pu, N), dtype=torch.float64, device='cuda')
+            one = offs[:-1][sizes == 1]
+            if one.size:
+                cols = torch.as_tensor(one, device='cuda')
+                zi = cols[None, :] * B + torch.arange(B, device='cuda')[:, None]
+                dev[:, :, cols] = torch.sqrt(torch.clamp(var[:, :, cols], min=0.0)) * zd[zi].reshape(ns, pu, -1)
+            for s in sorted(set(sizes[sizes > 1].tolist())):
+                ks = np.nonzero(sizes == s)[0]
+                S = torch.stack([Sig[k] for k in ks]).reshape(-1, s, s)
+                zz = torch.stack([zd[B * offs[k]:B * offs[k + 1]] for k in ks]).reshape(-1, s)
+                d_, info = ops.chol_draw(S, zz)
+                if bool(info.any()):                  # a block rejected by the Cholesky draw: eigen-factor, as wPred falls back
+                    lam, Qm = torch.linalg.eigh(S)
+                    d_ = torch.einsum('bij,bj->bi', Qm, torch.sqrt(torch.clamp(lam, min=0.0)) * zz)
+                d_ = d_.reshape(len(ks), ns, pu, s)
+                for t, k in enumerate(ks):
+                    dev[:, :, offs[k]:offs[k + 1]] = d_[t]
+            self.w = (mu + dev).permute(0, 2, 1).contiguous().cpu().numpy()      # (ns, N, pu)
+        else:
+            torch.cuda.current_stream().synchronize()

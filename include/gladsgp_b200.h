@@ -167,6 +167,18 @@ int ggp_pred_cov_f64(const double* Xp, int n, int d, const double* beta, const d
 long long ggp_chol_draw_workspace_bytes(int n, int B);
 int ggp_chol_draw_f64(const double* Sigma, int n, int B, const double* z, double* dev_out, int* info_out,
                       void* workspace, long long workspace_bytes, void* stream);
+/* Cross-validation from the factor of the FULL training covariance (SepiaXvalEmulatorPrediction; SEPIA refits a
+ * sub-model per fold instead).  For every block b and held-out training row i = idx[t]:
+ *   z = L[b]^-1 e_i   (zero above row i),   alpha_out[b][t] = z . u[b],   pdiag_out[b][t] = z . z = (S22^-1)_ii
+ * and, if Z_out is not null, Z_out[b][t][0:ggp_padded_m(m)] = z (zero padded).  A leave-one-out fold needs only these:
+ * mean = w_i - alpha / p, variance = 1 / p - 1 / (LamSim lamWOs); a larger fold F needs the rows z_i, i in F
+ * ((S22^-1)_FF = Z_F Z_F^T).  factor / u as for ggp_predict_f64; idx[nidx] int32 in any order (ascending order lets each
+ * row skip the panels above its index: about m^3/3 flop per block instead of m^3); an entry outside [0, m) gives a zero
+ * row.  Sums are in a fixed order (deterministic).  workspace: ggp_xval_workspace_bytes(m, nidx, B). */
+long long ggp_xval_workspace_bytes(int m, int nidx, int B);
+int ggp_xval_solve_f64(const double* factor, const double* u, int m, int B, const int* idx, int nidx,
+                       double* alpha_out, double* pdiag_out, double* Z_out, void* workspace, long long workspace_bytes,
+                       void* stream);
 
 /* SepiaEmulatorPrediction.get_y (SURVEY 8a row a8; assess_all_models.py:492), float32:
  *   y[r][c] = (sum_p w[r][p] K[p][c]) * sd[c] + mean[c],  r < R (= nsamp*npred), c < n_y.
