@@ -804,6 +804,7 @@ static int check_shard_args(const ggp_mcmc_args* args)
     GGP_ARG(args, "null args");
     const ggp_mcmc_args& a = *args;
     GGP_ARG(a.m > 0 && a.d > 0 && a.pu > 0 && a.n_chains > 0, "sizes must be positive");
+    GGP_ARG(a.d <= 64, "d must be <= 64");
     GGP_ARG(a.theta && a.sigwl && a.workspace && a.fixed && a.step, "null state / table pointer");
     GGP_ARG((long long)a.workspace_bytes >= workspace_bytes_impl(a.m, a.d, a.pu, a.n_chains, false), "workspace too small");
     if (a.replay) GGP_ARG(a.r_cand && a.r_logacorr && a.r_logu && a.r_valid, "replay tables missing");

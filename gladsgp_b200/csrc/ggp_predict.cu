@@ -441,13 +441,17 @@ static int launch_stats(const float* w, const float* K, const float* sd, int sd_
 {
     const dim3 grid((unsigned)((n_y + RC_COLS - 1) / RC_COLS), (unsigned)npred);
     const size_t smem = ((size_t)nsamp * PUMAX + nsamp) * sizeof(float);
-    if (i0 + 2 <= 4)
+    // the staged samples exceed the default 48 KB of dynamic shared memory from about 700 samples at pu = 16
+    if (i0 + 2 <= 4) {
+        GGP_CUDA(cudaFuncSetAttribute(reconstruct_stats_kernel<PUMAX, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         reconstruct_stats_kernel<PUMAX, 4><<<grid, 256, smem, st>>>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu,
                                                                    n_y, i0, frac, ymean, ylo, yhi, ytest, mape_floor, err_part);
-    else
+    } else {
+        GGP_CUDA(cudaFuncSetAttribute(reconstruct_stats_kernel<PUMAX, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         reconstruct_stats_kernel<PUMAX, 8><<<grid, 256, smem, st>>>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu,
                                                                    n_y, i0, frac, ymean, ylo, yhi, ytest, mape_floor, err_part);
-    return 0;
+    }
+    return GGP_OK;
 }
 
 template <int PUMAX>
@@ -622,10 +626,12 @@ int ggp_reconstruct_stats_f32(const float* w, const float* K, const float* sd, i
         return GGP_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    if (pu <= 4) launch_stats<4>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
-    else if (pu <= 8) launch_stats<8>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
-    else if (pu <= 12) launch_stats<12>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
-    else launch_stats<16>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
+    int rc;
+    if (pu <= 4) rc = launch_stats<4>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
+    else if (pu <= 8) rc = launch_stats<8>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
+    else if (pu <= 12) rc = launch_stats<12>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
+    else rc = launch_stats<16>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st);
+    if (rc != GGP_OK) return rc;
     GGP_CUDA(cudaGetLastError());
     return GGP_OK;
 }
@@ -661,10 +667,12 @@ int ggp_reconstruct_errstats_f32(const float* w, const float* K, const float* sd
     }
     cudaStream_t st = (cudaStream_t)stream;
     double* part = reinterpret_cast<double*>(workspace);
-    if (pu <= 4) launch_stats<4>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
-    else if (pu <= 8) launch_stats<8>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
-    else if (pu <= 12) launch_stats<12>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
-    else launch_stats<16>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
+    int rc;
+    if (pu <= 4) rc = launch_stats<4>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
+    else if (pu <= 8) rc = launch_stats<8>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
+    else if (pu <= 12) rc = launch_stats<12>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
+    else rc = launch_stats<16>(w, K, sd, sd_len, mean, mean_len, noise, nsamp, npred, pu, n_y, i0, frac, ymean_out, ylo_out, yhi_out, st, y_test, mape_floor, part);
+    if (rc != GGP_OK) return rc;
     GGP_CUDA(cudaGetLastError());
     const int ntile = (int)((n_y + RC_COLS - 1) / RC_COLS);
     errstats_reduce_kernel<<<(npred * 6 + 127) / 128, 128, 0, st>>>(part, ntile, npred, err_out);

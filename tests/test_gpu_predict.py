@@ -277,3 +277,138 @@ def test_scalar_gp_cfg2_size_10000_designs_against_oracle(cuda):
     for s in range(3):
         np.testing.assert_allclose(mean[s, idx], mu[s], rtol=PRED_RTOL, atol=PRED_RTOL * np.abs(mu).max())
         np.testing.assert_allclose(var[s, idx], np.diag(Sig[s]), rtol=PRED_RTOL, atol=1e-9)
+
+
+def _dense_posterior_device(X, Xp, W, beta, lamz, dadd):
+    """Dense FP64 references on the device from coordinate differences and torch's Cholesky: L of S22, Vr = L^-1 S21
+    (m, n) and u = L^-1 w."""
+    import torch
+    Xd, Xpd = torch.as_tensor(X, device='cuda'), torch.as_tensor(Xp, device='cuda')
+    bd = torch.as_tensor(beta, device='cuda')
+
+    def sq(A, Bm):
+        D = torch.zeros((A.shape[0], Bm.shape[0]), dtype=torch.float64, device='cuda')
+        for k in range(A.shape[1]):
+            D += bd[k] * (A[:, None, k] - Bm[None, :, k]) ** 2
+        return D
+    C = torch.exp(-sq(Xd, Xd)) / lamz
+    C.diagonal().fill_(1.0 / lamz + dadd)
+    L = torch.linalg.cholesky(C)
+    del C
+    Vr = torch.linalg.solve_triangular(L, torch.exp(-sq(Xd, Xpd)) / lamz, upper=False)
+    u = torch.linalg.solve_triangular(L, torch.as_tensor(W, device='cuda')[:, None], upper=False)[:, 0]
+    return L, Vr, u, torch.exp(-sq(Xpd, Xpd)) / lamz
+
+
+def _check_xval_rows(P, b, L, u, rows):
+    import torch
+    m = L.shape[0]
+    E = torch.zeros((m, len(rows)), dtype=torch.float64, device='cuda')
+    E[torch.as_tensor(rows, device='cuda'), torch.arange(len(rows), device='cuda')] = 1.0
+    Zr = torch.linalg.solve_triangular(L, E, upper=False).T                     # row i = L^-1 e_i
+    alpha, p, Z = P.xval_solve(rows, want_Z=True, b0=b, nb=1)
+    assert float((Z[0, :, :m] - Zr).abs().max()) <= PRED_RTOL * float(Zr.abs().max())
+    assert not Z[0, :, m:].any().item()
+    ra = Zr @ u
+    assert float((alpha[0] - ra).abs().max()) <= PRED_RTOL * float(ra.abs().max())
+    assert float(((p[0] - (Zr * Zr).sum(1)) / (Zr * Zr).sum(1)).abs().max()) <= PRED_RTOL
+
+
+def test_prediction_at_cfg5_size_against_dense_fp64(cuda):
+    """BASELINE.json configs[4] shape (m = 4096, d = 17), 2 blocks, 257 designs (a second 256-design task holding one
+    design): mean, var and V against the dense solve, pred_cov on the first 65 designs, xval_solve rows against L^-1 e_i."""
+    import torch
+    from gladsgp_b200 import ops
+    m, q, B, n = 4096, 16, 2, 257
+    X = np.concatenate([0.5 * np.ones((m, 1)), synthetic.design(m, q).astype(np.float64)], axis=1)
+    Xp = np.concatenate([0.5 * np.ones((n, 1)), synthetic.test_design(n, q).astype(np.float64)], axis=1)
+    rng = np.random.default_rng(17)
+    beta = np.exp(rng.uniform(np.log(0.05), np.log(1.0), size=(B, q + 1)))
+    lamz = np.array([1.1, 0.8]); lamws = np.array([900.0, 2500.0])
+    dadd = 3e-3 + 1.0 / lamws; s11 = 1.0 / lamz + 1.0 / lamws
+    W = rng.standard_normal((B, m))
+    P = ops.Predictor(X, W, beta, lamz, dadd, s11)
+    assert not P.info.any().item()
+    mean, var, V = P.predict(Xp, want_V=True)
+    Sg = P.pred_cov(Xp[:65], V[:, :65].contiguous())
+    for b in range(B):
+        L, Vr, u, S11 = _dense_posterior_device(X, Xp, W[b], beta[b], lamz[b], dadd[b])
+        mu = Vr.T @ u
+        vr = s11[b] - (Vr * Vr).sum(0)
+        assert float((mean[b] - mu).abs().max()) <= PRED_RTOL * float(mu.abs().max())
+        assert float(((var[b] - vr) / vr).abs().max()) <= PRED_RTOL
+        assert float((V[b, :, :m] - Vr.T).abs().max()) <= PRED_RTOL * float(Vr.abs().max())
+        assert not V[b, :, m:].any().item()
+        S11 = S11[:65, :65].clone()
+        S11.diagonal().fill_(s11[b])
+        Sig = S11 - Vr[:, :65].T @ Vr[:, :65]
+        assert float((Sg[b] - Sig).abs().max()) <= PRED_RTOL * float(Sig.abs().max())
+        _check_xval_rows(P, b, L, u, [0, 1, 31, 32, 2047, 4064, 4095])
+        del L, Vr
+        torch.cuda.empty_cache()
+
+
+def test_prediction_at_the_largest_supported_m(cuda):
+    """m = 8192 fills the kernels' 1024-entry slab-offset table (256 panels x 4 sub-slabs): moments and xval_solve rows
+    against torch FP64 on the device; m = 8193 is refused by both entry points."""
+    import torch
+    from gladsgp_b200 import ops, _lib
+    m, q, n = 8192, 8, 5
+    X = np.concatenate([0.5 * np.ones((m, 1)), synthetic.design(m, q).astype(np.float64)], axis=1)
+    Xp = np.concatenate([0.5 * np.ones((n, 1)), synthetic.test_design(n, q).astype(np.float64)], axis=1)
+    rng = np.random.default_rng(8192)
+    beta = np.exp(rng.uniform(np.log(0.1), np.log(2.0), size=(1, q + 1)))
+    lamz = np.array([1.3]); lamws = np.array([1500.0])
+    dadd = 2e-3 + 1.0 / lamws; s11 = 1.0 / lamz + 1.0 / lamws
+    W = rng.standard_normal((1, m))
+    P = ops.Predictor(X, W, beta, lamz, dadd, s11)
+    assert not P.info.any().item()
+    mean, var = P.predict(Xp)
+    L, Vr, u, _ = _dense_posterior_device(X, Xp, W[0], beta[0], lamz[0], dadd[0])
+    mu = Vr.T @ u
+    vr = s11[0] - (Vr * Vr).sum(0)
+    assert float((mean[0] - mu).abs().max()) <= PRED_RTOL * float(mu.abs().max())
+    assert float(((var[0] - vr) / vr).abs().max()) <= PRED_RTOL
+    _check_xval_rows(P, 0, L, u, [0, 4095, 8160, 8191])
+    del L, Vr, P
+    torch.cuda.empty_cache()
+    lib = _lib.load()
+    x = torch.zeros(64, dtype=torch.float64, device='cuda')
+    idx = torch.zeros(1, dtype=torch.int32, device='cuda')
+    p = _lib.ptr
+    rc = lib.ggp_predict_f64(p(x), 8193, 1, p(x), p(x), p(x), p(x), p(x), p(x), 1, 1, p(x), p(x), None, p(x), x.numel() * 8,
+                             _lib.stream_ptr())
+    assert rc == -1 and b'8192' in lib.ggp_last_error_string()
+    rc = lib.ggp_xval_solve_f64(p(x), p(x), 8193, 1, p(idx), 1, p(x), p(x), None, p(x), x.numel() * 8, _lib.stream_ptr())
+    assert rc == -1 and b'8192' in lib.ggp_last_error_string()
+
+
+@pytest.mark.parametrize('d', [17, 22])
+@pytest.mark.parametrize('n', [1, 31, 32, 33, 63, 64, 65, 129, 1024])
+def test_pred_cov_ragged_tile_edges(cuda, n, d):
+    """pred_cov walks the lower triangle in 64 x 32 tiles (row tile rt holds min(n_ct, 2 rt + 2) column tiles): every
+    entry, both triangles, against S11 - S21^T S22^-1 S21 at sizes around the tile edges and at 1024 designs."""
+    import scipy.linalg
+    from gladsgp_b200 import ops
+    m, B = 100, 2
+    rng = np.random.default_rng(n * 7 + d)
+    X = rng.uniform(0, 1, size=(m, d))
+    Xp = rng.uniform(0, 1, size=(n, d))
+    beta = rng.uniform(0.05, 1.0, size=(B, d)); lamz = rng.uniform(0.5, 2.0, size=B)
+    lamws = rng.uniform(300, 3000, size=B); dadd = 1.0 / lamws + 1e-3
+    P = ops.Predictor(X, rng.standard_normal((B, m)), beta, lamz, dadd, 1.0 / lamz + 1.0 / lamws)
+    _, _, V = P.predict(Xp, want_V=True)
+    Sg = P.pred_cov(Xp, V).cpu().numpy()
+    for b in range(B):
+        def cov(A, Bm):
+            D = np.zeros((A.shape[0], Bm.shape[0]))
+            for k in range(d):
+                D += beta[b, k] * (A[:, None, k] - Bm[None, :, k]) ** 2
+            return np.exp(-D) / lamz[b]
+        S22 = cov(X, X)
+        np.fill_diagonal(S22, 1.0 / lamz[b] + dadd[b])
+        S21 = cov(X, Xp)
+        S11 = cov(Xp, Xp)
+        np.fill_diagonal(S11, 1.0 / lamz[b] + 1.0 / lamws[b])
+        Sig = S11 - S21.T @ scipy.linalg.cho_solve(scipy.linalg.cho_factor(S22, lower=True), S21)
+        np.testing.assert_allclose(Sg[b], Sig, rtol=PRED_RTOL, atol=PRED_RTOL * np.abs(Sig).max())
