@@ -301,6 +301,38 @@ reconstruct_kernel(const float* __restrict__ w, const float* __restrict__ K, con
     }
 }
 
+// error statistics of one output against its test value (assess_all_models.py:523-538), accumulated in FP64 per thread:
+// e = { resid^2, |resid / y_test| and its count over y_test >= mape_floor, covered count, lower limit, upper limit }
+__device__ __forceinline__ void errstats_add(double (&e)[6], float vm, float vl, float vh, float yt, float mape_floor)
+{
+    const float res = vm - yt;
+    e[0] += (double)(res * res);
+    if (!(yt < mape_floor)) { e[1] += (double)fabsf(res / yt); e[2] += 1.0; }
+    if (yt >= vl && yt <= vh) e[3] += 1.0;
+    e[4] += (double)vl;
+    e[5] += (double)vh;
+}
+
+// fixed-order reduction of e over a 256-thread block -> row[0..5] (summed over the tiles in order by errstats_reduce_kernel)
+__device__ __forceinline__ void errstats_block_store(double (&e)[6], double* __restrict__ row)
+{
+    __shared__ double red[8][6];
+    const int tid = threadIdx.x;
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) e[k] += __shfl_xor_sync(0xffffffffu, e[k], o);
+    if ((tid & 31) == 0)
+#pragma unroll
+        for (int k = 0; k < 6; ++k) red[tid >> 5][k] = e[k];
+    __syncthreads();
+    if (tid < 6) {
+        double sacc = 0.0;
+        for (int wv = 0; wv < 8; ++wv) sacc += red[wv][tid];
+        row[tid] = sacc;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Fused predictive-distribution statistics (SURVEY 8f rank 1; the post-processing every caller does right
 // after get_y: assess_all_models.py:493-500, plot_test_error.py:81-87).  For design t and output c, over the
@@ -375,8 +407,7 @@ reconstruct_stats_kernel(const float* __restrict__ w, const float* __restrict__ 
         }
     }
     const float inv_n = 1.f / (float)nsamp;
-    // error statistics against the test field (assess_all_models.py:523-538), accumulated in FP64 per thread
-    double e_sq = 0.0, e_ape = 0.0, e_cnt = 0.0, e_cov = 0.0, e_lo = 0.0, e_hi = 0.0;
+    double e[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
         if (col[c] < n_y) {
@@ -391,35 +422,31 @@ reconstruct_stats_kernel(const float* __restrict__ w, const float* __restrict__ 
                 __stcs(ylo + o, vl);
                 __stcs(yhi + o, vh);
             }
-            if (ytest) {
-                const float yt = __ldcs(ytest + o);
-                const float res = vm - yt;
-                e_sq += (double)(res * res);
-                if (!(yt < mape_floor)) { e_ape += (double)fabsf(res / yt); e_cnt += 1.0; }
-                if (yt >= vl && yt <= vh) e_cov += 1.0;
-                e_lo += (double)vl;
-                e_hi += (double)vh;
-            }
+            if (ytest) errstats_add(e, vm, vl, vh, __ldcs(ytest + o), mape_floor);
         }
     }
-    if (ytest) {
-        // fixed-order block reduction -> one partial row per CTA (summed in order by errstats_reduce_kernel)
-        __shared__ double red[8][6];
-        double v[6] = {e_sq, e_ape, e_cnt, e_cov, e_lo, e_hi};
+    if (ytest) errstats_block_store(e, err_part + ((size_t)t * gridDim.x + blockIdx.x) * 6);
+}
+
+// The same error sums from stored mean / limit fields (of ggp_reconstruct_quantiles_f32): the tiles, the per-thread
+// columns and the reduction order are those of reconstruct_stats_kernel.  Block b = (design t, tile b % ntile).
+__global__ void __launch_bounds__(256)
+fields_errstats_kernel(const float* __restrict__ ymean, const float* __restrict__ ylo, const float* __restrict__ yhi,
+                       const float* __restrict__ ytest, long long n_y, int ntile, float mape_floor,
+                       double* __restrict__ err_part)
+{
+    const int t = blockIdx.x / ntile;
+    const long long c0 = (long long)(blockIdx.x - t * ntile) * RC_COLS;
+    double e[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
 #pragma unroll
-        for (int k = 0; k < 6; ++k)
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-        if ((tid & 31) == 0)
-#pragma unroll
-            for (int k = 0; k < 6; ++k) red[tid >> 5][k] = v[k];
-        __syncthreads();
-        if (tid < 6) {
-            double sacc = 0.0;
-            for (int wv = 0; wv < 8; ++wv) sacc += red[wv][tid];
-            err_part[((size_t)t * gridDim.x + blockIdx.x) * 6 + tid] = sacc;
+    for (int c = 0; c < 4; ++c) {
+        const long long col = c0 + threadIdx.x + 256 * c;
+        if (col < n_y) {
+            const size_t o = (size_t)t * n_y + col;
+            errstats_add(e, __ldcs(ymean + o), __ldcs(ylo + o), __ldcs(yhi + o), __ldcs(ytest + o), mape_floor);
         }
     }
+    errstats_block_store(e, err_part + (size_t)blockIdx.x * 6);
 }
 
 // err[t][k] = sum over the column tiles of err_part[t][tile][k], in tile order
@@ -609,6 +636,12 @@ int ggp_reconstruct_f32(const float* w, const float* K, const float* sd, int sd_
     return GGP_OK;
 }
 
+int ggp_reconstruct_stats_supported(int nsamp, int pu, double q)
+{
+    const int i0 = (int)floor(q * (nsamp - 1));
+    return !(pu > 16 || i0 + 2 > 8 || i0 + 2 > nsamp || (size_t)nsamp * 17 * sizeof(float) > 200 * 1024);
+}
+
 int ggp_reconstruct_stats_f32(const float* w, const float* K, const float* sd, int sd_len, const float* mean,
                               int mean_len, const float* noise, int nsamp, int npred, int pu, long long n_y, double q,
                               float* ymean_out, float* ylo_out, float* yhi_out, void* stream)
@@ -621,7 +654,7 @@ int ggp_reconstruct_stats_f32(const float* w, const float* K, const float* sd, i
     const double pos = q * (nsamp - 1);
     const int i0 = (int)floor(pos);
     const float frac = (float)(pos - i0);
-    if (pu > 16 || i0 + 2 > 8 || i0 + 2 > nsamp || (size_t)nsamp * 17 * sizeof(float) > 200 * 1024) {
+    if (!ggp_reconstruct_stats_supported(nsamp, pu, q)) {
         set_error("ggp_reconstruct_stats_f32: unsupported (pu=%d > 16 or quantile needs %d > 8 order statistics)", pu, i0 + 2);
         return GGP_ERR_UNSUPPORTED;
     }
@@ -656,7 +689,7 @@ int ggp_reconstruct_errstats_f32(const float* w, const float* K, const float* sd
     const double pos = q * (nsamp - 1);
     const int i0 = (int)floor(pos);
     const float frac = (float)(pos - i0);
-    if (pu > 16 || i0 + 2 > 8 || i0 + 2 > nsamp || (size_t)nsamp * 17 * sizeof(float) > 200 * 1024) {
+    if (!ggp_reconstruct_stats_supported(nsamp, pu, q)) {
         set_error("ggp_reconstruct_errstats_f32: unsupported (pu=%d > 16 or quantile needs %d > 8 order statistics)", pu, i0 + 2);
         return GGP_ERR_UNSUPPORTED;
     }
@@ -676,6 +709,28 @@ int ggp_reconstruct_errstats_f32(const float* w, const float* K, const float* sd
     GGP_CUDA(cudaGetLastError());
     const int ntile = (int)((n_y + RC_COLS - 1) / RC_COLS);
     errstats_reduce_kernel<<<(npred * 6 + 127) / 128, 128, 0, st>>>(part, ntile, npred, err_out);
+    GGP_CUDA(cudaGetLastError());
+    return GGP_OK;
+}
+
+int ggp_fields_errstats_f32(const float* ymean, const float* ylo, const float* yhi, const float* y_test, int npred,
+                            long long n_y, float mape_floor, double* err_out, void* workspace, long long workspace_bytes,
+                            void* stream)
+{
+    GGP_ARG(ymean && ylo && yhi && y_test && err_out && workspace, "null pointer");
+    GGP_ARG(npred > 0 && n_y > 0, "npred, n_y must be positive");
+    const long long ntile = (n_y + RC_COLS - 1) / RC_COLS;
+    GGP_ARG(6 * ntile * npred < (1LL << 31), "6 npred ceil(n_y / 1024) must be below 2^31");
+    const long long need = ggp_errstats_workspace_bytes(npred, n_y);
+    if (workspace_bytes < need) {
+        set_error("ggp_fields_errstats_f32: workspace too small (%lld < %lld)", workspace_bytes, need);
+        return GGP_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    double* part = reinterpret_cast<double*>(workspace);
+    fields_errstats_kernel<<<(unsigned)(ntile * npred), 256, 0, st>>>(ymean, ylo, yhi, y_test, n_y, (int)ntile, mape_floor, part);
+    GGP_CUDA(cudaGetLastError());
+    errstats_reduce_kernel<<<(npred * 6 + 127) / 128, 128, 0, st>>>(part, (int)ntile, npred, err_out);
     GGP_CUDA(cudaGetLastError());
     return GGP_OK;
 }

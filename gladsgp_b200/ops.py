@@ -631,3 +631,52 @@ def reconstruct_errstats(w, K, sd, mean, y_test, mape_floor, q=0.025, noise=None
                                            ptr(outs[2]), ptr(err), ptr(ws), need, stream_ptr()),
           'ggp_reconstruct_errstats_f32')
     return err.cpu().numpy(), (tuple(outs) if want_fields else None)
+
+
+def _f32(t):
+    torch = _lib.require_cuda()
+    if not torch.is_tensor(t):
+        t = torch.as_tensor(np.ascontiguousarray(np.asarray(t, dtype=np.float32)))
+    return t.to(device='cuda', dtype=torch.float32).contiguous()
+
+
+def stats_supported(nsamp, pu, q):
+    """True if reconstruct_stats / reconstruct_errstats serve (nsamp, pu, q) (ggp_reconstruct_stats_supported)."""
+    return bool(_lib.load().ggp_reconstruct_stats_supported(int(nsamp), int(pu), float(q)))
+
+
+def reconstruct_quantiles(w, K, sd, mean, quantiles, noise=None):
+    """Mean over samples of get_y and exact np.quantile fields of get_y + sd * noise[s, t] (float32, method 'linear'), any
+    sample count up to 16 384, 1-32 quantiles in [0, 1], pu <= 32.  w (nsamp,npred,pu) f32, noise (nsamp,npred) f32 or None
+    -> (ymean (npred, n_y), yq (nq, npred, n_y)) f32 on the device."""
+    torch = _lib.require_cuda()
+    lib = _lib.load()
+    w = _f32(w); K = _f32(K); sd = _f32(sd).reshape(-1); mean = _f32(mean).reshape(-1)
+    nsamp, npred, pu = w.shape
+    n_y = K.shape[1]
+    nz = None if noise is None else _f32(noise).reshape(nsamp, npred)
+    q = np.ascontiguousarray(np.atleast_1d(np.asarray(quantiles, dtype=np.float64)).reshape(-1))
+    ymean = torch.empty((npred, n_y), dtype=torch.float32, device='cuda')
+    yq = torch.empty((q.size, npred, n_y), dtype=torch.float32, device='cuda')
+    check(lib.ggp_reconstruct_quantiles_f32(ptr(w), ptr(K), ptr(sd), sd.numel(), ptr(mean), mean.numel(), ptr(nz), nsamp,
+                                            npred, pu, n_y, q.ctypes.data_as(C.POINTER(C.c_double)), q.size, ptr(ymean),
+                                            ptr(yq), stream_ptr()),
+          'ggp_reconstruct_quantiles_f32')
+    return ymean, yq
+
+
+def fields_errstats(ymean, ylo, yhi, y_test, mape_floor):
+    """The six per-design error sums of reconstruct_errstats from stored fields, each (npred, n_y) f32 (device tensors or
+    arrays) -> err (npred, 6) float64 host array (same columns, same summation order)."""
+    torch = _lib.require_cuda()
+    lib = _lib.load()
+    ymean = _f32(ymean)
+    npred, n_y = ymean.shape
+    ylo, yhi, yt = (_f32(a).reshape(npred, n_y) for a in (ylo, yhi, y_test))
+    need = lib.ggp_errstats_workspace_bytes(npred, n_y)
+    ws = torch.empty(need, dtype=torch.uint8, device='cuda')
+    err = torch.empty((npred, 6), dtype=torch.float64, device='cuda')
+    check(lib.ggp_fields_errstats_f32(ptr(ymean), ptr(ylo), ptr(yhi), ptr(yt), npred, n_y, float(mape_floor), ptr(err),
+                                      ptr(ws), need, stream_ptr()),
+          'ggp_fields_errstats_f32')
+    return err.cpu().numpy()

@@ -23,6 +23,7 @@ from .. import ops, _lib
 
 CHOL_DRAW_MAX_N = 16384   # ggp_chol_draw_f64 keeps an n-vector and n/8 offsets in shared memory
 MAX_JOINT = 1024      # above this many designs per call the joint covariance is not formed unless joint=True is passed
+FIELD_CHUNK_BYTES = 1 << 30   # get_y_error_stats beyond the fused kernels: mean / limit fields of at most ~1 GiB at a time
 
 
 def _samples_key(samples, model, add_resid):
@@ -251,17 +252,45 @@ class SepiaEmulatorPrediction(SepiaPrediction):
         sd = self.model.data.sim_data
         return sd.K_device() if np.asarray(sd.K).dtype == np.float32 else sd.K
 
+    def _stats_inputs(self):
+        """float32 w and the device basis, sd and mean of the statistics kernels; a scalar-output model is the unit 1 x 1
+        basis (get_y: y = w sd + mean)."""
+        torch = _lib.require_cuda()
+        sd = self.model.data.sim_data
+        K = torch.ones((1, 1), dtype=torch.float32, device='cuda') if self.model.data.scalar_out else self._basis_device()
+        sdd, mud = sd.stats_device()
+        return np.asarray(self.w, dtype=np.float32), K, sdd, mud
+
+    @staticmethod
+    def _fused_serves(w, quantile):
+        """The fused (q, 1-q) kernels run wherever they support the call -- every call that worked before keeps its bits --
+        and for an out-of-range quantile, which they reject; everything else goes through reconstruct_quantiles."""
+        ns, npred, pu = w.shape
+        return not (0.0 < quantile < 0.5) or (npred <= 65535 and ops.stats_supported(ns, pu, quantile))
+
+    def get_y_quantiles(self, quantiles=(0.025, 0.5, 0.975), noise=None, device=False):
+        """Extension (SURVEY 8f rank 1): mean over samples of get_y() and np.quantile(get_y() + sd_y * noise[s, t], q, axis=0)
+        for every q in `quantiles` (1-32 values in [0, 1]; NumPy's 'linear' method on the float32 values, bit for bit), for
+        up to 16 384 samples -- the per-sample fields are never materialised.  `noise` as in get_y_stats.
+        Returns dict(mean (npred, n_y), quantiles (nq, npred, n_y), q (nq,)), float32 fields."""
+        w, K, sdd, mud = self._stats_inputs()
+        q = np.atleast_1d(np.asarray(quantiles, dtype=np.float64)).reshape(-1)
+        m_, yq = ops.reconstruct_quantiles(w, K, sdd, mud, q, noise=noise)
+        if device:
+            return dict(mean=m_, quantiles=yq, q=q)
+        return dict(mean=m_.cpu().numpy(), quantiles=yq.cpu().numpy(), q=q)
+
     def get_y_stats(self, quantile=0.025, noise=None, device=False):
         """Extension (SURVEY 8f rank 1): mean over samples of get_y() and the (quantile, 1-quantile) quantiles of
         get_y() + sd_y * noise[s, t], fused on the GPU -- the per-sample fields are never materialised.  This is
         the post-processing of assess_all_models.py:493-500 / plot_test_error.py:81-87 (`noise[s, t]` there is
         np.random.normal(scale=1/sqrt(lamWOs[s]))).  Returns dict(mean, lq, uq), each (npred, n_y) float32."""
-        sd = self.model.data.sim_data
-        if self.model.data.scalar_out:
-            raise NotImplementedError('get_y_stats is for multivariate (K basis) models')
-        sdd, mud = sd.stats_device()
-        m_, lo, hi = ops.reconstruct_stats(np.asarray(self.w, dtype=np.float32), self._basis_device(), sdd, mud,
-                                           q=quantile, noise=noise)
+        w, K, sdd, mud = self._stats_inputs()
+        if self._fused_serves(w, quantile):
+            m_, lo, hi = ops.reconstruct_stats(w, K, sdd, mud, q=quantile, noise=noise)
+        else:
+            m_, yq = ops.reconstruct_quantiles(w, K, sdd, mud, (quantile, 1.0 - quantile), noise=noise)
+            lo, hi = yq[0], yq[1]
         if device:
             return dict(mean=m_, lq=lo, uq=hi)
         return dict(mean=m_.cpu().numpy(), lq=lo.cpu().numpy(), uq=hi.cpu().numpy())
@@ -273,9 +302,6 @@ class SepiaEmulatorPrediction(SepiaPrediction):
         y_test (npred, n_y) in native units; `noise` as in get_y_stats; `mape_floor`: outputs below it are left out of the
         MAPE (the reference uses the 10 % quantile of its whole test matrix; default: that quantile of `y_test`).
         Returns dict(rmse, mape, lq, uq, frac_covered (each (npred,)), integrated_ci, mape_floor[, mean, lq_field, uq_field])."""
-        sd = self.model.data.sim_data
-        if self.model.data.scalar_out:
-            raise NotImplementedError('get_y_error_stats is for multivariate (K basis) models')
         torch = _lib.require_cuda()
         yt = y_test if torch.is_tensor(y_test) else torch.as_tensor(np.ascontiguousarray(np.asarray(y_test, dtype=np.float32)))
         yt = yt.to(device='cuda', dtype=torch.float32)
@@ -287,9 +313,12 @@ class SepiaEmulatorPrediction(SepiaPrediction):
             lo_v = torch.kthvalue(flat, k0 + 1).values
             hi_v = torch.kthvalue(flat, min(k0 + 2, flat.numel())).values
             mape_floor = float(lo_v + (hi_v - lo_v) * (pos - k0))
-        sdd, mud = sd.stats_device()
-        err, fl = ops.reconstruct_errstats(np.asarray(self.w, dtype=np.float32), self._basis_device(), sdd, mud, yt,
-                                           mape_floor, q=quantile, noise=noise, want_fields=fields)
+        w, K, sdd, mud = self._stats_inputs()
+        yt = yt.reshape(w.shape[1], K.shape[1])
+        if self._fused_serves(w, quantile):
+            err, fl = ops.reconstruct_errstats(w, K, sdd, mud, yt, mape_floor, q=quantile, noise=noise, want_fields=fields)
+        else:
+            err, fl = self._fields_error_stats(w, K, sdd, mud, yt, mape_floor, quantile, noise, fields)
         n_y = yt.shape[1]
         out = dict(rmse=np.sqrt(err[:, 0] / n_y), mape=err[:, 1] / err[:, 2], lq=err[:, 4] / n_y, uq=err[:, 5] / n_y,
                    frac_covered=err[:, 3] / n_y, integrated_ci=float(np.mean((err[:, 5] - err[:, 4]) / n_y)),
@@ -297,6 +326,25 @@ class SepiaEmulatorPrediction(SepiaPrediction):
         if fields:
             out.update(mean=fl[0], lq_field=fl[1], uq_field=fl[2])
         return out
+
+    @staticmethod
+    def _fields_error_stats(w, K, sdd, mud, yt, mape_floor, quantile, noise, fields):
+        """get_y_error_stats where the fused kernels do not serve the call: mean and (q, 1-q) quantile fields of a chunk of
+        designs (about FIELD_CHUNK_BYTES of them; all at once when the fields are returned), then their error sums."""
+        ns, npred, _ = w.shape
+        n_y = K.shape[1]
+        nz = None if noise is None else ops._f32(noise).reshape(ns, npred)
+        chunk = npred if fields else max(1, min(npred, FIELD_CHUNK_BYTES // (3 * 4 * n_y)))
+        err, fl = [], []
+        for t0 in range(0, npred, chunk):
+            t1 = min(npred, t0 + chunk)
+            m_, yq = ops.reconstruct_quantiles(w[:, t0:t1], K, sdd, mud, (quantile, 1.0 - quantile),
+                                               noise=None if nz is None else nz[:, t0:t1])
+            err.append(ops.fields_errstats(m_, yq[0], yq[1], yt[t0:t1], mape_floor))
+            if fields:
+                fl = (m_, yq[0], yq[1])
+            del m_, yq
+        return np.concatenate(err, axis=0), (fl if fields else None)
 
 
 def _check_folds(folds, m):

@@ -195,6 +195,23 @@ int ggp_reconstruct_f32(const float* w, const float* K, const float* sd, int sd_
 int ggp_reconstruct_stats_f32(const float* w, const float* K, const float* sd, int sd_len, const float* mean,
                               int mean_len, const float* noise, int nsamp, int npred, int pu, long long n_y, double q,
                               float* ymean_out, float* ylo_out, float* yhi_out, void* stream);
+/* 1 if ggp_reconstruct_stats_f32 / ggp_reconstruct_errstats_f32 serve (nsamp, pu, q) -- the order statistic
+ * floor(q (nsamp-1)) + 2 <= 8 and <= nsamp, pu <= 16, the staged samples within 200 KB -- else 0 (they return
+ * GGP_ERR_UNSUPPORTED).  Argument errors are not judged here. */
+int ggp_reconstruct_stats_supported(int nsamp, int pu, double q);
+
+/* Exact quantile fields over the posterior samples, for any sample count up to 16 384, up to 32 quantiles and pu <= 32
+ * (csrc/ggp_quantile.cu).  y_s, z_s as above (noise nullable; without it z_s = y_s), formed with the same float32
+ * operations as ggp_reconstruct_f32 and `y + sd * noise`:
+ *   ymean_out[t][c] = mean_s y_s (FP64 sum in a fixed order, rounded once; nullable),
+ *   yq_out[k][t][c] = np.quantile(z, q_host[k]) of the float32 z_s (NumPy 2.x, method 'linear', float32 arithmetic:
+ *                     pos = float32(nsamp-1) float32(q), i = floor(pos), t = pos - i, j = min(i+1, nsamp-1),
+ *                     d = x_j - x_i, x_j - d (1-t) if t >= 0.5 else x_i + d t); a NaN sample makes every quantile NaN.
+ * q_host[nq] is a HOST array of values in [0, 1], 1 <= nq <= 32.  Any npred.  GGP_ERR_UNSUPPORTED for nsamp > 16384 or
+ * pu > 32. */
+int ggp_reconstruct_quantiles_f32(const float* w, const float* K, const float* sd, int sd_len, const float* mean,
+                                  int mean_len, const float* noise, int nsamp, int npred, int pu, long long n_y,
+                                  const double* q_host, int nq, float* ymean_out, float* yq_out, void* stream);
 
 /* Same pass with the test-error statistics of assess_all_models.py:523-538 fused in: for every test design t
  *   err[t] = { sum (ymean - y_test)^2,  sum |ymean - y_test| / y_test over y_test >= mape_floor,  count(y_test >= mape_floor),
@@ -207,6 +224,12 @@ int ggp_reconstruct_errstats_f32(const float* w, const float* K, const float* sd
                                  int mean_len, const float* noise, int nsamp, int npred, int pu, long long n_y, double q,
                                  const float* y_test, float mape_floor, float* ymean_out, float* ylo_out, float* yhi_out,
                                  double* err_out, void* workspace, long long workspace_bytes, void* stream);
+/* The same six sums from stored fields (e.g. those of ggp_reconstruct_quantiles_f32): ymean, ylo, yhi, y_test [npred][n_y].
+ * The column tiles and the summation order are those of ggp_reconstruct_errstats_f32, so fed that function's own fields
+ * it returns its err bit for bit.  workspace: ggp_errstats_workspace_bytes(npred, n_y). */
+int ggp_fields_errstats_f32(const float* ymean, const float* ylo, const float* yhi, const float* y_test, int npred,
+                            long long n_y, float mape_floor, double* err_out, void* workspace, long long workspace_bytes,
+                            void* stream);
 
 /* ---- Sobol' / Saltelli sensitivity statistics (SURVEY 8f rank 3) --------------------------------
  * src/utils.py:80-92 (point estimates), :97-118 and :213-243 (the statistics scipy.stats.bootstrap evaluates 9999 times and
