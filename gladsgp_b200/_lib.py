@@ -68,6 +68,8 @@ SIGNATURES = {
     'ggp_reconstruct_stats_supported': (_I, [_I, _I, _D]),
     'ggp_reconstruct_quantiles_f32': (_I, [_P, _P, _P, _I, _P, _I, _P, _I, _I, _I, _LL, C.POINTER(_D), _I, _P, _P, _P]),
     'ggp_fields_errstats_f32': (_I, [_P, _P, _P, _P, _I, _LL, _F, _P, _P, _LL, _P]),
+    'ggp_chain_diag_workspace_bytes': (_LL, [_I, _I, _I]),
+    'ggp_chain_diag_f64': (_I, [_P, _I, _I, _I, _LL, _LL, _LL, _P, _P, _P, _P, _LL, _P]),
     'ggp_sobol_stats_f64': (_I, [_P, _P, _P, _I, _I, _I, _P, _LL, _I, _I, _I, _P, _P, _P]),
     'ggp_rsvd_workspace_bytes': (_LL, [_I]),
     'ggp_rsvd_sketch_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P, _LL, _P]),

@@ -108,3 +108,18 @@ class ModelBatch:
                     b.val = v0
                 o += k
             mm.params.lp.val = float(lps[-1, i]) if update_vals else saved_lp[i]
+
+    def mcmc_diagnostics(self, nburn=0):
+        """SepiaModel.mcmc_diagnostics of every model's recorded chain, in one device call: element (model i, parameter p)
+        is one chain of the (n, models x (P + 1)) array of draws and logPost.  Returns one dict per model, equal bit for
+        bit to that model's own mcmc_diagnostics()."""
+        from . import diagnostics
+        chains = [mm._recorded_chain() for mm in self.models]
+        n = chains[0][0].shape[0]
+        if n == 0 or any(d.shape[0] != n for d, _ in chains):
+            raise ValueError('every model needs the same, non-zero number of recorded draws')
+        x = np.stack([np.concatenate([d, l[:, None]], axis=1) for d, l in chains], axis=1)   # (n, models, P + 1)
+        res = diagnostics.chain_diagnostics(x.reshape(n, 1, -1), nburn=nburn)
+        Q = self.P + 1
+        return [diagnostics.by_block(mm._blocks()[0], {k: v[i * Q:(i + 1) * Q] for k, v in res.items()})
+                for i, mm in enumerate(self.models)]

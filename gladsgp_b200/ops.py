@@ -680,3 +680,33 @@ def fields_errstats(ymean, ylo, yhi, y_test, mape_floor):
                                       ptr(ws), need, stream_ptr()),
           'ggp_fields_errstats_f32')
     return err.cpu().numpy()
+
+
+CHAIN_DIAG_WS_BYTES = 8 << 30        # workspace of chain_diagnostics: at most 8 GiB, more elements go in several launches
+
+
+def chain_diagnostics(x):
+    """Rank-normalized split R-hat, bulk ESS and tail ESS per element (csrc/ggp_chain_diag.cu; DESIGN.md section 2).
+    x: CUDA float64 tensor (n_draws, n_chains, n_elem), any strides.  Returns (rhat, ess_bulk, ess_tail), three (n_elem,)
+    float64 device tensors.  Elements are processed CHAIN_DIAG_WS_BYTES of workspace at a time; the results do not depend
+    on how they are grouped."""
+    torch = _lib.require_cuda()
+    lib = _lib.load()
+    if not torch.is_tensor(x) or not x.is_cuda or x.dtype != torch.float64 or x.dim() != 3:
+        raise ValueError('x must be a CUDA float64 tensor (n_draws, n_chains, n_elem)')
+    n, C, E = x.shape
+    per = lib.ggp_chain_diag_workspace_bytes(n, C, 1)
+    if per < 0:
+        raise ValueError('chain_diagnostics needs n_draws >= 4, n_chains >= 1 and n_chains * n_draws < 2^31 (got %d x %d)'
+                         % (n, C))
+    out = [torch.empty(E, dtype=torch.float64, device=x.device) for _ in range(3)]
+    if E == 0:
+        return tuple(out)
+    chunk = max(1, min(E, CHAIN_DIAG_WS_BYTES // per))
+    ws = torch.empty(chunk * per, dtype=torch.uint8, device=x.device)
+    sd, sc, se = x.stride()
+    for e0 in range(0, E, chunk):
+        ne = min(chunk, E - e0)
+        check(lib.ggp_chain_diag_f64(ptr(x[:, :, e0]), n, C, ne, sd, sc, se, ptr(out[0][e0:]), ptr(out[1][e0:]),
+                                     ptr(out[2][e0:]), ptr(ws), ws.numel(), stream_ptr()), 'ggp_chain_diag_f64')
+    return tuple(out)

@@ -209,9 +209,10 @@ class SepiaModel:
         return lp
 
     # ------------------------------------------------------------------ sampling
-    def _run(self, nsteps, step, do_propMH, n_chains=1, record_accept=False, prog=None, chunk=None):
+    def _run(self, nsteps, step, do_propMH, n_chains=1, record_accept=False, prog=None, chunk=None, device=False):
         """Run nsteps on the device, feeding the global np.random stream exactly as SEPIA would consume
-        it: draw an upper bound of uniforms, then rewind and advance by the number actually used."""
+        it: draw an upper bound of uniforms, then rewind and advance by the number actually used.
+        device=True: draws and logPost stay the CUDA tensors the engine wrote."""
         eng, tb = self._get_engine(n_chains)
         P = tb['theta'].size
         draws, lps, accs = [], [], []
@@ -230,8 +231,8 @@ class SepiaModel:
             if n_chains == 1:
                 np.random.set_state(state)
                 np.random.random_sample(int(used[0]))
-            draws.append(eng.to_host(out['draws'], 'draws'))
-            lps.append(eng.to_host(out['lp'], 'lp'))
+            draws.append(out['draws'] if device else eng.to_host(out['draws'], 'draws'))
+            lps.append(out['lp'] if device else eng.to_host(out['lp'], 'lp'))
             if record_accept:
                 accs.append(eng.to_host(out['accepted'], 'accepted'))
             self.launches += (1 if init else 0) + 1 + k          # [initial per-PC terms] + plan + one step kernel per step
@@ -239,8 +240,10 @@ class SepiaModel:
             done += k
             if prog is not None:
                 prog.update(k)
-        draws = np.concatenate(draws, axis=0)
-        lps = np.concatenate(lps, axis=0)
+        if device:
+            draws, lps = eng.torch.cat(draws, dim=0), eng.torch.cat(lps, dim=0)
+        else:
+            draws, lps = np.concatenate(draws, axis=0), np.concatenate(lps, axis=0)
         accs = np.concatenate(accs, axis=0) if record_accept else None
         return draws, lps, accs
 
@@ -277,15 +280,42 @@ class SepiaModel:
         draws, lps, _ = self._run(1, tb['step'], do_propMH)
         self._record(draws[:, 0, :], lps[:, 0])
 
-    def do_mcmc_chains(self, nsamp, n_chains, seed=None, do_propMH=True):
+    def do_mcmc_chains(self, nsamp, n_chains, seed=None, do_propMH=True, device=False):
         """Extension: n_chains independent chains of this model in one batched run (chains x PCs CTAs).
         Returns draws (nsamp, n_chains, P) and logPost (nsamp, n_chains); the model's own draw lists
-        are not touched.  Each chain gets its own slice of the np.random stream."""
+        are not touched.  Each chain gets its own slice of the np.random stream.
+        device=True: the draws and logPost are returned as the CUDA tensors the sampler wrote, without a download, so
+        that a large run can be diagnosed where it lives (mcmc_diagnostics)."""
         if seed is not None:
             np.random.seed(seed)
         _, tb = self._get_engine(n_chains)
-        draws, lps, _ = self._run(int(nsamp), tb['step'], do_propMH, n_chains=n_chains)
+        draws, lps, _ = self._run(int(nsamp), tb['step'], do_propMH, n_chains=n_chains, device=device)
         return draws, lps
+
+    def _recorded_chain(self):
+        """The recorded chain as (n, P) draws in the sampler's element order and (n,) logPost."""
+        blocks, _ = self._blocks()
+        cols = [np.asarray(b.mcmc.draws, dtype=np.float64).reshape((-1,) + b.val_shape).transpose(0, 2, 1)
+                .reshape(-1, b.val.size) for b in blocks]
+        return np.concatenate(cols, axis=1), np.asarray(self.params.lp.mcmc.draws, dtype=np.float64)
+
+    def mcmc_diagnostics(self, draws=None, lps=None, nburn=0):
+        """Rank-normalized split R-hat, bulk ESS and tail ESS per parameter element (DESIGN.md section 2), on the GPU.
+        Without arguments: the model's recorded chain (one chain, split in two).  draws (n, C, P) and lps (n, C), NumPy
+        arrays or CUDA tensors as do_mcmc_chains returns them: those chains.  The first nburn draws are left out.
+        Returns {name: dict(rhat, ess_bulk, ess_tail)} for betaU, lamUz, lamWs, lamWOs (arrays in each block's val_shape)
+        and logPost (scalars).  A fixed element, or one outside mcmcList, is constant: R-hat NaN, ESS = 2 C floor(n / 2)."""
+        from .. import diagnostics
+        if draws is None:
+            if lps is not None:
+                raise ValueError('lps without draws')
+            d, l = self._recorded_chain()
+            if d.shape[0] == 0:
+                raise ValueError('no recorded draws')
+            draws, lps = d[:, None, :], l[:, None]
+        elif lps is None:
+            raise ValueError('draws and lps go together')
+        return diagnostics.by_block(self._blocks()[0], diagnostics.chain_diagnostics(draws, lps, nburn))
 
     # ------------------------------------------------------------------ step-size tuning (SURVEY A.6)
     def tune_step_sizes(self, n_burn, n_levels, prog=True, diagnostics=False, update_vals=True, verbose=False,

@@ -242,6 +242,20 @@ int ggp_sobol_stats_f64(const double* fA, const double* fB, const double* fAB, i
                         const int* idx, long long idx_stride, int n, int R, int clamp,
                         double* first_out, double* total_out, void* stream);
 
+/* ---- MCMC convergence diagnostics (csrc/ggp_chain_diag.cu; DESIGN.md section 2 "Chain diagnostics") ----------------
+ * Rank-normalized split R-hat, bulk ESS and tail ESS of Vehtari et al. (2021), as ArviZ computes rhat(method="rank"),
+ * ess(method="bulk") and ess(method="tail"), with the autocovariance as a direct sum.  Draw i of chain c of element e is
+ * x[i*s_draw + c*s_chain + e*s_elem] (strides in doubles), which covers the sampler's (n_steps, n_chains, P) draws, its
+ * (n_steps, n_chains) logPost and one-chain-per-model layouts.  Per element: rhat_out[e], ess_bulk_out[e], ess_tail_out[e]
+ * (device, FP64; all three NaN if a draw is NaN or +-inf; R-hat NaN and ESS = 2 n_chains floor(n_draws/2) for a constant
+ * element).  Deterministic; an element's results do not depend on the other elements of the call.
+ * GGP_ERR_ARG: a null pointer, n_draws < 4, n_chains < 1, n_elem < 1, n_chains * n_draws >= 2^31, or workspace_bytes below
+ * ggp_chain_diag_workspace_bytes(n_draws, n_chains, n_elem) (which is -1 for arguments the call refuses). */
+long long ggp_chain_diag_workspace_bytes(int n_draws, int n_chains, int n_elem);
+int ggp_chain_diag_f64(const double* x, int n_draws, int n_chains, int n_elem, long long s_draw, long long s_chain,
+                       long long s_elem, double* rhat_out, double* ess_bulk_out, double* ess_tail_out, void* workspace,
+                       long long workspace_bytes, void* stream);
+
 /* ---- (4) randomized SVD passes -----------------------------------------------------------------
  * src/svd.py:52  Y = X @ omega           -> ggp_rsvd_sketch_f32 (OmegaT = omega^T, [r][n])
  * src/svd.py:56  Y = X @ X.T @ Y         -> ggp_rsvd_xty_f32 then ggp_rsvd_sketch_f32 (X (X^T Y))
