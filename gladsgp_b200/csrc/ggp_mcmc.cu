@@ -37,12 +37,23 @@ __device__ inline double elem_log_prior(int kind, double a, double b, double x)
     }
 }
 
+// pl.valid of a site: what the step kernel does there
+enum { SITE_REJECT = 0,      // nothing to evaluate: out of bounds, fixed, aCorr = 0, or a neutral site whose candidate the plan rejected
+       SITE_EVAL = 1,        // evaluate the candidate, then accept / reject
+       SITE_ACCEPT = 2 };    // neutral site whose candidate the plan accepted: th[s] = cand, the PC's term is unchanged
+enum { FIXED_NEUTRAL = 3 };  // fixed table: sampled betaU element of a constant input column (include/gladsgp_b200.h)
+
 struct Plan {
     double* cand;      // [n_chains][P]
     double* lacorr;    // [n_chains][P]
     double* logu;      // [n_chains][P]
-    int* valid;        // [n_chains][P]
+    int* valid;        // [n_chains][P]  SITE_*
 };
+
+__device__ __forceinline__ size_t chain_prior_off(const ggp_mcmc_args& a, int c)
+{
+    return a.per_chain_data ? (size_t)c * ((size_t)a.d * a.pu + 2 * a.pu + 1) : 0;
+}
 
 // candidates of step t for chain c (one thread)
 __device__ inline void plan_chain(const ggp_mcmc_args& a, const Plan& pl, int t, int c)
@@ -57,15 +68,17 @@ __device__ inline void plan_chain(const ggp_mcmc_args& a, const Plan& pl, int t,
         double cand, lac = 0.0, lu = 0.0;
         int valid;
         if (a.fixed[s] == 2) {            // block not in mcmcList: never visited, consumes no randomness
-            pl.cand[o] = th[s]; pl.lacorr[o] = 0.0; pl.logu[o] = 0.0; pl.valid[o] = 0;
+            pl.cand[o] = th[s]; pl.lacorr[o] = 0.0; pl.logu[o] = 0.0; pl.valid[o] = SITE_REJECT;
             continue;
         }
+        const bool neutral = a.fixed[s] == FIXED_NEUTRAL && s < a.d * a.pu;
+        const bool sampled = a.fixed[s] == 0 || neutral;
         if (a.replay) {
             const size_t ro = ((size_t)t * a.n_chains + c) * P + s;
             cand = a.r_cand[ro];
             lac = a.r_logacorr[ro];
             lu = a.r_logu[ro];
-            valid = a.r_valid[ro] && !a.fixed[s];
+            valid = a.r_valid[ro] && sampled;
         } else {
             const double x = th[s];
             const double st = step[s];
@@ -84,11 +97,21 @@ __device__ inline void plan_chain(const ggp_mcmc_args& a, const Plan& pl, int t,
                 const double w1 = fmax(1.0, cand / 3.0);
                 acorr = (x > cand + w1) ? 0.0 : w / w1;
             }
-            valid = !a.fixed[s] && (acorr > 0.0) && (cand >= a.lo[s]) && (cand <= a.hi[s]);
+            valid = sampled && (acorr > 0.0) && (cand >= a.lo[s]) && (cand <= a.hi[s]);
             if (valid) {
                 lu = log(us[pos++]);
                 lac = log(acorr);
             }
+        }
+        // Neutral site: the column is constant, so the candidate leaves the covariance and the PC's term exactly as they
+        // are (ll_new == ll_old) and the step kernel's rule ((ll_new - ll_old) + dprior) + lacorr reduces to the one below.
+        // th[s] is still its start-of-step value when the sweep reaches s (only site s writes it).  An infinite candidate
+        // (BetaRho, rho <= 0) would put inf * 0 into the covariance: it is evaluated as before.
+        if (valid && neutral && isfinite(cand)) {
+            const size_t po = chain_prior_off(a, c) + s;
+            const double dprior = elem_log_prior(a.prior_kind[s], a.prior_a[po], a.prior_b[po], cand) -
+                                  elem_log_prior(a.prior_kind[s], a.prior_a[po], a.prior_b[po], th[s]);
+            valid = (lu < dprior + lac) ? SITE_ACCEPT : SITE_REJECT;
         }
         pl.cand[o] = cand;
         pl.lacorr[o] = lac;
@@ -113,11 +136,6 @@ __device__ __forceinline__ double chain_lamsim(const ggp_mcmc_args& a, int c, in
 {
     return a.lamsim[(size_t)(a.per_chain_data ? c : 0) * a.pu + j];
 }
-__device__ __forceinline__ size_t chain_prior_off(const ggp_mcmc_args& a, int c)
-{
-    return a.per_chain_data ? (size_t)c * ((size_t)a.d * a.pu + 2 * a.pu + 1) : 0;
-}
-
 // parameters of PC j under the current state, optionally with one site replaced by its candidate
 __device__ inline void gather_block_params(const ggp_mcmc_args& a, const double* th, int c, int j, int site, double cand,
                                            double* beta_sm, double& lamz, double& diag_add)
@@ -248,8 +266,14 @@ sweep_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_str
         const int s = wos ? P - 1 : ((sl < d) ? j * d + sl : (sl == d ? d * pu + j : d * pu + pu + j));
         const size_t o = (size_t)c * P + s;
         const int valid = pl.valid[o];
-        if (!valid) {
-            if (lead && accd && !wos) accd[s] = 0;
+        if (valid != SITE_EVAL) {                  // decided by the plan (the lamWOs candidate is never SITE_ACCEPT)
+            const bool acc = valid == SITE_ACCEPT;
+            if (lead && !wos) {
+                if (acc) th[s] = pl.cand[o];
+                if (accd) accd[s] = acc ? 1 : 0;
+                if (shard) xrow[d + 4 + sl] = acc ? 1.0 : 0.0;
+            }
+            if (CL && acc) cluster_sync_all();     // the other CTAs of the cluster gather th[s] for the next evaluation
             continue;
         }
         const double cand = pl.cand[o];
@@ -325,14 +349,17 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p)
 }
 
 // st = private state of one lane: [0, d) betaU[:, j], [d] lamUz[j], [d + 1] lamWs[j], [d + 2] SigWl[j];  evaluation index
-// e: e < d betaU element, d lamUz, d + 1 lamWs, d + 2 lamWOs.  Up to two entries are replaced by candidates.
+// e: e < d betaU element, d lamUz, d + 1 lamWs, d + 2 lamWOs.  Up to two entries are replaced by candidates.  Neutral
+// sites the plan accepted (bits of nacc, candidates in ncand) are not in st until the end of the step: an evaluation
+// at index lim sees the candidates of those before it.
 __device__ inline void gather_spec(const ggp_mcmc_args& a, const double* st, double lamwos_cur, int c, int j,
-                                   int ea, double ca, int eb, double cb, double* beta_sm, double& lamz, double& diag_add)
+                                   int ea, double ca, int eb, double cb, unsigned long long nacc, const double* ncand, int lim,
+                                   double* beta_sm, double& lamz, double& diag_add)
 {
     const int d = a.d;
     if (threadIdx.x < d) {
         const int e = threadIdx.x;
-        beta_sm[e] = (e == ea) ? ca : ((e == eb) ? cb : st[e]);
+        beta_sm[e] = (e == ea) ? ca : ((e == eb) ? cb : ((e < lim && ((nacc >> e) & 1ULL)) ? ncand[e] : st[e]));
     }
     lamz = (ea == d) ? ca : ((eb == d) ? cb : st[d]);
     const double lamws = (ea == d + 1) ? ca : ((eb == d + 1) ? cb : st[d + 1]);
@@ -356,6 +383,7 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
     __shared__ double beta_sm[64];
     __shared__ int ev_sm[SPEC_MAXEV];
     __shared__ int nev_sm;
+    __shared__ unsigned long long nacc_sm;
     const int Mp = round_up32(a.m);
     const int G = (int)cluster_nctarank();
     const int cl = blockIdx.x / G;                       // cluster index along x: (PC, lane)
@@ -379,15 +407,26 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
         for (int e = 0; e < d + 2; ++e) xrow[d + 4 + e] = 0.0;
     }
     auto site_of = [&](int e) { return e < d ? j * d + e : (e == d ? d * pu + j : (e == d + 1 ? d * pu + pu + j : P - 1)); };
+    const double* ncand = pl.cand + (size_t)c * P + (size_t)j * d;       // candidates of the PC's betaU sites
 
-    // private state and the list of valid evaluations (identical in the three lanes)
+    // private state, the list of evaluations and the neutral sites the plan accepted (identical in the three lanes)
     if (threadIdx.x == 0) {
         int n = 0;
+        unsigned long long nacc = 0ULL;
         for (int e = 0; e < E; ++e) {
-            if (pl.valid[(size_t)c * P + site_of(e)]) ev_sm[n++] = e;
-            else if (lead && accd && lane_id == 0 && e < d + 2) accd[site_of(e)] = 0;
+            const int v = pl.valid[(size_t)c * P + site_of(e)];
+            if (v == SITE_EVAL) {
+                ev_sm[n++] = e;
+                continue;
+            }
+            if (v == SITE_ACCEPT) nacc |= 1ULL << e;
+            if (lead && lane_id == 0 && e < d + 2) {
+                if (accd) accd[site_of(e)] = (v == SITE_ACCEPT) ? 1 : 0;
+                if (shard) xrow[d + 4 + e] = (v == SITE_ACCEPT) ? 1.0 : 0.0;
+            }
         }
         nev_sm = n;
+        nacc_sm = nacc;
         if (cluster_ctarank() == 0) {
             for (int e = 0; e < d; ++e) st[e] = th[j * d + e];
             st[d] = th[d * pu + j];
@@ -397,6 +436,7 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
     }
     cluster_sync_all();
     const int nev = nev_sm;
+    const unsigned long long nacc = nacc_sm;
     const int nrounds = (nev + 1) >> 1;
 
     for (int r = 0; r < nrounds; ++r) {
@@ -412,9 +452,9 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
         if (work) {
             double lamz, diag_add;
             __syncthreads();
-            if (lane_id == 0) gather_spec(a, st, lamwos_cur, c, j, e0, c0, -1, 0.0, beta_sm, lamz, diag_add);
-            else if (lane_id == 1) gather_spec(a, st, lamwos_cur, c, j, e0, c0, e1, c1, beta_sm, lamz, diag_add);
-            else gather_spec(a, st, lamwos_cur, c, j, e1, c1, -1, 0.0, beta_sm, lamz, diag_add);
+            if (lane_id == 0) gather_spec(a, st, lamwos_cur, c, j, e0, c0, -1, 0.0, nacc, ncand, e0, beta_sm, lamz, diag_add);
+            else if (lane_id == 1) gather_spec(a, st, lamwos_cur, c, j, e0, c0, e1, c1, nacc, ncand, e1, beta_sm, lamz, diag_add);
+            else gather_spec(a, st, lamwos_cur, c, j, e1, c1, -1, 0.0, nacc, ncand, e1, beta_sm, lamz, diag_add);
             __syncthreads();
             ll = eval_dispatch<true, false, RA>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, wj, Lp, 0);
         }
@@ -468,6 +508,9 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
         // every launch adds the same number of arrivals to the counter, whatever the number of valid evaluations
         const int rcap = (E + 1) >> 1;
         if (nrounds < rcap) atomicAdd(cnt, (unsigned)(rcap - nrounds));
+        if (lane_id == 0)
+            for (int e = 0; e < d; ++e)
+                if ((nacc >> e) & 1ULL) st[e] = ncand[e];
         if (lane_id == 0 && shard) {
             for (int e = 0; e < d + 3; ++e) xrow[e] = st[e];                     // betaU[:, j], lamUz[j], lamWs[j], SigWl[j]
             if (pl.valid[(size_t)c * P + (P - 1)]) xrow[d + 3] = sig_cand[(size_t)c * pu + j];

@@ -82,13 +82,29 @@ def factor_unpack(factor_ws, m):
 
 PRIOR_KIND = {'Uniform': 0, 'Gamma': 1, 'Beta': 2, 'Normal': 3}
 PROP_KIND = {'Uniform': 0, 'BetaRho': 1, 'PropMH': 2}
+FIXED_NEUTRAL = 3
+
+
+def mark_neutral_sites(X, fixed, pu):
+    """The fixed table with every sampled betaU element (k, j) whose column k of X (m, d) is constant marked
+    FIXED_NEUTRAL.  Such a column adds beta * (x_ik - x_jk)^2 = 0 to every covariance entry whatever beta is, so the PC's
+    log-likelihood does not change under a betaU[k, j] proposal: the sampler decides it from the prior ratio alone
+    (include/gladsgp_b200.h).  betaU comes first in the table, in Fortran order (element k + j d)."""
+    X = np.asarray(X, dtype=np.float64)
+    d = X.shape[1]
+    const = np.all(X == X[:1], axis=0) & np.all(np.isfinite(X), axis=0)
+    fx = np.array(fixed, dtype=np.uint8).reshape(-1)
+    beta = fx[:d * pu].reshape(pu, d)                   # view: row j = PC j
+    beta[(beta == 0) & const[None, :]] = FIXED_NEUTRAL
+    return fx
 
 
 class McmcEngine:
     """Owns the device-side model + tables of one sim-only SEPIA model and runs chains on it.
 
     X (m,d) = zt, W (pu,m) PC weights, lamsim (pu,).  tables: dict of length-P numpy arrays
-    (prior_kind, prior_a, prior_b, lo, hi, prop_kind, fixed) in SEPIA sampling order.
+    (prior_kind, prior_a, prior_b, lo, hi, prop_kind, fixed) in SEPIA sampling order.  The betaU elements of constant
+    columns of X are marked in the device's fixed table (mark_neutral_sites): decided without an evaluation.
     per_chain=True: chain c is its own model on the shared design -- W (n_chains,pu,m), lamsim (n_chains,pu),
     tables['prior_a'] / ['prior_b'] (n_chains,P); the other tables are shared.
     """
@@ -111,6 +127,7 @@ class McmcEngine:
         else:
             self.pu = self.W.shape[0]
         self.P = self.d * self.pu + 2 * self.pu + 1
+        self.X_host = self.X.cpu().numpy()
         self.set_tables(tables)
         nb = self.lib.ggp_mcmc_workspace_bytes(self.m, self.d, self.pu, self.n_chains)
         self.ws = torch.empty(nb, dtype=torch.uint8, device=dev)
@@ -131,7 +148,8 @@ class McmcEngine:
         self.t_lo = _f64(np.asarray(tb['lo']).reshape(P), torch, dev)
         self.t_hi = _f64(np.asarray(tb['hi']).reshape(P), torch, dev)
         self.t_prop_kind = torch.as_tensor(np.asarray(tb['prop_kind'], dtype=np.int32).reshape(P), device=dev)
-        self.t_fixed = torch.as_tensor(np.asarray(tb['fixed'], dtype=np.uint8).reshape(P), device=dev)
+        fixed = mark_neutral_sites(self.X_host, np.asarray(tb['fixed'], dtype=np.uint8).reshape(P), self.pu)
+        self.t_fixed = torch.as_tensor(fixed, device=dev)
 
     def set_state(self, theta):
         th = _f64(np.asarray(theta, dtype=np.float64).reshape(-1, self.P), self.torch, 'cuda')

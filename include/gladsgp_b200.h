@@ -67,7 +67,11 @@ int ggp_factor_unpack_f64(const double* factor_ws, int m, int B, double* L_dense
  * chains of one model.  Parameter vector theta[P], P = d*pu + 2*pu + 1, in SEPIA's sampling order:
  * betaU in Fortran order (all d inputs of PC 0, then PC 1, ...), lamUz[pu], lamWs[pu], lamWOs.
  * Per-element tables have length P.  fixed: 0 sampled, 1 fixed (SEPIA still draws the candidate, then
- * rejects), 2 not in mcmcList (never visited, no draw).  Enumerations:
+ * rejects), 2 not in mcmcList (never visited, no draw), 3 sampled and likelihood-neutral: a betaU element
+ * (k, j) whose input column k of X holds the same finite value in every row (the dummy x of a model without
+ * x_sim).  Its beta multiplies (x_ik - x_jk)^2 = 0, so the PC's term does not depend on it; the sampler draws
+ * the candidate and the uniforms as for 0 and decides from the prior ratio alone, without an evaluation.
+ * Code 3 on any other element reads as 0.  Enumerations:
  *   prior_kind: 0 Uniform, 1 Gamma(a, b = rate), 2 Beta(a, b) on rho = exp(-x/4) (rho clamped to
  *               0.999), 3 Normal(a = mean, b = sd)
  *   prop_kind : 0 Uniform  x + step*U(-.5,.5);  1 BetaRho;  2 PropMH (Uniform when !do_propMH)
