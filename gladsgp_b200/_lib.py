@@ -71,6 +71,9 @@ SIGNATURES = {
     'ggp_chain_diag_workspace_bytes': (_LL, [_I, _I, _I]),
     'ggp_chain_diag_f64': (_I, [_P, _I, _I, _I, _LL, _LL, _LL, _P, _P, _P, _P, _LL, _P]),
     'ggp_sobol_stats_f64': (_I, [_P, _P, _P, _I, _I, _I, _P, _LL, _I, _I, _I, _P, _P, _P]),
+    'ggp_gp_sens_workspace_bytes': (_LL, [_I, _I, _I, _I, _I]),
+    'ggp_gp_sens_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _P, _P, _LL, _P]),
+    'ggp_main_effects_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _I, _P, _P, _LL, _P]),
     'ggp_rsvd_workspace_bytes': (_LL, [_I]),
     'ggp_rsvd_sketch_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P, _LL, _P]),
     'ggp_rsvd_xty_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P]),

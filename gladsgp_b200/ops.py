@@ -728,3 +728,46 @@ def chain_diagnostics(x):
         check(lib.ggp_chain_diag_f64(ptr(x[:, :, e0]), n, C, ne, sd, sc, se, ptr(out[0][e0:]), ptr(out[1][e0:]),
                                      ptr(out[2][e0:]), ptr(ws), ws.numel(), stream_ptr()), 'ggp_chain_diag_f64')
     return tuple(out)
+
+
+def _gp_sens_args(Z, beta, a, S, pu, mode):
+    torch = _lib.require_cuda()
+    Z = _f64(Z, torch, 'cuda')
+    if Z.dim() != 2:
+        raise ValueError('Z must be (m, q)')
+    m, q = Z.shape
+    beta = _f64(beta, torch, 'cuda').reshape(-1)
+    a = _f64(a, torch, 'cuda').reshape(-1)
+    if beta.numel() != S * pu * q or a.numel() != S * pu * m:
+        raise ValueError('beta must hold (S * pu, q) and a (S * pu, m) values')
+    if mode not in (0, 1):
+        raise ValueError("mode must be 0 ('samples') or 1 ('mean')")
+    nb = _lib.load().ggp_gp_sens_workspace_bytes(m, q, S, pu, mode)
+    if nb < 0:
+        raise ValueError('gp_sens needs m, S, pu >= 1 and 1 <= q <= 32 (got m=%d, q=%d, S=%d, pu=%d)' % (m, q, S, pu))
+    return torch, Z, beta, a, m, q, torch.empty(nb, dtype=torch.uint8, device='cuda')
+
+
+def gp_sens(Z, beta, a, S, pu, mode=0):
+    """Exact Sobol' moments of f = sum_n a_n prod_k exp(-beta_nk (x_k - z_nk)^2) on [0,1]^q (csrc/ggp_gp_sens.cu).
+    Z (m, q) training inputs, beta (S*pu, q) and a (S*pu, m) per block b = s*pu + j.  mode 0: one function per block;
+    mode 1: one per PC over every sample's terms (the weights as given).  Returns (M (F, 2q+1), E0 (F,)) float64 device
+    tensors: M[:, k] = M({k}), M[:, q+k] = M(all\\k), M[:, 2q] = M(all)."""
+    torch, Z, beta, a, m, q, ws = _gp_sens_args(Z, beta, a, S, pu, mode)
+    F = S * pu if mode == 0 else pu
+    M = torch.empty((F, 2 * q + 1), dtype=torch.float64, device='cuda')
+    E0 = torch.empty(F, dtype=torch.float64, device='cuda')
+    check(_lib.load().ggp_gp_sens_f64(ptr(Z), m, q, ptr(beta), ptr(a), S, pu, mode, ptr(M), ptr(E0), ptr(ws), ws.numel(),
+                                      stream_ptr()), 'ggp_gp_sens_f64')
+    return M, E0
+
+
+def main_effects(Z, beta, a, S, pu, grid, mode=0):
+    """Main-effect curves E[f | x_k = g] of the functions of gp_sens at the values of grid -> (F, q, ngrid) device tensor."""
+    torch, Z, beta, a, m, q, ws = _gp_sens_args(Z, beta, a, S, pu, mode)
+    g = _f64(grid, torch, 'cuda').reshape(-1)
+    F = S * pu if mode == 0 else pu
+    out = torch.empty((F, q, g.numel()), dtype=torch.float64, device='cuda')
+    check(_lib.load().ggp_main_effects_f64(ptr(Z), m, q, ptr(beta), ptr(a), S, pu, mode, ptr(g), g.numel(), ptr(out),
+                                           ptr(ws), ws.numel(), stream_ptr()), 'ggp_main_effects_f64')
+    return out

@@ -12,6 +12,10 @@ scipy's `_bca_interval`.  There is no CPU fallback.
 
 `emulator_mean_function(model, samples)` builds the `func` of sensitivity_indices.py:73-91 on the cached-factor device
 predictor: posterior-sample average of the emulator's PC weights at N designs per call.
+
+`gp_sensitivity_indices(model, samples, option, pcvar, ngrid)` computes the indices of that function (and of each
+posterior sample's mean function) exactly instead: the mean is a sum of product squared-exponential kernels, so every
+Sobol' integral over uniform inputs is a closed form in erf and exp (csrc/ggp_gp_sens.cu).
 """
 from collections import namedtuple
 from dataclasses import dataclass
@@ -155,3 +159,78 @@ def emulator_mean_function(model, samples):
         mean, _ = pred.predict(xp)
         return mean.reshape(ns, pu, xp.shape[0]).mean(dim=0).T.contiguous().cpu().numpy()
     return func
+
+
+def emulator_expansion(model, samples):
+    """The emulator's predictive mean of PC j under posterior sample s as a sum of product kernels over the inputs,
+    mu_sj(x) = sum_i a_sji prod_k exp(-beta_sjk (x_k - z_ik)^2),  a_sj = S22_sj^-1 w_j / lamUz_sj.
+    The inputs are the columns of model.num.zt except a dummy x (prediction puts x = 0.5 there, as in every training
+    row, so its kernel factor is 1).  S22^-1 w comes from the factors SepiaEmulatorPrediction caches with the model (built
+    and cached here if absent): (S22^-1 w)_i = z_i . u with z_i = L^-1 e_i.
+    Returns (Z (m, q), beta (ns*pu, q), a (ns*pu, m), ns), float64 device tensors, block b = s*pu + j."""
+    from .sepia.SepiaPredict import SepiaEmulatorPrediction
+    num = model.num
+    dummy = bool(model.data.dummy_x)
+    cols = np.arange(1 if dummy else 0, num.p + num.q)
+    if cols.size == 0:
+        raise ValueError('the model has no inputs to analyse (q = 0)')
+    x_pred = None if dummy else np.full((1, num.p), 0.5)
+    t_pred = np.full((1, num.q), 0.5) if num.q else None
+    proto = SepiaEmulatorPrediction(x_pred=x_pred, t_pred=t_pred, samples=samples, model=model, do_call=False)
+    ns = proto._predictor()
+    pred = proto._pred
+    alpha, _ = pred.xval_solve(np.arange(num.m))
+    a = alpha / pred.lamz[:, None]
+    c = pred.torch.as_tensor(cols, device='cuda')
+    return pred.X[:, c].contiguous(), pred.beta[:, c].contiguous(), a, ns
+
+
+def gp_sensitivity_indices(model, samples, option='samples', pcvar=None, ngrid=21):
+    """Exact first-order and total Sobol' indices and main-effect curves of the emulator's predictive mean, inputs
+    independent and uniform on [0, 1] in the transformed scale (csrc/ggp_gp_sens.cu; no sampling, no bootstrap).
+
+    option='samples': f = mu_sj for every posterior sample s and PC j: first, total (ns, pu, q); variance, mean (ns, pu);
+    the spread over s is the index's posterior uncertainty.  option='mean': f_j = mean_s mu_sj, the function
+    emulator_mean_function(model, samples) evaluates: first, total (pu, q); variance, mean (pu,).
+    An input with beta = 0 (for every sample, in 'mean') does not enter f: its indices are exactly 0.
+    pcvar (pu,): also general_first / general_total = sum_j pcvar_j S_jk, as PCA_saltelli_sensitivity_indices weights them.
+    grid = linspace(0, 1, ngrid); main_effect (..., q, ngrid) = E[f | x_k = grid] in PC-weight units; for a scalar-output
+    model also main_effect_native = main_effect * sd + mean.  Returns a dict of NumPy arrays."""
+    if option not in ('samples', 'mean'):
+        raise ValueError("option must be 'samples' or 'mean'")
+    ngrid = int(ngrid)
+    if ngrid < 1:
+        raise ValueError('ngrid must be at least 1')
+    pu = model.num.pu
+    if pcvar is not None:
+        pcvar = np.asarray(pcvar, dtype=np.float64).reshape(-1)
+        if pcvar.size != pu:
+            raise ValueError('pcvar must have one entry per PC (%d)' % pu)
+    Z, beta, a, ns = emulator_expansion(model, samples)
+    q = Z.shape[1]
+    mode = 0 if option == 'samples' else 1
+    if mode == 1:
+        a = a / ns
+    M, E0 = ops.gp_sens(Z, beta, a, ns, pu, mode)
+    grid = np.linspace(0.0, 1.0, ngrid)
+    me = ops.main_effects(Z, beta, a, ns, pu, grid, mode)
+    lead = (ns, pu) if mode == 0 else (pu,)
+    M = M.cpu().numpy().reshape(lead + (2 * q + 1,))
+    E0 = E0.cpu().numpy().reshape(lead)
+    zero = (beta == 0).cpu().numpy().reshape(ns, pu, q)
+    if mode == 1:
+        zero = np.all(zero, axis=0)
+    e2 = (E0 * E0)[..., None]
+    V = M[..., 2 * q] - E0 * E0
+    first = np.where(zero, 0.0, (M[..., :q] - e2) / V[..., None])
+    total = np.where(zero, 0.0, 1.0 - (M[..., q:2 * q] - e2) / V[..., None])
+    out = dict(first=first, total=total, variance=V, mean=E0, grid=grid,
+               main_effect=me.cpu().numpy().reshape(lead + (q, ngrid)))
+    if pcvar is not None:
+        out['general_first'] = np.einsum('...jk,j->...k', first, pcvar)
+        out['general_total'] = np.einsum('...jk,j->...k', total, pcvar)
+    if model.data.scalar_out:
+        sd = model.data.sim_data
+        out['main_effect_native'] = (out['main_effect'] * float(np.asarray(sd.orig_y_sd).reshape(-1)[0]) +
+                                     float(np.asarray(sd.orig_y_mean).reshape(-1)[0]))
+    return out

@@ -246,6 +246,26 @@ int ggp_sobol_stats_f64(const double* fA, const double* fB, const double* fAB, i
                         const int* idx, long long idx_stride, int n, int R, int clamp,
                         double* first_out, double* total_out, void* stream);
 
+/* ---- Closed-form GP sensitivity (csrc/ggp_gp_sens.cu) -------------------------------------------
+ * Exact Sobol' moments of f(x) = sum_n a_n prod_k exp(-beta_nk (x_k - z_nk)^2) with independent inputs uniform on
+ * [0,1]^q (the emulator's predictive mean of a PC weight: a = S22^-1 w / lamUz).  Blocks b = s * pu + j carry beta[b][q]
+ * and the weights a[b][m] of the m training rows Z[m][q] (the inputs only: no dummy-x column).
+ *   mode 0: one function per block, terms n = i (F = S pu functions);
+ *   mode 1: one function per PC j, terms n = (s, i) over every sample (F = pu; scale a by 1/S for the posterior mean).
+ * Per function f, with M(u) = E_{x_u}[(E_{x_~u} f)^2]:
+ *   M_out[f][k] = M({k}),  M_out[f][q + k] = M(all \ k)  (k < q),  M_out[f][2q] = M(all);   E0_out[f] = E[f].
+ * Then V = M(all) - E0^2, first-order S_k = (M({k}) - E0^2) / V, total T_k = 1 - (M(all\k) - E0^2) / V.
+ * ggp_main_effects_f64: out[f][k][g] = E[f | x_k = grid[g]] for a device grid[ngrid].
+ * FP64 libdevice erf / exp; sums in a fixed order (bit-identical between identical calls).  Both entry points take
+ * workspace_bytes >= ggp_gp_sens_workspace_bytes(m, q, S, pu, mode) (-1 for arguments the calls refuse).  GGP_ERR_ARG: a
+ * null pointer, m, S, pu or ngrid < 1, q outside [1, 32], mode not 0 or 1, S pu or S m >= 2^31. */
+long long ggp_gp_sens_workspace_bytes(int m, int q, int S, int pu, int mode);
+int ggp_gp_sens_f64(const double* Z, int m, int q, const double* beta, const double* a, int S, int pu, int mode,
+                    double* M_out, double* E0_out, void* workspace, long long workspace_bytes, void* stream);
+int ggp_main_effects_f64(const double* Z, int m, int q, const double* beta, const double* a, int S, int pu, int mode,
+                         const double* grid, int ngrid, double* out, void* workspace, long long workspace_bytes,
+                         void* stream);
+
 /* ---- MCMC convergence diagnostics (csrc/ggp_chain_diag.cu; DESIGN.md section 2 "Chain diagnostics") ----------------
  * Rank-normalized split R-hat, bulk ESS and tail ESS of Vehtari et al. (2021), as ArviZ computes rhat(method="rank"),
  * ess(method="bulk") and ess(method="tail"), with the autocovariance as a direct sum.  Draw i of chain c of element e is
