@@ -169,7 +169,7 @@ standardize_t_kernel(const float* __restrict__ Yt, long long ld, int m, long lon
 // ---------------------------------------------------------------------------------------------------------
 // projection on the basis, FP64 accumulation:  P[i][k] = sum_c X[i][c] * Kt[k][c]  (k < pu),
 // P[i][pu] = sum_c X[i][c],  P[i][pu+1] = sum_c X[i][c]^2.
-// Same streaming structure as the rSVD sketch (ggp_rsvd.cu): the CTA pulls 32-column chunks of its 256*RPT rows
+// Same streaming structure as the FP32-FMA rSVD sketch of commit 667fe96 (csrc/ggp_rsvd.cu): the CTA pulls 32-column chunks of its 256*RPT rows
 // through a padded shared-memory tile, each thread owns RPT rows and keeps their pu + 2 sums in registers.
 constexpr int PJ_THREADS = 256;
 

@@ -1,20 +1,20 @@
 // Randomized-SVD passes on the 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM).
 //
-// Same products as ggp_rsvd.cu (/root/reference/src/svd.py:52-60) -- Y = X Omega and Bt = Y^T X over the (m x n)
-// float32 ensemble -- but the multiply-adds run as 3xTF32 split products on the tensor pipe, so that the pass is
-// bound by the HBM read of X instead of the FP32 FMA rate:
+// The products of the reference's src/svd.py:52-60 -- Y = X Omega and Bt = Y^T X over the (m x n) float32 ensemble --
+// with the multiply-adds as 3xTF32 split products on the tensor pipe, so that the pass is bound by the HBM read of X
+// instead of the FP32 FMA rate:
 //     x = x_hi + x_lo (x_hi = tf32(x), x_lo = tf32(x - x_hi)),   x*o ~= x_hi*o_hi + x_hi*o_lo + x_lo*o_hi
 // (error ~2^-21 relative per product, i.e. FP32-level; the dropped x_lo*o_lo term is 2^-22 smaller than the product).
 // The tensor core adds into its FP32 accumulator with truncation, so a K-chunk (32 columns, 12 accumulator updates)
 // is summed in TMEM and then added to round-to-nearest FP32 register accumulators by the CUDA cores -- the long sum
 // over n never runs inside the tensor core.
 //
-// Operands are staged by the producer warps: global -> registers (split hi/lo) -> shared memory in the UMMA
-// canonical K-major 128-byte-swizzle layout (the one TMA would write; TMA cannot be used because the row pitch of
-// the reference's ensembles, 4*n_y bytes with n_y = 3693*365, is not a multiple of 16 bytes).  One elected thread of
-// the MMA warp issues tcgen05.mma and signals completion with tcgen05.commit on an mbarrier.
+// Operands reach shared memory in the UMMA canonical K-major 128-byte-swizzle layout.  Y = X Omega has one kernel per
+// pitch class: when the row pitch is a multiple of 16 bytes and both bases are 16-byte aligned, TMA writes the tiles
+// (sketch_tma_kernel); otherwise -- e.g. the reference's ensembles, 4*n_y bytes with n_y = 3693*365 -- the producer
+// warps stage them through registers (sketch_tc_kernel).  Bt = Y^T X writes its X operand straight into tensor memory
+// (xty_ts_kernel).  One elected thread issues tcgen05.mma and signals completion with tcgen05.commit on an mbarrier.
 #include <cuda.h>                 // CUtensorMap and the cuTensorMapEncodeTiled prototype (resolved at run time, no -lcuda)
-#include <cstdlib>
 #include "ggp_common.cuh"
 #include "../../include/gladsgp_b200.h"
 
@@ -29,10 +29,6 @@ constexpr int TC_A_BYTES = TC_ROWS * TC_K * 4;  // 32 KB (one of hi / lo)
 constexpr int TC_B_BYTES = 32 * TC_K * 4;       // 4 KB
 constexpr int TC_STAGE_BYTES = 2 * TC_A_BYTES + 2 * TC_B_BYTES;    // 72 KB
 constexpr int TC_TMEM_COLS = 128;            // 2 buffers x 2 tiles x 32 columns
-
-#ifndef GGP_TC_LD
-#define GGP_TC_LD __ldcs
-#endif
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -177,16 +173,11 @@ sketch_tc_kernel(const float* __restrict__ X, int m, long long n, const float* _
     const uint32_t tmem_base = tmem_base_sh;
 
     const long long nchunk = (n + TC_K - 1) / TC_K;
-#ifdef GGP_TC_INTERLEAVE
-    const int n_my = (blockIdx.x < nchunk) ? (int)((nchunk - 1 - blockIdx.x) / gridDim.x + 1) : 0;
-    auto chunk_col = [&](int it) { return ((long long)blockIdx.x + (long long)it * gridDim.x) * TC_K; };
-#else
     // a contiguous range of chunks per CTA: successive loads of a thread walk along one row of X
     const long long per = (nchunk + gridDim.x - 1) / gridDim.x;
     const long long ch_begin = (long long)blockIdx.x * per;
     const int n_my = (int)(ch_begin >= nchunk ? 0 : (nchunk - ch_begin < per ? nchunk - ch_begin : per));
     auto chunk_col = [&](int it) { return (ch_begin + it) * TC_K; };
-#endif
 
     if (warp < NPW) {
         // ================= producers =================
@@ -214,7 +205,7 @@ sketch_tc_kernel(const float* __restrict__ X, int m, long long n, const float* _
                     if (!((row_ok >> u) & 1)) {
                         xv[u][0] = 0.f; xv[u][1] = 0.f; xv[u][2] = 0.f; xv[u][3] = 0.f;
                     } else if (VEC) {
-                        const float4 q = GGP_TC_LD(reinterpret_cast<const float4*>(src));
+                        const float4 q = __ldcs(reinterpret_cast<const float4*>(src));
                         xv[u][0] = q.x; xv[u][1] = q.y; xv[u][2] = q.z; xv[u][3] = q.w;
                     } else {
 #pragma unroll
@@ -362,15 +353,26 @@ sketch_tc_kernel(const float* __restrict__ X, int m, long long n, const float* _
 // ---------------------------------------------------------------------------------------------------------
 // Y = X * Omega with the operand tiles brought in by TMA (cp.async.bulk.tensor, SWIZZLE_128B: the hardware writes the
 // 256 x 32 tile of X and the 32 x 32 tile of Omega^T straight into the K-major 128-byte-swizzle layout the MMA
-// descriptors expect).  Needs a row pitch that is a multiple of 16 bytes (n % 4 == 0) and a 16-byte aligned base; other
-// shapes keep the register-staged kernel above.  Raw stages (written by TMA) and derived stages (written by the splitters):
+// descriptors expect).  Needs a row pitch that is a multiple of 16 bytes (n % 4 == 0) and 16-byte aligned bases; other
+// shapes take the register-staged kernel above.  Raw stages (written by TMA) and derived stages (written by the splitters):
 //   warp 12     lane 0: per chunk, waits for the stage to be free, arms raw_full[stage] with the byte count and issues the
 //               two tensor copies (out-of-range rows / columns are zero-filled by the hardware)
-//   warps 0-7   splitters: wait for raw_full, turn every 16-byte piece x into tf32(x) (written back in place) and x - tf32(x)
-//               (written to the lo tile at the same swizzled offset), fence.proxy.async, arrive on full[stage]
-//   warps 8-11  MMA issue + epilogue, unchanged
-// The split, the order of the MMAs and the epilogue are those of sketch_tc_kernel: the two kernels give identical bits.
+//   warps 0-7   splitters: wait for raw_full, write x - trunc_tf32(x) of every 16-byte piece of X to the lo tile (same
+//               swizzled offset) and the hi and lo tiles of Omega, fence.proxy.async, arrive on full[stage]
+//   warps 8-11  MMA issue + epilogue
+// The hi tile of X is the raw float32 tile as TMA delivered it: the tensor core takes the upper 19 bits of each operand
+// element, i.e. tf32(x) by truncation (same accuracy against the float64 product as the rounded split of sketch_tc_kernel).
+// The two products that share it, x_hi o_hi and x_hi o_lo, are ONE MMA with N = 64 (the hi and lo tiles of Omega are adjacent,
+// i.e. rows 0-31 / 32-63 of one K-major operand), x_lo o_hi is a second one with N = 32: 16 instead of 24 MMAs per chunk, and
+// the X tiles are read from shared memory twice instead of three times.  The three partial sums live in separate TMEM columns
+// and are added in the epilogue (round-to-nearest FP32).  The result agrees with sketch_tc_kernel to FP32 level, not bitwise.
+// Shared memory: a ring of TMA_RAW raw stages [X raw 32 KB | Omega raw 4 KB] that only TMA writes -- four chunks of
+// prefetch, 108 KB in flight per SM -- and a ring of two derived stages [X lo 32 KB | Omega hi 4 KB | Omega lo 4 KB].
 constexpr int TMA_THREADS = 384 + 32;
+constexpr int TMA_RAW = 4;
+constexpr int TMA_RAW_BYTES = TC_A_BYTES + TC_B_BYTES;            // 36 KB
+constexpr int TMA_LO_BYTES = TC_A_BYTES + 2 * TC_B_BYTES;         // 40 KB
+constexpr int TMA_SMEM_BYTES = TMA_RAW * TMA_RAW_BYTES + 2 * TMA_LO_BYTES;   // 224 KB
 
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes)
 {
@@ -384,39 +386,12 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
         : "memory");
 }
 
-// FUSE: the two products that share the hi tile of X, x_hi o_hi and x_hi o_lo, are ONE MMA with N = 64 (the hi and lo tiles of
-// Omega are adjacent, i.e. rows 0-31 / 32-63 of one K-major operand), x_lo o_hi is a second one with N = 32: 16 instead of 24
-// MMAs per chunk and the X tiles are read from shared memory twice instead of three times.  The three partial sums live in
-// separate TMEM columns and are added in the epilogue (round-to-nearest FP32).
-// RAWHI: the hi tile of X is the raw float32 tile as TMA delivered it -- the tensor core takes the upper 19 bits of each operand
-// element, i.e. tf32(x) by truncation (checked: same accuracy against the float64 product) -- and the splitters only write
-// x - trunc_tf32(x) to the lo tile.
-// Shared memory: a ring of TMA_RAW raw stages [X raw 32 KB | Omega raw 4 KB] that only TMA writes (RAWHI) -- four chunks of
-// prefetch, 108 KB in flight per SM -- and a ring of two derived stages [X lo 32 KB | Omega hi 4 KB | Omega lo 4 KB].
-#ifndef GGP_TMA_BURST
-#define GGP_TMA_BURST 1      // adjacent chunks requested together (2: measured, no gain)
-#endif
-constexpr int TMA_BURST = GGP_TMA_BURST;
-constexpr int TMA_RAW = 4;
-constexpr int TMA_RAW_BYTES = TC_A_BYTES + TC_B_BYTES;            // 36 KB
-constexpr int TMA_LO_BYTES = TC_A_BYTES + 2 * TC_B_BYTES;         // 40 KB
-constexpr int TMA_SMEM_BYTES = TMA_RAW * TMA_RAW_BYTES + 2 * TMA_LO_BYTES;   // 224 KB
-
-__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, int c0, int c1, int c2, uint64_t* bar)
-{
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-
-template <bool FUSE, bool RAWHI, int DRY = 0>      // DRY (developer timing only, wrong results): 1 = no split, 2 = no split, no MMA
 __global__ void __launch_bounds__(TMA_THREADS, 1)
 sketch_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapO, int m, long long n,
-                  int r, int k0, float* __restrict__ partial, int dry_tiled = 0)
+                  int r, int k0, float* __restrict__ partial)
 {
-    constexpr int DCOLS = FUSE ? 96 : 32;                       // TMEM columns per 128-row tile and buffer
-    constexpr int TCOLS = FUSE ? 512 : TC_TMEM_COLS;            // 2 buffers x 2 tiles x DCOLS, rounded up to a power of two
+    constexpr int DCOLS = 96;                                   // TMEM columns per 128-row tile and buffer
+    constexpr int TCOLS = 512;                                  // 2 buffers x 2 tiles x DCOLS, rounded up to a power of two
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t raw_bar[TMA_RAW];          // TMA bytes of a raw stage have landed
     __shared__ __align__(8) uint64_t rawfree_bar[TMA_RAW];      // MMAs reading a raw stage are done
@@ -450,26 +425,16 @@ sketch_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constan
 
     if (warp == 12) {
         // ================= TMA producer (one thread) =================
+        // (The pure TMA stream of 256-row x 128-byte boxes, without split and MMA, tops out at 4.0 TB/s = 0.61 of the copy peak.)
         if (lane == 0) {
-            // (TMA_BURST > 1: adjacent chunks requested together -- their 128-byte row pieces are adjacent in memory; no gain measured.
-            //  The pure TMA stream of 256-row x 128-byte boxes, without split and MMA, tops out at 4.0 TB/s = 0.61 of the copy peak.)
-            for (int it0 = 0; it0 < n_my; it0 += TMA_BURST) {
-                const int nb = (n_my - it0 < TMA_BURST) ? n_my - it0 : TMA_BURST;
-                for (int b = 0; b < nb; ++b) {
-                    const int it = it0 + b, s = it % TMA_RAW;
-                    if (it >= TMA_RAW) mbar_wait(&rawfree_bar[s], (uint32_t)((it / TMA_RAW - 1) & 1));
-                }
-                for (int b = 0; b < nb; ++b) {
-                    const int it = it0 + b, s = it % TMA_RAW;
-                    unsigned char* st = smem_raw + (size_t)s * TMA_RAW_BYTES;
-                    const int c0 = (int)((ch_begin + it) * TC_K);
-                    mbar_arrive_expect_tx(&raw_bar[s], (uint32_t)TMA_RAW_BYTES);
-                    // (dry_tiled, DRY runs only: mapX describes the same bytes as contiguous 32 KB tiles -- what a tile-major copy
-                    //  of the ensemble would stream)
-                    if (DRY && dry_tiled) tma_load_2d(st, &mapX, 0, (int)(((long long)blockIdx.y * nchunk + ch_begin + it) * TC_ROWS), &raw_bar[s]);
-                    else tma_load_2d(st, &mapX, c0, row_base, &raw_bar[s]);
-                    tma_load_2d(st + TC_A_BYTES, &mapO, c0, k0, &raw_bar[s]);
-                }
+            for (int it = 0; it < n_my; ++it) {
+                const int s = it % TMA_RAW;
+                if (it >= TMA_RAW) mbar_wait(&rawfree_bar[s], (uint32_t)((it / TMA_RAW - 1) & 1));
+                unsigned char* st = smem_raw + (size_t)s * TMA_RAW_BYTES;
+                const int c0 = (int)((ch_begin + it) * TC_K);
+                mbar_arrive_expect_tx(&raw_bar[s], (uint32_t)TMA_RAW_BYTES);
+                tma_load_2d(st, &mapX, c0, row_base, &raw_bar[s]);
+                tma_load_2d(st + TC_A_BYTES, &mapO, c0, k0, &raw_bar[s]);
             }
         }
     } else if (warp < 8) {
@@ -480,26 +445,17 @@ sketch_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constan
             if (it >= 2) mbar_wait(&lofree_bar[l], (uint32_t)((it / 2 - 1) & 1));       // MMAs of chunk it-2 done with the slot
             unsigned char* st = smem_raw + (size_t)s * TMA_RAW_BYTES;
             unsigned char* lt = lo_base + (size_t)l * TMA_LO_BYTES;
-            if (DRY) { fence_async_smem(); mbar_arrive(&full_bar[l]); continue; }
             // 2048 16-byte pieces of X per stage, 8 per thread; consecutive threads, consecutive pieces (conflict-free);
-            // hi and lo share the (swizzled) offset, so the swizzle never has to be computed here
+            // the raw and the lo tile share the (swizzled) offset, so the swizzle never has to be computed here
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
                 const uint32_t off = (uint32_t)(u * 256 + tid) * 16u;
                 const uint4 x = *reinterpret_cast<const uint4*>(st + off);
-                uint4 hi, lo;
-                if (RAWHI) {
-                    lo.x = __float_as_uint(__uint_as_float(x.x) - __uint_as_float(x.x & 0xFFFFE000u));
-                    lo.y = __float_as_uint(__uint_as_float(x.y) - __uint_as_float(x.y & 0xFFFFE000u));
-                    lo.z = __float_as_uint(__uint_as_float(x.z) - __uint_as_float(x.z & 0xFFFFE000u));
-                    lo.w = __float_as_uint(__uint_as_float(x.w) - __uint_as_float(x.w & 0xFFFFE000u));
-                } else {
-                    split_tf32(__uint_as_float(x.x), hi.x, lo.x);
-                    split_tf32(__uint_as_float(x.y), hi.y, lo.y);
-                    split_tf32(__uint_as_float(x.z), hi.z, lo.z);
-                    split_tf32(__uint_as_float(x.w), hi.w, lo.w);
-                    *reinterpret_cast<uint4*>(st + off) = hi;
-                }
+                uint4 lo;
+                lo.x = __float_as_uint(__uint_as_float(x.x) - __uint_as_float(x.x & 0xFFFFE000u));
+                lo.y = __float_as_uint(__uint_as_float(x.y) - __uint_as_float(x.y & 0xFFFFE000u));
+                lo.z = __float_as_uint(__uint_as_float(x.z) - __uint_as_float(x.z & 0xFFFFE000u));
+                lo.w = __float_as_uint(__uint_as_float(x.w) - __uint_as_float(x.w & 0xFFFFE000u));
                 *reinterpret_cast<uint4*>(lt + off) = lo;
             }
             {
@@ -541,22 +497,15 @@ sketch_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constan
                 const uint32_t bh0 = al0 + (TC_A_BYTES >> 4);
                 const uint32_t d0 = tmem_base + (uint32_t)((it & 1) * 2 * DCOLS);
 #pragma unroll
-                for (int t = 0; t < (DRY == 2 ? 0 : 4); ++t) {
-                    const uint64_t bh = umma_join(bh0 + 2 * t, UMMA_SW128_HI);          // (FUSE: N = 64 spans the hi and the lo tile)
-                    const uint64_t bl = umma_join(bh0 + (TC_B_BYTES >> 4) + 2 * t, UMMA_SW128_HI);
+                for (int t = 0; t < 4; ++t) {
+                    const uint64_t bh = umma_join(bh0 + 2 * t, UMMA_SW128_HI);          // N = 64 spans the hi and the lo tile
 #pragma unroll
                     for (int tile = 0; tile < 2; ++tile) {
                         const uint64_t ah = umma_join(ah0 + tile * 1024 + 2 * t, UMMA_SW128_HI);
                         const uint64_t al = umma_join(al0 + tile * 1024 + 2 * t, UMMA_SW128_HI);
                         const uint32_t d = d0 + tile * DCOLS;
-                        if (FUSE) {
-                            if (t == 0) { umma_tf32<false>(d, ah, bh, idesc64); umma_tf32<false>(d + 64, al, bh, idesc); }
-                            else { umma_tf32<true>(d, ah, bh, idesc64); umma_tf32<true>(d + 64, al, bh, idesc); }
-                        } else {
-                            if (t == 0) umma_tf32<false>(d, al, bh, idesc); else umma_tf32<true>(d, al, bh, idesc);
-                            umma_tf32<true>(d, ah, bl, idesc);
-                            umma_tf32<true>(d, ah, bh, idesc);
-                        }
+                        if (t == 0) { umma_tf32<false>(d, ah, bh, idesc64); umma_tf32<false>(d + 64, al, bh, idesc); }
+                        else { umma_tf32<true>(d, ah, bh, idesc64); umma_tf32<true>(d + 64, al, bh, idesc); }
                     }
                 }
                 umma_commit(&rawfree_bar[s]);
@@ -569,31 +518,20 @@ sketch_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constan
                 mbar_wait(&tmem_full_bar[j & 1], (uint32_t)((j >> 1) & 1));
                 tc_fence_after();
                 const uint32_t tb = tmem_base + t_lane + (uint32_t)((j & 1) * 2 * DCOLS);
-                if (FUSE) {
-                    // per tile: columns [0, 32) x_hi o_hi, [32, 64) x_hi o_lo, [64, 96) x_lo o_hi: small terms first, then the sum
+                // per tile: columns [0, 32) x_hi o_hi, [32, 64) x_hi o_lo, [64, 96) x_lo o_hi: small terms first, then the sum
 #pragma unroll
-                    for (int tile = 0; tile < 2; ++tile)
+                for (int tile = 0; tile < 2; ++tile)
 #pragma unroll
-                        for (int h = 0; h < 2; ++h) {                              // 16 columns at a time: register budget
-                            uint32_t vh[16], vl[16], vx[16];
-                            tmem_ld16(tb + tile * DCOLS + 16 * h, vh);
-                            tmem_ld16(tb + tile * DCOLS + 32 + 16 * h, vl);
-                            tmem_ld16(tb + tile * DCOLS + 64 + 16 * h, vx);
-                            tmem_ld_wait();
+                    for (int h = 0; h < 2; ++h) {                              // 16 columns at a time: register budget
+                        uint32_t vh[16], vl[16], vx[16];
+                        tmem_ld16(tb + tile * DCOLS + 16 * h, vh);
+                        tmem_ld16(tb + tile * DCOLS + 32 + 16 * h, vl);
+                        tmem_ld16(tb + tile * DCOLS + 64 + 16 * h, vx);
+                        tmem_ld_wait();
 #pragma unroll
-                            for (int c = 0; c < 16; ++c)
-                                acc[tile][16 * h + c] += (__uint_as_float(vl[c]) + __uint_as_float(vx[c])) + __uint_as_float(vh[c]);
-                        }
-                } else {
-                    uint32_t v0[32], v1[32];
-                    tmem_ld32(tb, v0);
-                    tmem_ld32(tb + 32, v1);
-                    tmem_ld_wait();
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) acc[0][c] += __uint_as_float(v0[c]);
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) acc[1][c] += __uint_as_float(v1[c]);
-                }
+                        for (int c = 0; c < 16; ++c)
+                            acc[tile][16 * h + c] += (__uint_as_float(vl[c]) + __uint_as_float(vx[c])) + __uint_as_float(vh[c]);
+                    }
                 tc_fence_before();
             }
             asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -698,10 +636,10 @@ xty_ts_kernel(const float* __restrict__ X, int m, long long n, const float* __re
             const float* src = X + (size_t)i0 * n + col;
             if (col < n && i0 + 32 <= m) {
 #pragma unroll
-                for (int k = 0; k < 32; ++k) xv[k] = GGP_TC_LD(src + (size_t)k * n);
+                for (int k = 0; k < 32; ++k) xv[k] = __ldcs(src + (size_t)k * n);
             } else {
 #pragma unroll
-                for (int k = 0; k < 32; ++k) xv[k] = (col < n && i0 + k < m) ? GGP_TC_LD(src + (size_t)k * n) : 0.f;
+                for (int k = 0; k < 32; ++k) xv[k] = (col < n && i0 + k < m) ? __ldcs(src + (size_t)k * n) : 0.f;
             }
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
@@ -824,203 +762,6 @@ xty_ts_kernel(const float* __restrict__ X, int m, long long n, const float* __re
     }
 }
 
-// ---------------------------------------------------------------------------------------------------------
-// Bt = Y^T X with TMA-fed operand tiles (row pitch of X a multiple of 16 bytes).  The output column block (256 columns = two
-// M = 128 tiles) is the MMA's M dimension and the m rows are K:  D[c][k] = sum_i X[i][c] Y[i][k].  X is row-major, i.e.
-// contiguous along M: the A operand is MN-major, whose one legal layout for 32-bit elements is the "128-byte swizzle with
-// 32-byte atoms" (32 consecutive columns of one row per 128-byte line, the 32-byte unit u of line k at position u ^ (k % 4);
-// blocks of 32 columns 4096 bytes apart) -- exactly what TMA writes with CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B from a box of
-// 32 columns x 32 rows.  A chunk is eight such boxes side by side: 32 rows x 1 KB contiguous per row.  Y^T (r x m, a few KB,
-// transposed once by a small kernel) is the K-major B operand as Omega^T is in the sketch pass.  Raw / derived rings, splitters,
-// fused hi products and epilogue accumulation as in sketch_tma_kernel; a CTA walks down the rows of its column block in 32-row
-// chunks and writes the block of Bt after the last one.
-__device__ __forceinline__ uint64_t umma_desc_mn_sw128_32b(uint32_t saddr, uint32_t lbo, uint32_t sbo)
-{
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFF) << 32) | (1ull << 46) | (1ull << 61);
-}
-
-__global__ void transpose_pad_kernel(const float* __restrict__ Y, int m, int r, float* __restrict__ Yt, int pitch)
-{
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;               // Yt[k][i], k < r, i < pitch (zero beyond m)
-    if (idx >= r * pitch) return;
-    const int k = idx / pitch, i = idx - k * pitch;
-    Yt[idx] = (i < m) ? Y[(size_t)i * r + k] : 0.f;
-}
-
-// BOX3 (n a multiple of 32): X is described to TMA as a 3-D tensor {32 columns, m rows, n / 32 column blocks} (strides 4 n and 128
-// bytes), so that ONE box {32, 32, 8} brings the eight 32 x 32 blocks of a chunk in block-major order -- nine copies per chunk
-// were what bounded the 2-D version (1.15 ms against 0.95 for the register -> TMEM kernel).
-template <bool BOX3, int DRY = 0>
-__global__ void __launch_bounds__(TMA_THREADS, 1)
-xty_tma_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUtensorMap mapY, int m, long long n,
-               int r, int k0, float* __restrict__ Bt)
-{
-    constexpr int DCOLS = 96;
-    constexpr int TCOLS = 512;
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    __shared__ __align__(8) uint64_t raw_bar[TMA_RAW];
-    __shared__ __align__(8) uint64_t rawfree_bar[TMA_RAW];
-    __shared__ __align__(8) uint64_t full_bar[2];
-    __shared__ __align__(8) uint64_t lofree_bar[2];
-    __shared__ __align__(8) uint64_t tmem_full_bar[2];
-    __shared__ uint32_t tmem_base_sh;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    unsigned char* lo_base = smem_raw + TMA_RAW * TMA_RAW_BYTES;
-
-    if (tid == 0) {
-        for (int s = 0; s < TMA_RAW; ++s) { mbar_init(&raw_bar[s], 1); mbar_init(&rawfree_bar[s], 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(&full_bar[s], 256); mbar_init(&lofree_bar[s], 1); mbar_init(&tmem_full_bar[s], 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 8) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)),
-                     "r"(TCOLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_sh;
-
-    const int nk = (m + 31) / 32;                                           // K chunks per column block
-    const long long nblk = (n + TC_ROWS - 1) / TC_ROWS;                     // column blocks of 256
-    const int blk_my = (blockIdx.x < nblk) ? (int)((nblk - 1 - blockIdx.x) / gridDim.x + 1) : 0;
-    const int n_my = blk_my * nk;
-    auto blk_col = [&](int b) { return ((long long)blockIdx.x + (long long)b * gridDim.x) * TC_ROWS; };
-
-    if (warp == 12) {
-        if (lane == 0) {
-            for (int it = 0; it < n_my; ++it) {
-                const int s = it % TMA_RAW;
-                if (it >= TMA_RAW) mbar_wait(&rawfree_bar[s], (uint32_t)((it / TMA_RAW - 1) & 1));
-                unsigned char* st = smem_raw + (size_t)s * TMA_RAW_BYTES;
-                const int b = it / nk, kc = it - b * nk;
-                const int c0 = (int)blk_col(b), i0 = kc * 32;
-                mbar_arrive_expect_tx(&raw_bar[s], (uint32_t)TMA_RAW_BYTES);
-                if (BOX3) tma_load_3d(st, &mapX, 0, i0, c0 >> 5, &raw_bar[s]);
-                else {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) tma_load_2d(st + j * 4096, &mapX, c0 + 32 * j, i0, &raw_bar[s]);
-                }
-                tma_load_2d(st + TC_A_BYTES, &mapY, i0, k0, &raw_bar[s]);
-            }
-        }
-    } else if (warp < 8) {
-        for (int it = 0; it < n_my; ++it) {
-            const int s = it % TMA_RAW, l = it & 1;
-            mbar_wait(&raw_bar[s], (uint32_t)((it / TMA_RAW) & 1));
-            if (it >= 2) mbar_wait(&lofree_bar[l], (uint32_t)((it / 2 - 1) & 1));
-            unsigned char* st = smem_raw + (size_t)s * TMA_RAW_BYTES;
-            unsigned char* lt = lo_base + (size_t)l * TMA_LO_BYTES;
-            if (DRY) { fence_async_smem(); mbar_arrive(&full_bar[l]); continue; }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {                                   // X: raw tile = hi operand, lo = x - trunc_tf32(x)
-                const uint32_t off = (uint32_t)(u * 256 + tid) * 16u;
-                const uint4 x = *reinterpret_cast<const uint4*>(st + off);
-                uint4 lo;
-                lo.x = __float_as_uint(__uint_as_float(x.x) - __uint_as_float(x.x & 0xFFFFE000u));
-                lo.y = __float_as_uint(__uint_as_float(x.y) - __uint_as_float(x.y & 0xFFFFE000u));
-                lo.z = __float_as_uint(__uint_as_float(x.z) - __uint_as_float(x.z & 0xFFFFE000u));
-                lo.w = __float_as_uint(__uint_as_float(x.w) - __uint_as_float(x.w & 0xFFFFE000u));
-                *reinterpret_cast<uint4*>(lt + off) = lo;
-            }
-            {
-                const uint32_t off = (uint32_t)tid * 16u;                   // Y^T: hi and lo to the derived stage
-                const uint4 x = *reinterpret_cast<const uint4*>(st + TC_A_BYTES + off);
-                uint4 hi, lo;
-                split_tf32(__uint_as_float(x.x), hi.x, lo.x);
-                split_tf32(__uint_as_float(x.y), hi.y, lo.y);
-                split_tf32(__uint_as_float(x.z), hi.z, lo.z);
-                split_tf32(__uint_as_float(x.w), hi.w, lo.w);
-                *reinterpret_cast<uint4*>(lt + TC_A_BYTES + off) = hi;
-                *reinterpret_cast<uint4*>(lt + TC_A_BYTES + TC_B_BYTES + off) = lo;
-            }
-            fence_async_smem();
-            mbar_arrive(&full_bar[l]);
-        }
-    } else {
-        constexpr uint32_t idesc = umma_idesc_tf32(128, 32) | (1u << 15);       // A is MN-major
-        constexpr uint32_t idesc64 = umma_idesc_tf32(128, 64) | (1u << 15);
-        const int ew = warp - 8;
-        const uint32_t t_lane = (uint32_t)(32 * ew) << 16;
-        const uint32_t der_lo0 = umma_sw128_lo(smem_u32(lo_base));
-        float acc[2][32];
-#pragma unroll
-        for (int t = 0; t < 2; ++t)
-#pragma unroll
-            for (int c = 0; c < 32; ++c) acc[t][c] = 0.f;
-#pragma unroll 1
-        for (int it = 0; it <= n_my; ++it) {
-            if (it < n_my && warp == 8 && lane == 0) {
-                const int s = it % TMA_RAW, l = it & 1;
-                mbar_wait(&full_bar[l], (uint32_t)((it / 2) & 1));
-                tc_fence_after();
-                const uint32_t a_hi = smem_u32(smem_raw + (size_t)s * TMA_RAW_BYTES);
-                const uint32_t a_lo = smem_u32(lo_base + (size_t)l * TMA_LO_BYTES);
-                const uint32_t bh0 = der_lo0 + (uint32_t)l * (TMA_LO_BYTES >> 4) + (TC_A_BYTES >> 4);
-                const uint32_t d0 = tmem_base + (uint32_t)((it & 1) * 2 * DCOLS);
-#pragma unroll
-                for (int t = 0; t < (DRY == 2 ? 0 : 4); ++t) {
-                    const uint64_t bh = umma_join(bh0 + 2 * t, UMMA_SW128_HI);          // N = 64 spans the hi and the lo tile of Y^T
-#pragma unroll
-                    for (int tile = 0; tile < 2; ++tile) {
-                        const uint64_t ah = umma_desc_mn_sw128_32b(a_hi + tile * 16384 + t * 1024, 4096, 512);
-                        const uint64_t al = umma_desc_mn_sw128_32b(a_lo + tile * 16384 + t * 1024, 4096, 512);
-                        const uint32_t d = d0 + tile * DCOLS;
-                        if (t == 0) { umma_tf32<false>(d, ah, bh, idesc64); umma_tf32<false>(d + 64, al, bh, idesc); }
-                        else { umma_tf32<true>(d, ah, bh, idesc64); umma_tf32<true>(d + 64, al, bh, idesc); }
-                    }
-                }
-                umma_commit(&rawfree_bar[s]);
-                umma_commit(&lofree_bar[l]);
-                umma_commit(&tmem_full_bar[it & 1]);
-            }
-            __syncwarp();
-            if (it >= 1) {
-                const int j = it - 1;
-                mbar_wait(&tmem_full_bar[j & 1], (uint32_t)((j >> 1) & 1));
-                tc_fence_after();
-                const uint32_t tb = tmem_base + t_lane + (uint32_t)((j & 1) * 2 * DCOLS);
-#pragma unroll
-                for (int tile = 0; tile < 2; ++tile)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        uint32_t vh[16], vl[16], vx[16];
-                        tmem_ld16(tb + tile * DCOLS + 16 * h, vh);
-                        tmem_ld16(tb + tile * DCOLS + 32 + 16 * h, vl);
-                        tmem_ld16(tb + tile * DCOLS + 64 + 16 * h, vx);
-                        tmem_ld_wait();
-#pragma unroll
-                        for (int c = 0; c < 16; ++c)
-                            acc[tile][16 * h + c] += (__uint_as_float(vl[c]) + __uint_as_float(vx[c])) + __uint_as_float(vh[c]);
-                    }
-                tc_fence_before();
-                if ((j + 1) % nk == 0) {
-                    // last chunk of a column block: write Bt[k0 + c][col] and restart the sums
-                    const long long c0 = blk_col(j / nk);
-#pragma unroll
-                    for (int tile = 0; tile < 2; ++tile) {
-                        const long long col = c0 + tile * 128 + 32 * ew + lane;
-#pragma unroll
-                        for (int c = 0; c < 32; ++c) {
-                            if (col < n && k0 + c < r) __stcs(Bt + (size_t)(k0 + c) * n + col, acc[tile][c]);
-                            acc[tile][c] = 0.f;
-                        }
-                    }
-                }
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 8) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TCOLS));
-    }
-}
-
 // fixed-order FP64 sum of the per-CTA partials [nparts][m][32] -> Y[m][r] columns k0 .. k0+31
 __global__ void tc_reduce_kernel(const float* __restrict__ partial, int nparts, int m, int r, int k0,
                                  float* __restrict__ Y)
@@ -1054,22 +795,18 @@ static tmap_encode_fn tmap_encoder()
     }
     return fn;
 }
-// row-major float32 [rows][cols] (pitch = cols), box = box_rows x 32 columns, 128-byte swizzle, zero fill outside
-static bool make_tmap_f32(CUtensorMap* map, const float* base, long long rows, long long cols, int box_rows,
-                          long long pitch = 0, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B)
+// row-major float32 [rows][cols], box = box_rows x 32 columns, 128-byte swizzle, zero fill outside.  L2 promotion: a 128-byte
+// row piece pulls its 256-byte neighbourhood into L2 -- the other half is the same CTA's next chunk.
+static bool make_tmap_f32(CUtensorMap* map, const float* base, long long rows, long long cols, int box_rows)
 {
     tmap_encode_fn enc = tmap_encoder();
     if (!enc) return false;
     const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {(cuuint64_t)(pitch > 0 ? pitch : cols) * sizeof(float)};
+    const cuuint64_t strides[1] = {(cuuint64_t)cols * sizeof(float)};
     const cuuint32_t box[2] = {(cuuint32_t)TC_K, (cuuint32_t)box_rows};
     const cuuint32_t estr[2] = {1, 1};
-    // L2 promotion: a 128-byte row piece pulls its 256-byte neighbourhood into L2 -- the other half is the same CTA's next chunk
-    // (GGP_TMA_L2=128 / 256, developer experiments)
-    CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-    if (const char* e = getenv("GGP_TMA_L2")) promo = (atoi(e) == 128) ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : (atoi(e) == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
     return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, swz, promo,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
@@ -1110,25 +847,15 @@ int ggp_rsvd_sketch_tc_f32(const float* X, int m, long long n, const float* Omeg
     if (gx < 1) gx = 1;
     if (gx > nchunk) gx = nchunk;
     const size_t smem = (size_t)TC_STAGES * TC_STAGE_BYTES;
-    const bool vec = (n % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
-    // TMA-fed kernel: pitch a multiple of 16 bytes, 16-byte aligned bases, coordinates within int32 (GGP_TMA=0 switches it off)
-    const char* env_tma = getenv("GGP_TMA");
-    bool tma = vec && ((reinterpret_cast<uintptr_t>(OmegaT) & 15) == 0) && n < (1LL << 31) && !(env_tma && atoi(env_tma) == 0);
+    // 16-byte loads of both operands: row pitch a multiple of 16 bytes and 16-byte aligned bases
+    const bool vec = (n % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && ((reinterpret_cast<uintptr_t>(OmegaT) & 15) == 0);
+    // TMA-fed kernel: additionally, column coordinates within int32 and both tensor maps encode
     CUtensorMap mapX, mapO;
-    if (tma) tma = make_tmap_f32(&mapX, X, m, n, TC_ROWS) && make_tmap_f32(&mapO, OmegaT, r, n, 32);
+    const bool tma = vec && n < (1LL << 31) && make_tmap_f32(&mapX, X, m, n, TC_ROWS) && make_tmap_f32(&mapO, OmegaT, r, n, 32);
     if (tma) {
-        // GGP_TMA: 1 = same split and MMA order as the register-staged kernel (identical bits); 2 = fused hi products;
-        // 3 (default) = fused products + raw hi tile
-        const int mode = env_tma ? atoi(env_tma) : 3;
-        auto kern = (mode == 1) ? sketch_tma_kernel<false, false> : (mode == 2) ? sketch_tma_kernel<true, false> :
-                    (mode == 8) ? sketch_tma_kernel<true, true, 1> : (mode == 9) ? sketch_tma_kernel<true, true, 2> : sketch_tma_kernel<true, true>;
-        GGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_SMEM_BYTES));
-        int dry_tiled = 0;
-        if (mode >= 8 && getenv("GGP_TMA_TILED") && (long long)m * n % (32LL * TC_ROWS) == 0 && m % TC_ROWS == 0) {
-            dry_tiled = make_tmap_f32(&mapX, X, (long long)m * n / 32, 32, TC_ROWS) ? 1 : 0;
-        }
+        GGP_CUDA(cudaFuncSetAttribute(sketch_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_SMEM_BYTES));
         for (int k0 = 0; k0 < r; k0 += 32) {
-            kern<<<dim3((unsigned)gx, gy), TMA_THREADS, TMA_SMEM_BYTES, st>>>(mapX, mapO, m, n, r, k0, partial, dry_tiled);
+            sketch_tma_kernel<<<dim3((unsigned)gx, gy), TMA_THREADS, TMA_SMEM_BYTES, st>>>(mapX, mapO, m, n, r, k0, partial);
             GGP_CUDA(cudaGetLastError());
             tc_reduce_kernel<<<(m * 32 + 255) / 256, 256, 0, st>>>(partial, (int)gx, m, r, k0, Y_out);
             GGP_CUDA(cudaGetLastError());
@@ -1155,45 +882,6 @@ int ggp_rsvd_xty_tc_f32(const float* X, int m, long long n, const float* Y, int 
     const long long nblk = (n + TC_ROWS - 1) / TC_ROWS;
     long long gx = tc_sm_count();
     if (gx > nblk) gx = nblk;
-    // TMA-fed kernel (pitch of X a multiple of 16 bytes, aligned base): OFF by default, GGP_TMA_XTY=1 selects it.  Measured at cfg3
-    // size: 1.09-1.15 ms against 0.95 ms for the register -> TMEM kernel below; with split and MMA switched off its pure TMA stream
-    // (256 lines of 128 bytes per chunk, as one 3-D box or as eight 2-D boxes) runs at 3.3 TB/s -- the same ~9 cycles per 128-byte
-    // line per SM that bound the sketch pass's stream at 4.0 TB/s.  Kept as a tested, documented negative result.
-    const char* env_tma = getenv("GGP_TMA_XTY");
-    bool tma = (n % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && n < (1LL << 31) && (env_tma && atoi(env_tma) != 0);
-    if (tma) {
-        const int pitch = (m + 3) & ~3;
-        float* Yt = nullptr;
-        if (cudaMallocAsync(reinterpret_cast<void**>(&Yt), (size_t)r * pitch * sizeof(float), st) != cudaSuccess) { cudaGetLastError(); tma = false; }
-        CUtensorMap mapX, mapY;
-        const bool box3 = (n % 32 == 0);
-        if (tma && box3) {
-            tmap_encode_fn enc = tmap_encoder();
-            const cuuint64_t dims[3] = {32, (cuuint64_t)m, (cuuint64_t)(n / 32)};
-            const cuuint64_t strides[2] = {(cuuint64_t)n * sizeof(float), 32 * sizeof(float)};
-            const cuuint32_t box[3] = {32, 32, 8};
-            const cuuint32_t estr[3] = {1, 1, 1};
-            tma = enc && enc(&mapX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(X), dims, strides, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-        } else if (tma) {
-            tma = make_tmap_f32(&mapX, X, m, n, 32, 0, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
-        }
-        if (tma) tma = make_tmap_f32(&mapY, Yt, r, m, 32, pitch);
-        if (tma) {
-            transpose_pad_kernel<<<(r * pitch + 255) / 256, 256, 0, st>>>(Y, m, r, Yt, pitch);
-            const int mode = atoi(env_tma);             // 1 = the kernel; 8 / 9 = dry modes (developer timing only, wrong results)
-            auto kern = !box3 ? xty_tma_kernel<false> : (mode == 8) ? xty_tma_kernel<true, 1> : (mode == 9) ? xty_tma_kernel<true, 2> : xty_tma_kernel<true>;
-            GGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_SMEM_BYTES));
-            for (int k0 = 0; k0 < r; k0 += 32) {
-                kern<<<(unsigned)gx, TMA_THREADS, TMA_SMEM_BYTES, st>>>(mapX, mapY, m, n, r, k0, Bt_out);
-                GGP_CUDA(cudaGetLastError());
-            }
-            GGP_CUDA(cudaFreeAsync(Yt, st));
-            return GGP_OK;
-        }
-        if (Yt) cudaFreeAsync(Yt, st);
-    }
     for (int k0 = 0; k0 < r; k0 += 32) {
         xty_ts_kernel<<<(unsigned)gx, TC_THREADS, 0, st>>>(X, m, n, Y, r, k0, Bt_out);
         GGP_CUDA(cudaGetLastError());

@@ -493,32 +493,6 @@ def reconstruct_stats(w, K, sd, mean, q=0.025, noise=None):
     return tuple(outs)
 
 
-def rsvd_sketch(X, omegaT, ws=None):
-    """Y = X @ omega  (src/svd.py:52), omegaT = omega.T (r,n) f32 device tensor."""
-    torch = _lib.require_cuda()
-    lib = _lib.load()
-    m, n = X.shape
-    r = omegaT.shape[0]
-    need = lib.ggp_rsvd_workspace_bytes(m)
-    if ws is None or ws.numel() < need:
-        ws = torch.empty(need, dtype=torch.uint8, device='cuda')
-    Y = torch.empty((m, r), dtype=torch.float32, device='cuda')
-    check(lib.ggp_rsvd_sketch_f32(ptr(X), m, n, ptr(omegaT), r, ptr(Y), ptr(ws), ws.numel(), stream_ptr()),
-          'ggp_rsvd_sketch_f32')
-    return Y
-
-
-def rsvd_xty(X, Y):
-    """Bt (r,n) = Y^T X  (src/svd.py:60 with Y = Q)."""
-    torch = _lib.require_cuda()
-    lib = _lib.load()
-    m, n = X.shape
-    r = Y.shape[1]
-    Bt = torch.empty((r, n), dtype=torch.float32, device='cuda')
-    check(lib.ggp_rsvd_xty_f32(ptr(X), m, n, ptr(Y.contiguous()), r, ptr(Bt), stream_ptr()), 'ggp_rsvd_xty_f32')
-    return Bt
-
-
 # ------------------------------------------------------------------ ensemble ingest (SURVEY 8f rank 2)
 def _ens_dims(Y, transposed):
     if Y.dim() != 2 or Y.stride(1) != 1 or Y.dtype != _lib.require_cuda().float32:

@@ -2,9 +2,8 @@
 
 Same signature and return shapes; the three products over the (m, n) float32 ensemble
 (src/svd.py:52,56,60) run as streaming passes on the tcgen05 tensor cores (3xTF32 split products with
-FP32-level accuracy, csrc/ggp_rsvd_tc.cu; the FP32-FMA kernels of csrc/ggp_rsvd.cu remain available as
-ops.rsvd_sketch / ops.rsvd_xty), the m x r QR and the r x r eigen-problem run in FP64 in torch/cuSOLVER on the
-device.  The Gaussian test matrix is drawn from the global np.random stream exactly as the reference does
+FP32-level accuracy, csrc/ggp_rsvd_tc.cu), the m x r QR and the r x r eigen-problem run in FP64 in
+torch/cuSOLVER on the device.  The Gaussian test matrix is drawn from the global np.random stream exactly as the reference does
 (src/svd.py:51) unless `omega` is injected.
 """
 import numpy as np

@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define GGP_VERSION 200
+#define GGP_VERSION 201
 
 int ggp_version(void);
 const char* ggp_last_error_string(void);
@@ -281,16 +281,11 @@ int ggp_chain_diag_f64(const double* x, int n_draws, int n_chains, int n_elem, l
                        long long workspace_bytes, void* stream);
 
 /* ---- (4) randomized SVD passes -----------------------------------------------------------------
- * src/svd.py:52  Y = X @ omega           -> ggp_rsvd_sketch_f32 (OmegaT = omega^T, [r][n])
- * src/svd.py:56  Y = X @ X.T @ Y         -> ggp_rsvd_xty_f32 then ggp_rsvd_sketch_f32 (X (X^T Y))
- * src/svd.py:60  B = Q.T @ X             -> ggp_rsvd_xty_f32 (Bt_out[r][n] = Y^T X)
- * X[m][n] float32 row-major.  workspace: ggp_rsvd_workspace_bytes(m). */
-long long ggp_rsvd_workspace_bytes(int m);
-int ggp_rsvd_sketch_f32(const float* X, int m, long long n, const float* OmegaT, int r, float* Y_out,
-                        void* workspace, long long workspace_bytes, void* stream);
-int ggp_rsvd_xty_f32(const float* X, int m, long long n, const float* Y, int r, float* Bt_out, void* stream);
-/* The same products on the tcgen05 tensor cores (3xTF32 split, FP32-level accuracy; csrc/ggp_rsvd_tc.cu): bound by
- * the HBM read of X instead of the FP32 FMA rate.  Any m.  workspace: ggp_rsvd_tc_workspace_bytes(m). */
+ * src/svd.py:52  Y = X @ omega           -> ggp_rsvd_sketch_tc_f32 (OmegaT = omega^T, [r][n])
+ * src/svd.py:56  Y = X @ X.T @ Y         -> ggp_rsvd_xty_tc_f32 then ggp_rsvd_sketch_tc_f32 (X (X^T Y))
+ * src/svd.py:60  B = Q.T @ X             -> ggp_rsvd_xty_tc_f32 (Bt_out[r][n] = Y^T X)
+ * X[m][n] float32 row-major, any m.  The products run on the tcgen05 tensor cores (3xTF32 split, FP32-level accuracy;
+ * csrc/ggp_rsvd_tc.cu), bound by the HBM read of X.  workspace: ggp_rsvd_tc_workspace_bytes(m). */
 long long ggp_rsvd_tc_workspace_bytes(int m);
 int ggp_rsvd_sketch_tc_f32(const float* X, int m, long long n, const float* OmegaT, int r, float* Y_out,
                            void* workspace, long long workspace_bytes, void* stream);

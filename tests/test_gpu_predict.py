@@ -93,11 +93,11 @@ def test_rsvd_passes_match_numpy(cuda, m, n, r):
     X = rng.standard_normal((m, n)).astype(np.float32)
     om = rng.standard_normal((n, r)).astype(np.float32)
     Xd = torch.as_tensor(X, device='cuda')
-    Y = ops.rsvd_sketch(Xd, torch.as_tensor(om.T.copy(), device='cuda')).cpu().numpy()
+    Y = ops.rsvd_sketch_tc(Xd, torch.as_tensor(om.T.copy(), device='cuda')).cpu().numpy()
     ref = X.astype(np.float64) @ om.astype(np.float64)
     np.testing.assert_allclose(Y, ref, rtol=0, atol=3e-5 * np.abs(ref).max())
     Yq = rng.standard_normal((m, r)).astype(np.float32)
-    Bt = ops.rsvd_xty(Xd, torch.as_tensor(Yq, device='cuda')).cpu().numpy()
+    Bt = ops.rsvd_xty_tc(Xd, torch.as_tensor(Yq, device='cuda')).cpu().numpy()
     refB = Yq.astype(np.float64).T @ X.astype(np.float64)
     np.testing.assert_allclose(Bt, refB, rtol=0, atol=3e-5 * np.abs(refB).max())
 

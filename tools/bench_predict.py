@@ -68,10 +68,10 @@ def main():
     # rSVD passes on a 512 x 1.46M float32 ensemble
     Xe = torch.randn(m, n_y, device='cuda')
     om = torch.randn(25, n_y, device='cuda')
-    ws = torch.empty(_lib.load().ggp_rsvd_workspace_bytes(m), dtype=torch.uint8, device='cuda')
-    ts = ev(lambda: ops.rsvd_sketch(Xe, om, ws), iters=3, warm=1)
-    Y = ops.rsvd_sketch(Xe, om, ws)
-    tx = ev(lambda: ops.rsvd_xty(Xe, Y), iters=3, warm=1)
+    ws = torch.empty(_lib.load().ggp_rsvd_tc_workspace_bytes(m), dtype=torch.uint8, device='cuda')
+    ts = ev(lambda: ops.rsvd_sketch_tc(Xe, om, ws), iters=3, warm=1)
+    Y = ops.rsvd_sketch_tc(Xe, om, ws)
+    tx = ev(lambda: ops.rsvd_xty_tc(Xe, Y), iters=3, warm=1)
     res['rsvd_sketch_ms'] = ts; res['rsvd_sketch_gbs'] = 4.0 * m * n_y / ts / 1e6
     res['rsvd_xty_ms'] = tx; res['rsvd_xty_gbs'] = 4.0 * m * n_y / tx / 1e6
     print(json.dumps(res, indent=1))
