@@ -46,7 +46,6 @@ SIGNATURES = {
     'ggp_debug_exp_neg_f64': (_I, [_P, _P, _I, _P]),
     'ggp_factor_doubles': (_LL, [_I]),
     'ggp_padded_m': (_I, [_I]),
-    'ggp_set_lookahead': (_I, [_I]),
     'ggp_loglik_batched_f64': (_I, [_P, _I, _I, _P, _LL, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
     'ggp_factor_unpack_f64': (_I, [_P, _I, _I, _P, _P]),
     'ggp_sizeof_mcmc_args': (_I, []),

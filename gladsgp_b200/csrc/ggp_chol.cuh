@@ -16,10 +16,10 @@
 //   4. X = P * Minv^T again on DMMA: the accumulator fragments of step 2 are valid A fragments under a
 //      permutation of the k index, so no data movement is needed; X is stored to the packed factor
 //      straight from the fragments and the running forward solve of w is updated.
-// The covariance matrix itself never exists in memory.  Three schedules of the same arithmetic (bit-identical results):
-//   eval_block_loglik<false>   plain: steps 1-4 per panel, the CTA waits for the serial step 3;
-//   eval_block_loglik_la       look-ahead (default for one CTA per matrix): step 3 of panel j+1 runs while panel j is finished;
-//   eval_block_loglik<true>    one matrix per thread-block cluster (small batches, large matrices).
+// The covariance matrix itself never exists in memory.  Two schedules of the same arithmetic (bit-identical results):
+//   eval_block_loglik_la       look-ahead (one CTA per matrix): step 3 of panel j+1 runs while panel j is finished;
+//   eval_block_loglik<true>    one matrix per thread-block cluster (small batches, large matrices): steps 1-4 per panel.
+// eval_block_loglik<false, 1> runs steps 1-4 in one CTA on a given matrix (the prediction path's draw, ggp_chol_draw_f64).
 // The serial phase is written as compact loops over shared memory: a fully unrolled register version made the
 // kernel 200 KB of SASS and instruction-fetch bound (profiles/README.md).
 #pragma once
@@ -28,48 +28,8 @@
 
 namespace ggp {
 
-// optional phase timing (developer diagnostics): cycles spent by warp 0 and warp 7 of block 0 in each phase
-#ifdef GGP_PHASES
-__device__ unsigned long long g_phase[32];
-__device__ unsigned long long g_phase2[128];     // look-ahead variant: [warp][16] cycles per activity, block 0
-__device__ unsigned long long g_stage[4 * 64 * 2];  // look-ahead variant, block 0: [role][stage][0 = busy, 1 = wait at barrier (E)]
-#define LA_TICK(slot)                                                                       \
-    do {                                                                                    \
-        if (blockIdx.x == 0 && blockIdx.y == 0) {                                           \
-            unsigned long long now__ = clock64();                                           \
-            if ((threadIdx.x & 31) == 0) g_phase2[(threadIdx.x >> 5) * 16 + (slot)] += now__ - tla__; \
-            tla__ = now__;                                                                  \
-        }                                                                                   \
-    } while (0)
-#define GGP_TICK(slot)                                                                      \
-    do {                                                                                    \
-        if (blockIdx.x == 0 && blockIdx.y == 0 && lane == 0 && (warp == 0 || warp == 7)) {  \
-            unsigned long long now__ = clock64();                                           \
-            g_phase[(warp == 0 ? 0 : 16) + (slot)] += now__ - tlast__;                      \
-            tlast__ = now__;                                                                \
-        }                                                                                   \
-    } while (0)
-#define GGP_TICKW(w, slot, dep)                                                             \
-    do {                                                                                    \
-        if (blockIdx.x == 0 && blockIdx.y == 0 && warp == (w)) {                            \
-            unsigned long long now__ = clock64();                                           \
-            if ((dep) == 1.2345e300) now__ = 0;                                             \
-            if (lane == 0) { g_phase[(slot)] += now__ - tserial__; }                        \
-            tserial__ = now__;                                                              \
-        }                                                                                   \
-    } while (0)
-#else
-#define GGP_TICK(slot) do { } while (0)
-#define LA_TICK(slot) do { } while (0)
-#define GGP_TICKW(w, slot, dep) do { } while (0)
-#endif
-
 // entries of the shared-memory table of the in-kernel exponential (exp_neg below)
-#ifndef GGP_ETAB
-#define GGP_ETAB 64
-#endif
-constexpr int ETAB = GGP_ETAB;
-static_assert(ETAB == 32 || ETAB == 64, "exp table of 32 or 64 entries");
+constexpr int ETAB = 64;
 
 // DMMA steps / shared-memory doubles of the covariance distance product (see pair_cov)
 __host__ __device__ inline int cov_ksteps(int d) { return (d + 5) >> 2; }
@@ -94,11 +54,10 @@ __host__ __device__ inline size_t eval_smem_bytes(int Mp, int d) {
     return (size_t)(32 * D_LD + 32 * LT_LD + 32 * MI_LD + 32 + 32 + 8 + ETAB + Mp + (size_t)sc_doubles(d) + ((d + 1) & ~1)) * sizeof(double) + 16 + (size_t)(Mp / 8) * sizeof(int);
 }
 
-// shared-memory carve-out (percent of 228 KB) that just fits three CTAs: the rest stays L1 so that the
-// B-operand rows of a panel, shared by the eight warps, are served from L1 instead of L2
+// shared-memory carve-out (percent of 228 KB) that just fits CTAS_PER_SM CTAs: the rest stays L1 so that the
+// B-operand rows of a panel, shared by the warps of a CTA, are served from L1 instead of L2
 inline int eval_carveout_pct(size_t smem) {
-    if (const char* e = getenv("GGP_CARVEOUT_PCT")) return atoi(e);      // developer experiments
-    size_t need = GGP_CTAS_PER_SM * (smem + 1024);
+    size_t need = CTAS_PER_SM * (smem + 1024);
     int pct = (int)((need * 100 + 228 * 1024 - 1) / (228 * 1024));
     return pct > 100 ? 100 : pct;
 }
@@ -121,33 +80,25 @@ __device__ inline EvalSmem carve_eval_smem(unsigned char* base, int Mp, int d) {
     return s;
 }
 
-// exp(y) for y <= 0, ~1 ulp: y = (T n + j) ln2/T + r, |r| <= ln2/(2T), exp(y) = 2^n * 2^(j/T) * p(r), T = ETAB table entries.
-// T = 32: degree 7, 12 FP64 operations (libdevice exp: ~25) and a fraction of its code size; T = 64 (default since round 2):
-// |r| <= 0.0054, the r^6/720 term is below 4e-17, degree 5 is enough: 10 operations on the FP64 pipe the DMMAs share.
+// exp(y) for y <= 0, ~1 ulp: y = (T n + j) ln2/T + r, |r| <= ln2/(2T), exp(y) = 2^n * 2^(j/T) * p(r), T = ETAB = 64 table
+// entries.  |r| <= 0.0054, the r^6/720 term is below 4e-17, so degree 5 is enough: 10 operations on the FP64 pipe the DMMAs
+// share (libdevice exp: ~25), and a fraction of its code size.
 // Results below 1e-300 flush to 0 (covariance entries that small cannot influence any result at 1e-8).
 __device__ __forceinline__ double exp_neg(double y, const double* __restrict__ etab)
 {
-    constexpr double SC = (ETAB == 64) ? 2.0 : 1.0;
-    const double t = fma(y, SC * 46.166241308446828384, 6755399441055744.0);   // T/ln2, 1.5*2^52
+    const double t = fma(y, 92.33248261689366, 6755399441055744.0);          // T/ln2, 1.5*2^52
     const int nt = __double2loint(t);
     const double fn = t - 6755399441055744.0;
-    double r = fma(fn, -0.021660849390173098 / SC, y);                         // ln2/T high part (low 20 mantissa bits zero)
-    r = fma(fn, -2.325192846878874e-12 / SC, r);                                // ln2/T low part
-    double p;
-    if (ETAB == 64) {
-        p = 8.3333333333333332e-03;                                             // 1/120
-    } else {
-        p = 1.9841269841269841e-04;                                             // 1/5040
-        p = fma(p, r, 1.3888888888888889e-03);
-        p = fma(p, r, 8.3333333333333332e-03);
-    }
+    double r = fma(fn, -0.010830424695086549, y);                               // ln2/T high part (low 20 mantissa bits zero)
+    r = fma(fn, -1.162596423439437e-12, r);                                     // ln2/T low part
+    double p = 8.3333333333333332e-03;                                          // 1/120
     p = fma(p, r, 4.1666666666666664e-02);
     p = fma(p, r, 1.6666666666666666e-01);
     p = fma(p, r, 0.5);
     p = fma(p, r, 1.0);
     p = fma(p, r, 1.0);
     const double v = p * etab[nt & (ETAB - 1)];
-    const int n = nt >> ((ETAB == 64) ? 6 : 5);
+    const int n = nt >> 6;
     const double res = __hiloint2double(__double2hiint(v) + (n << 20), __double2loint(v));
     return (y < -690.0) ? 0.0 : res;
 }
@@ -175,19 +126,13 @@ __device__ inline void fill_slab_offsets(int* soff, int Mp)
 // Latency: the A fragment of the next sub-slab is loaded one iteration ahead into registers; further
 // ahead, lanes 0..4NU-1 pull the A lines of sub-slab s+6 into L2 and lanes 16..31 the B lines of
 // sub-slab s+2 into L1 (the B rows are shared by all warps of the CTA).
-#ifndef GGP_RA
-#define GGP_RA 2          // register ring depth of the A fragments (sub-slabs): loads run GGP_RA - 1 iterations ahead
-#endif
-#ifndef GGP_RB
-#define GGP_RB 2          // same for the B fragments
-#endif
-template <int NU, int RA = GGP_RA, int RB = GGP_RB>
+template <int NU>
 static __device__ __forceinline__ void panel_gemm(double (&acc)[2][4][2], const double* __restrict__ Ap,
                                                   const double* __restrict__ Lb, const int* __restrict__ soff, int j,
                                                   int row0, const int (&rb)[2], int g, int q, int a_ld)
 {
     constexpr int PD = 2;                    // prefetch distance in k-blocks (4 sub-slabs each)
-    static_assert(4 % RA == 0 && 4 % RB == 0, "ring depths must divide the 4 sub-slabs of a k-block");
+    constexpr int RA = 2, RB = 2;            // register ring depths (sub-slabs) of the A and B fragments: loads run R - 1 ahead
     const int lane = 4 * g + q;
     const int nsub = 4 * j;
     // sub-slab pointers: packed factor -> soff table; V workspace (a_ld != 0) -> s * a_ld * 8
@@ -265,65 +210,27 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-#ifndef GGP_DA
-#define GGP_DA 4          // depth (sub-slabs) of the per-warp shared-memory ring of A fragments; 0 = register ring (panel_gemm)
-#endif
-// per-warp scratch (doubles): covariance step (16 x 32) or the A ring of the product (DA slots x 2 units x 64)
-constexpr int SCR_DOUBLES = (GGP_DA * 128 > 512) ? GGP_DA * 128 : 512;
-constexpr int DA_SMALL = (GGP_DA > 4) ? 4 : GGP_DA;      // schedules whose scratch aliases LT + D (4 x 512 doubles)
-#ifndef GGP_PD
-#define GGP_PD 2
-#endif
-#ifndef GGP_LATRI
-#define GGP_LATRI 0       // look-ahead product of a diagonal block without its strictly upper 8 x 8 tiles (panel_gemm_cp, TRI):
-                          // 1 = one shared pattern (12 of 16 tiles), 2 = exact patterns (10 of 16), 0 = all 16.  Measured (bit-identical
-                          // results): the extra instantiations cost more (registers, code) than the 6 % of DMMAs they save:
-                          // batched 429 -> 371 / 365 k evaluations/s, sampler 394 -> 389 / 339 k (profiles/README.md)
-#endif
-#ifndef GGP_TAILSPLIT
-#define GGP_TAILSPLIT 0   // pairs at the end of a stage's pool that are handed out as single 8-row units (0: none; measured: no gain)
-#endif
-#ifndef GGP_BL1
-#define GGP_BL1 0         // 1: also pull the B lines of sub-slab s+2 k-blocks into L1 (pays only with a large L1 carve-out)
-#endif
-
 // Same product as panel_gemm (identical DMMA sequence per accumulator, hence bit-identical results), but the A
 // fragments travel global -> shared memory by cp.async (LDGSTS.128, L2 only) DA-1 sub-slabs ahead of their use instead
 // of one sub-slab ahead through registers: a warp no longer waits a full L2 / DRAM round trip per sub-slab, and the
 // loads in flight cost no registers.  The 16-byte piece a lane needs of an 8-row x 8-column unit block is piece number
 // `lane` of that block (row g, columns 2q..2q+1), so every lane copies exactly the pieces it later reads: no
 // cross-lane synchronisation, cp.async.wait_group alone orders the copy before the LDS.128 (conflict-free: consecutive
-// lanes, consecutive 16-byte pieces).  `ring`: per-warp shared memory, DA * NU * 64 doubles (the warp's covariance
+// lanes, consecutive 16-byte pieces).  `ring`: per-warp shared memory, DA * NU * 64 <= 512 doubles (the warp's covariance
 // scratch: idle during the product).  Packed-factor A operand only.
-// TRI (diagonal-block product of the look-ahead, NU = 2): strictly upper 8 x 8 tiles of the 32 x 32 block are left out.
-// TRI = 1: the warp's first unit needs column blocks 0..1 only, its second all four -- role 0 takes block rows 0 and 3,
-// role 1 block rows 1 and 2, so ONE pattern (6 of 8 tiles per warp, 12 of the block's 16, of which 10 are needed) serves both
-// warps; TRI = 2 / 3: the exact patterns (rows 0|3: 1 + 4 tiles, rows 1|2: 2 + 3 tiles), two more instantiations that cost
-// more registers than they save DMMAs.  The upper tiles were 6 % of all DMMAs of an evaluation and sat on the critical
-// chain; the tiles that are formed see the same DMMA sequence as before.
-template <int NU, int DA, int RB = GGP_RB, int TRI = 0>
+template <int NU>
 static __device__ __forceinline__ void panel_gemm_cp(double (&acc)[2][4][2], const double* __restrict__ Ap,
                                                      const double* __restrict__ Lb, const int* __restrict__ soff, int j,
                                                      int row0, const int (&rb)[2], int g, int q, double* __restrict__ ring)
 {
-    constexpr int PD = GGP_PD;               // L2 prefetch distance in k-blocks (4 sub-slabs each)
-    static_assert(DA == 2 || DA == 4 || DA == 8, "ring depth 2, 4 or 8 sub-slabs");
-    static_assert(TRI == 0 || NU == 2, "triangular form is for a pair");
-    constexpr int NCB = (TRI == 3) ? 3 : 4;                              // column blocks whose B fragments are needed
-    // column blocks of unit i: [0, cbn(i))
-    auto cbn = [](int i) constexpr {
-        return TRI == 0 ? 4 : (TRI == 1 ? (i == 0 ? 2 : 4) : (TRI == 2 ? (i == 0 ? 1 : 4) : (i == 0 ? 2 : 3)));
-    };
-    static_assert(4 % RB == 0, "B ring depth must divide the 4 sub-slabs of a k-block");
+    constexpr int PD = 2;                    // L2 prefetch distance in k-blocks (4 sub-slabs each)
+    constexpr int DA = 4;                    // depth (sub-slabs) of the shared-memory ring of A fragments
+    constexpr int RB = 2;                    // register ring depth of the B fragments
     const int lane = 4 * g + q;
     const int nsub = 4 * j;
     const int pa_unit = ((lane >> 4) < NU) ? (lane >> 4) : 0;
     const int pa_ks = (lane >> 2) & 3;
     const int pa_off = ((pa_unit == 0) ? rb[0] : rb[1]) * 8 + (lane & 3) * 16;
-#if GGP_BL1
-    const int pb_ks = lane >> 3;
-    const int pb_off = (row0 + 4 * (lane & 7)) * 8;
-#endif
     int aoff[NU];
 #pragma unroll
     for (int i = 0; i < NU; ++i) aoff[i] = (rb[i] + g) * 8 + 2 * q;
@@ -345,24 +252,16 @@ static __device__ __forceinline__ void panel_gemm_cp(double (&acc)[2][4][2], con
         if (t < nsub) {
             const double* sl = Lb + soff[t] + boff;
 #pragma unroll
-            for (int cb = 0; cb < NCB; ++cb) br[t][cb] = *reinterpret_cast<const double2*>(sl + 64 * cb);
+            for (int cb = 0; cb < 4; ++cb) br[t][cb] = *reinterpret_cast<const double2*>(sl + 64 * cb);
         }
     for (int kb = 0; kb < j; ++kb) {
-        if (kb + PD < j) {
-            const int sp = 4 * (kb + PD);
-            prefetch_l2(Ap + soff[sp + pa_ks] + pa_off);
-#if GGP_BL1
-            const double* pb = Lb + soff[sp + pb_ks] + pb_off;
-            prefetch_l1(pb);
-            prefetch_l1(pb + 16);
-#endif
-        }
+        if (kb + PD < j) prefetch_l2(Ap + soff[4 * (kb + PD) + pa_ks] + pa_off);
 #pragma unroll
         for (int ks = 0; ks < 4; ++ks) {
             const int s = 4 * kb + ks;
             if (s + DA - 1 < nsub) {
                 const double* sn = Ap + soff[s + DA - 1];
-                const int slot = (DA == 8) ? ((ks + 7) & 3) + 4 * ((kb + ((ks + 7) >> 2)) & 1) : (ks + DA - 1) % DA;
+                const int slot = (ks + DA - 1) % DA;
 #pragma unroll
                 for (int i = 0; i < NU; ++i) cp_async16(mine + (slot * NU + i) * 64, sn + aoff[i]);
             }
@@ -370,24 +269,21 @@ static __device__ __forceinline__ void panel_gemm_cp(double (&acc)[2][4][2], con
             if (s + RB - 1 < nsub) {
                 const double* sbn = Lb + soff[s + RB - 1] + boff;
 #pragma unroll
-                for (int cb = 0; cb < NCB; ++cb) br[(ks + RB - 1) % RB][cb] = *reinterpret_cast<const double2*>(sbn + 64 * cb);
+                for (int cb = 0; cb < 4; ++cb) br[(ks + RB - 1) % RB][cb] = *reinterpret_cast<const double2*>(sbn + 64 * cb);
             }
             cp_async_wait<DA - 1>();                          // sub-slab s has landed (the DA-1 younger groups may be in flight)
-            const int cur = (DA == 8) ? ks + 4 * (kb & 1) : ks % DA;
             double2 a[NU];
 #pragma unroll
-            for (int i = 0; i < NU; ++i) a[i] = *reinterpret_cast<const double2*>(mine + (cur * NU + i) * 64);
+            for (int i = 0; i < NU; ++i) a[i] = *reinterpret_cast<const double2*>(mine + (ks * NU + i) * 64);
             const double2 (&b)[4] = br[ks % RB];
 #pragma unroll
             for (int cb = 0; cb < 4; ++cb)
 #pragma unroll
-                for (int i = 0; i < NU; ++i)
-                    if (cb < cbn(i)) dmma884(acc[i][cb][0], acc[i][cb][1], a[i].x, b[cb].x);
+                for (int i = 0; i < NU; ++i) dmma884(acc[i][cb][0], acc[i][cb][1], a[i].x, b[cb].x);
 #pragma unroll
             for (int cb = 0; cb < 4; ++cb)
 #pragma unroll
-                for (int i = 0; i < NU; ++i)
-                    if (cb < cbn(i)) dmma884(acc[i][cb][0], acc[i][cb][1], a[i].y, b[cb].y);
+                for (int i = 0; i < NU; ++i) dmma884(acc[i][cb][0], acc[i][cb][1], a[i].y, b[cb].y);
         }
     }
 }
@@ -422,25 +318,17 @@ static __device__ __forceinline__ void unit_trsm(const double (&p)[4][2], double
 
 // -dist for NU units x 32 panel columns: dn += [x~, |x~|^2, 1] . B.  KS > 0: compile-time step count (the row values
 // stay in registers: every global load of the pair is in flight before the first use); KS = 0: runtime loop.
-#ifndef GGP_XPRE
-#define GGP_XPRE 0        // 1: the row coordinates of a pair are loaded before its DMMA product (d <= 10) instead of after it
-#endif
-constexpr int XPRE_KS = 3;                   // steps covered by the early load (d + 2 <= 12)
-
 template <int NU, int KS>
 static __device__ __forceinline__ void cov_dist(double (&dn)[2][4][2], const double* const (&xr)[2],
                                                 const double* __restrict__ SCB, const double* __restrict__ sb,
-                                                int d, int q, int lane, const double (*xpre)[XPRE_KS] = nullptr)
+                                                int d, int q, int lane)
 {
     if constexpr (KS > 0) {
         double x[NU][KS];
 #pragma unroll
         for (int i = 0; i < NU; ++i)
 #pragma unroll
-            for (int s = 0; s < KS; ++s) {
-                if (KS <= XPRE_KS && xpre != nullptr) x[i][s] = xpre[i][s];
-                else x[i][s] = (4 * s + q < d) ? __ldg(xr[i] + 4 * s + q) : 0.0;
-            }
+            for (int s = 0; s < KS; ++s) x[i][s] = (4 * s + q < d) ? __ldg(xr[i] + 4 * s + q) : 0.0;
         double rn[NU];
 #pragma unroll
         for (int i = 0; i < NU; ++i) {
@@ -510,8 +398,7 @@ static __device__ __forceinline__ void pair_cov(double (&p)[2][4][2], const doub
                                                 const bool (&row_ok)[2], const double* __restrict__ SCB,
                                                 const double* __restrict__ sb, int d, int m, int row0, int q,
                                                 double inv_lamz, double diag, bool self,
-                                                const double* __restrict__ etab, double* __restrict__ scr, int lane,
-                                                const double (*xpre)[XPRE_KS] = nullptr)
+                                                const double* __restrict__ etab, double* __restrict__ scr, int lane)
 {
     double dn[2][4][2];
     const double* xr[2];
@@ -521,14 +408,10 @@ static __device__ __forceinline__ void pair_cov(double (&p)[2][4][2], const doub
         for (int cb = 0; cb < 4; ++cb) { dn[i][cb][0] = 0.0; dn[i][cb][1] = 0.0; }
         xr[i] = Xr + (size_t)((i < NU && row_ok[i]) ? r[i] : 0) * d;
     }
-    const int ks = cov_ksteps(d);
-#ifdef GGP_PHASES
-    unsigned long long tla__ = clock64();
-#endif
-    switch (ks) {       // d <= 18 (every configuration of the reference: d = 2 -> 1 step, 9 -> 3, 17 -> 5): register-resident form
-        case 1: cov_dist<NU, 1>(dn, xr, SCB, sb, d, q, lane, xpre); break;
-        case 2: cov_dist<NU, 2>(dn, xr, SCB, sb, d, q, lane, xpre); break;
-        case 3: cov_dist<NU, 3>(dn, xr, SCB, sb, d, q, lane, xpre); break;
+    switch (cov_ksteps(d)) {       // d <= 18 (every configuration of the reference: d = 2 -> 1 step, 9 -> 3, 17 -> 5): register-resident form
+        case 1: cov_dist<NU, 1>(dn, xr, SCB, sb, d, q, lane); break;
+        case 2: cov_dist<NU, 2>(dn, xr, SCB, sb, d, q, lane); break;
+        case 3: cov_dist<NU, 3>(dn, xr, SCB, sb, d, q, lane); break;
         case 4: cov_dist<NU, 4>(dn, xr, SCB, sb, d, q, lane); break;
         case 5: cov_dist<NU, 5>(dn, xr, SCB, sb, d, q, lane); break;
         default: cov_dist<NU, 0>(dn, xr, SCB, sb, d, q, lane); break;
@@ -540,13 +423,8 @@ static __device__ __forceinline__ void pair_cov(double (&p)[2][4][2], const doub
             scr[(8 * i + 2 * cb) * 32 + lane] = dn[i][cb][0];
             scr[(8 * i + 2 * cb + 1) * 32 + lane] = dn[i][cb][1];
         }
-#ifdef GGP_PHASES
-    if (dn[0][0][0] == 1.2345e300) tla__ = 0;
-#endif
-    LA_TICK(8);
 #pragma unroll 8
     for (int e = 0; e < 8 * NU; ++e) scr[e * 32 + lane] = exp_neg(scr[e * 32 + lane], etab);
-    LA_TICK(9);
 #pragma unroll
     for (int i = 0; i < NU; ++i)
 #pragma unroll
@@ -601,12 +479,10 @@ static __device__ __forceinline__ void fill_panel_coords(double* __restrict__ SC
 // 8-row units are dealt round-robin to the G*NWARP warps, CTA 0 owns the diagonal block and publishes Minv / u
 // through global memory, panels are separated by cluster barriers (release/acquire), the running forward solve
 // of w lives in global memory.  Only CTA 0 returns the value.
-// RA: register ring depth of the A fragments in the pair GEMM (cluster kernels, 168 registers per thread: 4 for matrices up
-// to 1024 rows -- single-chain cfg3 +5 % -- and 2 above, where the deeper ring measured 10 % slower)
 // SRC = 1 (one CTA per matrix only): the matrix is GIVEN -- X points to a symmetric m x m row-major array instead of
 // coordinates (d = 0, beta unused) -- and the vector step is a product instead of a solve: u_out[0:m] = L w (the
 // multivariate-normal draw of the prediction path, ggp_chol_draw_f64).  The factorisation arithmetic is the same code.
-template <bool CL = false, int RA = GGP_RA, int SRC = 0>
+template <bool CL = false, int SRC = 0>
 static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, const double* __restrict__ X, int m, int Mp, int d,
                                     const double* beta, double lamz, double diag_add,
                                     const double* __restrict__ w, double* __restrict__ Lp,
@@ -636,10 +512,6 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
     if (tid == 0) sm.flag[0] = 0;
     double logdet = 0.0, quad = 0.0;    // partial sums, live in warp 0
     __syncthreads();
-#ifdef GGP_PHASES
-    unsigned long long tlast__ = clock64();
-    unsigned long long tserial__ = clock64();
-#endif
 
     for (int j = 0; j < nP; ++j) {
         const int row0 = j << 5;
@@ -653,7 +525,6 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
         if (CL) cluster_sync_all();                          // panel j-1 (factor rows, wres) visible cluster-wide
         if constexpr (SRC == 0) fill_panel_coords(sm.SC, X, sm.sb, d, m, row0);
         __syncthreads();
-        GGP_TICK(0);
         double* __restrict__ scr = LT + warp * 512;          // per-warp scratch of the covariance step (LT and D are idle then)
         static_assert(NWARP * 512 <= 32 * LT_LD + 32 * D_LD, "covariance scratch must fit in LT + D");
 
@@ -670,17 +541,10 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                 for (int cb = 0; cb < 4; ++cb) { acc[i][cb][0] = 0.0; acc[i][cb][1] = 0.0; }
             }
             // ------------------------------------------------------------------ 1. DMMA update
-            GGP_TICKW(2, 23, acc[0][0][0]);
             if (j > 0) {
-#if GGP_DA > 0
-                if (nu == 2) panel_gemm_cp<2, DA_SMALL>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, scr);
-                else if (nu == 1) panel_gemm_cp<1, DA_SMALL>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, scr);
-#else
-                if (nu == 2) panel_gemm<2, RA>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, 0);
-                else if (nu == 1) panel_gemm<1>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, 0);
-#endif
+                if (nu == 2) panel_gemm_cp<2>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, scr);
+                else if (nu == 1) panel_gemm_cp<1>(acc, Lp, Lp, sm.soff, j, row0, rb, g, q, scr);
             }
-            GGP_TICKW(2, 20, acc[0][0][0] + acc[1][3][1] + acc[0][3][1] + acc[1][0][0]);
             // ------------------------------------------------------------------ 2. covariance, P = C - S (registers)
             if constexpr (SRC == 0) {
                 const int rr[2] = {rb[0] + g, rb[1] + g};
@@ -704,7 +568,6 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                     }
                 }
             }
-            GGP_TICKW(2, 21, acc[0][0][0] + acc[1][3][1]);
 
             // ------------------------------------------------------------------ 3. diagonal block (first pair only)
             if (pr == 0) {
@@ -720,17 +583,14 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                                 D[(8 * u + g) * D_LD + 8 * cb + 2 * q + e] = acc[i][cb][e];
                     }
                 }
-                GGP_TICK(1);
                 if (!CL || crank == 0) {
                 __syncthreads();                                                 // (A)
-                GGP_TICK(2);
                 if (warp == 0) {
                     // Cholesky of the 32x32 block, lane = row.  Columns in blocks of 8 held in registers; pivots and
                     // multipliers are broadcast through shared memory (a double shuffle is ~25 SASS instructions
                     // with its divergence fallback); trailing columns get one rank-8 update per block.
                     double mypiv = 1.0;
                     int bad = 0;
-                    GGP_TICKW(0, 9, D[lane * D_LD]);
 #pragma unroll 1
                     for (int k0 = 0; k0 < 32; k0 += 8) {
                         double x[8];
@@ -765,13 +625,10 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                         __syncwarp();
                         if (bad) break;
                     }
-                    GGP_TICKW(0, 10, D[lane * D_LD + 31]);
                     if (bad) { if (lane == 0) { sm.flag[0] = bad; if (CL) aux[Mp + 32] = (double)bad; } }
                     else logdet += 0.5 * log(mypiv);
                 }
-                GGP_TICK(3);
                 __syncthreads();                                                 // (B0)
-                GGP_TICK(4);
                 const bool failed = sm.flag[0] != 0;
                 if (!CL && failed) {
                     if (tid == 0 && info) *info = sm.flag[0];
@@ -782,7 +639,6 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                     if constexpr (SRC == 0) {
                     // forward solve of the w block: u = Ljj^-1 wres[row0 : row0+32]
                     double b = wres[row0 + lane];
-                    GGP_TICKW(0, 11, b);
 #pragma unroll 1
                     for (int c = 0; c < 32; ++c) {
                         const double uc = __shfl_sync(0xffffffffu, b, c) * sm.rdiag[c];
@@ -812,12 +668,10 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                             *reinterpret_cast<double2*>(dst + c) = make_double2(D[lane * D_LD + cc], D[lane * D_LD + cc + 1]);
                         }
                     }
-                    GGP_TICKW(0, 12, quad);
                 } else if (warp == 1 && !failed) {
                     // Minv = Ljj^-1: lane k solves Ljj y = e_k.  Rows in blocks of 8: the contribution of all earlier
                     // rows is accumulated for the 8 rows at once (one own-column load + four broadcast LDS.128 of
                     // LT[t][i0..i0+7] per t), then an 8x8 triangular solve in registers.
-                    GGP_TICKW(1, 13, sm.rdiag[0]);
                     double* gm = Lp + minv_off(Mp) + 1024LL * j;
 #pragma unroll 1
                     for (int i0 = 0; i0 < 32; i0 += 8) {
@@ -848,11 +702,8 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                         }
                         __syncwarp();
                     }
-                    GGP_TICKW(1, 14, sm.Minv[lane]);
                 }
-                GGP_TICK(5);
                 __syncthreads();                                                 // (B)
-                GGP_TICK(6);
                 }
                 if (CL) {
                     cluster_sync_all();                      // Minv, u block, diagonal rows and flag published by CTA 0
@@ -874,7 +725,6 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
                 if (i < nu && !(pr == 0 && gw + TW * i < 4)) {
-                    GGP_TICKW(2, 23, acc[i][0][0]);
                     double xt[4][2];
                     unit_trsm(acc[i], xt, sm.Minv, g, q);
                     const int r = rb[i] + g;
@@ -891,13 +741,10 @@ static __device__ __forceinline__ double eval_block_loglik(const EvalSmem& sm, c
                     sdot += __shfl_xor_sync(0xffffffffu, sdot, 1);
                     sdot += __shfl_xor_sync(0xffffffffu, sdot, 2);
                     if (q == 0) wres[r] -= (SRC == 0) ? sdot : -sdot;
-                    GGP_TICKW(2, 22, sdot);
                 }
             }
         }
-        GGP_TICK(7);
         if (!CL) __syncthreads();                                                // (C)  (cluster variant: barrier at the top)
-        GGP_TICK(8);
     }
 
     if (warp == 0) {
@@ -943,7 +790,7 @@ struct LaSmem {
 
 __host__ __device__ inline size_t la_smem_bytes(int Mp, int d) {
     const int dpad = (d + 1) & ~1;
-    return (size_t)(32 * MI_LD + 32 * LT_LD + 32 * D_LD + 32 + 64 + 8 + ETAB + Mp + dpad + 2 * sc_doubles(d) + NWARP * SCR_DOUBLES) * sizeof(double) +
+    return (size_t)(32 * MI_LD + 32 * LT_LD + 32 * D_LD + 32 + 64 + 8 + ETAB + Mp + dpad + 2 * sc_doubles(d) + NWARP * 512) * sizeof(double) +
            16 + (size_t)(Mp / 8) * sizeof(int);
 }
 
@@ -961,7 +808,7 @@ __device__ inline LaSmem carve_la_smem(unsigned char* base, int Mp, int d) {
     s.wres = p;     p += Mp;
     s.sb = p;       p += dpad;
     s.SC = p;       p += 2 * sc_doubles(d);
-    s.scr = p;      p += NWARP * SCR_DOUBLES;
+    s.scr = p;      p += NWARP * 512;
     s.flag = reinterpret_cast<int*>(p);
     s.soff = s.flag + 4;
     s.scsz = sc_doubles(d);
@@ -979,34 +826,17 @@ __device__ __forceinline__ void bar01_wait(int id) { asm volatile("bar.sync %0, 
 // resident CTA, the DMMA pipes of two sub-partitions queue while the other two idle.  Each CTA therefore takes a rotation
 // from a per-SM arrival counter: the CTAs resident on one SM get different rotations, and every sub-partition sees the
 // same mix of roles.  Roles only decide WHICH warp computes an entry, never how: results are unchanged.
-#ifndef GGP_ROT
-#define GGP_ROT 1
-#endif
-#ifndef GGP_STAGGER_US
-#define GGP_STAGGER_US 0
-#endif
 static __device__ unsigned g_role_rot[1024];
 __device__ __forceinline__ int cta_role_rotation()          // every thread of the CTA; contains a __syncthreads
 {
-#if GGP_ROT
     __shared__ int rot_sm;
     if (threadIdx.x == 0) {
         unsigned smid;
         asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
         rot_sm = (int)(atomicAdd(&g_role_rot[smid & 1023u], 1u) & (unsigned)(NWARP - 1));
-#if GGP_STAGGER_US > 0
-        // developer experiment: start the CTAs resident on one SM a fraction of an evaluation apart
-        unsigned long long t0, t1;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-        const unsigned long long wait_ns = (unsigned long long)rot_sm * GGP_STAGGER_US * 1000ULL;
-        do { __nanosleep(2000); asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1)); } while (t1 - t0 < wait_ns);
-#endif
     }
     __syncthreads();
     return rot_sm;
-#else
-    return 0;
-#endif
 }
 
 static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, const double* __restrict__ X, int m, int Mp, int d,
@@ -1023,7 +853,7 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
     double* __restrict__ D = sm.D;
     double* __restrict__ LT = sm.LT;
     double* __restrict__ wres = sm.wres;
-    double* __restrict__ scr = sm.scr + warp * SCR_DOUBLES;
+    double* __restrict__ scr = sm.scr + warp * 512;
 
     __syncthreads();   // previous user of the shared buffers is done
     if (tid < d) sm.sb[tid] = sqrt(beta[tid]);
@@ -1033,71 +863,45 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
     if (tid == 0) sm.flag[0] = 0;
     double logdet = 0.0, quad = 0.0;    // partial sums, live in warp 0
     __syncthreads();
-#ifdef GGP_PHASES
-    unsigned long long tla__ = clock64();
-#endif
 
     for (int jc = 0; jc < nP; ++jc) {
-#ifdef GGP_PHASES
-        const unsigned long long tstage__ = clock64();
-#endif
         const int j = jc - 1;                       // panel finished in this stage (none in stage 0)
         if (j >= 0)                                 // inverse of block j, produced by the previous stage
             for (int idx = tid; idx < 1024; idx += NT) sm.Minv[(idx >> 5) * MI_LD + (idx & 31)] = D[(idx >> 5) * D_LD + (idx & 31)];
         fill_panel_coords(sm.SC + (jc & 1) * sm.scsz, X, sm.sb, d, m, jc << 5);
         if (tid == 0) sm.flag[1] = 0;
-        LA_TICK(0);
         __syncthreads();                                                         // (T)
-        LA_TICK(1);
         const int nreg = (j >= 0) ? ((Mp - 32 * j) >> 3) - 8 : 0;               // pool units of panel j (multiple of 4)
-        // pool tasks: 16-row pairs, except that the last GGP_TAILSPLIT pairs of the stage are handed out as 8-row units: the
-        // warps reach the end-of-stage barrier within one unit's time of each other instead of one pair's (the barrier
-        // was 20 % of all stall samples, profiles/r2a_sweep_kernel_lines.txt)
-        const int npair = nreg >> 1;
-        const int nsplit = (npair < GGP_TAILSPLIT) ? npair : GGP_TAILSPLIT;
-        const int nwhole = npair - nsplit;                   // tasks 0 .. nwhole-1 are pairs, the next 2 nsplit are units
+        const int npair = nreg >> 1;                         // pool tasks: 16-row pairs
         int phase = (warp < 2) ? (j >= 0 ? 0 : 1) : 2;       // 0 priority pair, 1 look-ahead pair, 2 pool, 3 inverse (warp 1)
         int pend = 0;        // warp 1: 1 = inverse of block jc still to do, 2 = do it after the pool pair in hand
 
 #pragma unroll 1
         while (true) {
             int cp = j, r0 = 0;
-#if GGP_TAILSPLIT > 0
-            bool single = false;                             // pool task of one 8-row unit (tail of the stage)
-#else
-            constexpr bool single = false;
-#endif
             if (phase == 2) {
                 if (pend == 2) phase = 3;
                 else {
                     int idx = 0;
                     if (lane == 0) idx = atomicAdd(&sm.flag[1], 1);
                     idx = __shfl_sync(0xffffffffu, idx, 0);
-                    if (idx >= nwhole + 2 * nsplit) {
+                    if (idx >= npair) {
                         if (pend == 0) break;
                         phase = 3;
                     } else {
                         if (pend == 1) pend = 2;
-#if GGP_TAILSPLIT > 0
-                        single = idx >= nwhole;
-#endif
-                        r0 = 32 * j + 64 + (single ? 16 * nwhole + 8 * (idx - nwhole) : 16 * idx);
+                        r0 = 32 * j + 64 + 16 * idx;
                     }
                 }
             } else {
                 cp = (phase == 0) ? j : jc;
                 r0 = 32 * jc + 16 * warp;
             }
-            // look-ahead pair (phase 1): role 0 takes the block's 8-row units 0 and 3, role 1 units 1 and 2 (5 lower tiles each)
-            const bool tri = GGP_LATRI && phase == 1;
-            const int u0 = tri ? warp : 2 * warp, u1 = tri ? 3 - warp : 2 * warp + 1;     // (phase 1 only)
             if (phase == 3) {
                 // warp 1 (after at most one pool pair, which overlaps warp 0's factorisation): inverse of block jc.
                 // Lane k solves Ljj y = e_k, rows in blocks of 8; result D[i][k] and the packed factor's inverse-block
                 // area (used by the prediction kernel)
-                LA_TICK(2);
                 bar01_wait(2);                                                   // (C) factor (LT, rdiag) or failure flag visible
-                LA_TICK(3);
                 if (sm.flag[0] == 0) {
                     double* gm = Lp + minv_off(Mp) + 1024LL * jc;
 #pragma unroll 1
@@ -1130,71 +934,25 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                         __syncwarp();
                     }
                 }
-                LA_TICK(4);
                 pend = 0;
                 phase = 2;
                 continue;
             }
             const int row0 = cp << 5;
-            const int rb[2] = {tri ? 32 * jc + 8 * u0 : r0, tri ? 32 * jc + 8 * u1 : r0 + 8};
+            const int rb[2] = {r0, r0 + 8};
             double acc[2][4][2];
 #pragma unroll
             for (int i = 0; i < 2; ++i)
 #pragma unroll
                 for (int cb = 0; cb < 4; ++cb) { acc[i][cb][0] = 0.0; acc[i][cb][1] = 0.0; }
-#if GGP_XPRE
-            // row coordinates of the pair for the covariance step: requested now, they arrive during the product
-            double xpre[2][XPRE_KS];
-            const bool use_xpre = cov_ksteps(d) <= XPRE_KS;
-            if (use_xpre) {
-#pragma unroll
-                for (int i = 0; i < 2; ++i) {
-                    const int r = rb[i] + g;
-                    const double* xrow = X + (size_t)(r < m ? r : 0) * d;
-#pragma unroll
-                    for (int s2 = 0; s2 < XPRE_KS; ++s2) xpre[i][s2] = (4 * s2 + q < d) ? __ldg(xrow + 4 * s2 + q) : 0.0;
-                }
-            }
-#endif
             // ------------------------------------------------------------------ 1. DMMA update
-            LA_TICK(2);
-#if GGP_DA > 0
-            if (cp > 0) {
-                if constexpr (GGP_TAILSPLIT > 0) { if (single) panel_gemm_cp<1, GGP_DA>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr); }
-                if (single) { }
-#if GGP_LATRI == 2
-                else if (tri && warp == 0) panel_gemm_cp<2, GGP_DA, GGP_RB, 2>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr);
-                else if (tri) panel_gemm_cp<2, GGP_DA, GGP_RB, 3>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr);
-#elif GGP_LATRI == 1
-                else if (tri) panel_gemm_cp<2, GGP_DA, GGP_RB, 1>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr);
-#endif
-                else panel_gemm_cp<2, GGP_DA>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr);
-            }
-#else
-            if (cp > 0) {
-                if constexpr (GGP_TAILSPLIT > 0) { if (single) panel_gemm<1>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, 0); }
-                if (!single) panel_gemm<2>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, 0);
-            }
-#endif
-#ifdef GGP_PHASES
-            if (acc[0][0][0] + acc[1][3][1] == 1.2345e300) tla__ = 0;
-#endif
-            LA_TICK(5);
+            if (cp > 0) panel_gemm_cp<2>(acc, Lp, Lp, sm.soff, cp, row0, rb, g, q, scr);
             // ------------------------------------------------------------------ 2. covariance, P = C - S (registers)
             {
                 const int rr[2] = {rb[0] + g, rb[1] + g};
-                const bool ok[2] = {rr[0] < m, rr[1] < m && !single};   // (a unit task runs the pair code with its second unit masked)
-#if GGP_XPRE
-                pair_cov<2>(acc, X, rr, ok, sm.SC + (cp & 1) * sm.scsz, sm.sb, d, m, row0, q, inv_lamz, diag, true, sm.etab, scr, lane,
-                            use_xpre ? xpre : nullptr);
-#else
+                const bool ok[2] = {rr[0] < m, rr[1] < m};
                 pair_cov<2>(acc, X, rr, ok, sm.SC + (cp & 1) * sm.scsz, sm.sb, d, m, row0, q, inv_lamz, diag, true, sm.etab, scr, lane);
-#endif
             }
-#ifdef GGP_PHASES
-            if (acc[0][0][0] + acc[1][3][1] == 1.2345e300) tla__ = 0;
-#endif
-            LA_TICK(6);
             if (phase == 1) {
                 // -------------------------------------------------------------- 3. diagonal block jc (look-ahead)
 #pragma unroll
@@ -1203,14 +961,12 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                     for (int cb = 0; cb < 4; ++cb)
 #pragma unroll
                         for (int e = 0; e < 2; ++e)
-                            D[(8 * (i == 0 ? u0 : u1) + g) * D_LD + 8 * cb + 2 * q + e] = acc[i][cb][e];
+                            D[(16 * warp + 8 * i + g) * D_LD + 8 * cb + 2 * q + e] = acc[i][cb][e];
                 if (warp == 1) {
                     bar01_arrive(1);                                             // (B) this half of the block is in D
                     pend = 1;                                                    // inverse after at most one pool pair
                 } else {
-                    LA_TICK(7);
                     bar01_wait(1);                                               // (B) block complete in D
-                    LA_TICK(3);
                     int failed;
                     {
                         // Cholesky of the 32x32 block, lane = row (same arithmetic as eval_block_loglik)
@@ -1254,7 +1010,6 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                         else logdet += 0.5 * log(mypiv);
                         failed = bad;
                     }
-                    LA_TICK(10);
                     bar01_arrive(2);                                             // (C) factor (LT, rdiag) or failure flag published
                     if (!failed) {
                         // forward solve of the w block: u = Ljj^-1 wres[row0 : row0+32]  (L read from LT: D is being
@@ -1283,7 +1038,6 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                             }
                         }
                     }
-                    LA_TICK(11);
                 }
                 phase = 2;
             } else {
@@ -1293,7 +1047,6 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                 const double* __restrict__ ujj = sm.uj + (j & 1) * 32;
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
-                    if (i == 1 && single) break;
                     double xt[4][2];
                     unit_trsm(acc[i], xt, sm.Minv, g, q);
                     const int r = rb[i] + g;
@@ -1311,27 +1064,13 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
                     sdot += __shfl_xor_sync(0xffffffffu, sdot, 2);
                     if (q == 0) wres[r] -= sdot;
                 }
-                LA_TICK(12);
                 if (phase == 0) {
                     bar_pair01();                                                // (A) rows of block jc complete in panels 0..j
                     phase = 1;
-                    LA_TICK(3);
                 }
             }
         }
-        LA_TICK(2);
-#ifdef GGP_PHASES
-        const unsigned long long te0__ = clock64();
-#endif
         __syncthreads();                                                         // (E)
-#ifdef GGP_PHASES
-        if (blockIdx.x == 0 && blockIdx.y == 0 && lane == 0 && jc < 64) {
-            const unsigned long long te1__ = clock64();
-            g_stage[(warp * 64 + jc) * 2 + 0] += te0__ - tstage__;
-            g_stage[(warp * 64 + jc) * 2 + 1] += te1__ - te0__;
-        }
-#endif
-        LA_TICK(13);
         if (sm.flag[0] != 0) {
             if (tid == 0 && info) *info = sm.flag[0];
             return -INFINITY;
@@ -1348,22 +1087,10 @@ static __device__ __forceinline__ double eval_block_loglik_la(const LaSmem& sm, 
     return sm.red[0];
 }
 
-// look-ahead variant on (default) / off: GGP_LOOKAHEAD=0 in the environment or ggp_set_lookahead(0) (tests, A/B runs)
-inline int& lookahead_flag()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GGP_LOOKAHEAD");
-        v = (e && atoi(e) == 0) ? 0 : 1;
-    }
-    return v;
-}
-inline bool use_lookahead() { return lookahead_flag() != 0; }
-
 // Cluster size for `ntasks` independent matrices: one CTA per matrix when the machine is already full, otherwise
-// the largest power of two that still fits all clusters in one wave of GGP_CL_CTAS_PER_SM resident CTAs per SM: up to 8
+// the largest power of two that still fits all clusters in one wave of CL_CTAS_PER_SM resident CTAs per SM: up to 8
 // (the portable cluster limit), 16 for matrices of 1024 rows and more (cfg 5: one chain of 20 PCs at m = 4096 runs
-// 0.80 -> 0.55 s per step).  GGP_CLUSTER=<n> overrides (developer experiments).
+// 0.80 -> 0.55 s per step).  GGP_CLUSTER=<n> overrides it, so that one input can run on both sides of the choice (tests).
 inline int choose_cluster(long long ntasks, int Mp)
 {
     if (const char* e = getenv("GGP_CLUSTER")) {
@@ -1373,7 +1100,7 @@ inline int choose_cluster(long long ntasks, int Mp)
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const long long slots = (long long)sms * GGP_CL_CTAS_PER_SM;      // resident CTAs of the cluster kernels
+    const long long slots = (long long)sms * CL_CTAS_PER_SM;      // resident CTAs of the cluster kernels
     const int gmax = (Mp >= 1024) ? 16 : 8;
     int g = 1;
     while (g < gmax && ntasks * (g * 2) <= slots) g *= 2;

@@ -29,17 +29,10 @@ int cuda_fail(cudaError_t e, const char* what);
     } while (0)
 
 constexpr int NB = 32;          // panel width of the blocked factorisation
-#ifndef GGP_NT
-#define GGP_NT 128
-#endif
-constexpr int NT = GGP_NT;      // threads per CTA of the fused kernels
+constexpr int NT = 128;         // threads per CTA of the fused kernels
 constexpr int NWARP = NT / 32;
-#ifndef GGP_CTAS_PER_SM
-#define GGP_CTAS_PER_SM 4     // 4 warps x 4 CTAs per SM, 128 registers per thread (tools/quick_bench.py sweep)
-#endif
-#ifndef GGP_CL_CTAS_PER_SM
-#define GGP_CL_CTAS_PER_SM 3  // cluster variant (few matrices in flight): 168 registers per thread, no spills
-#endif
+constexpr int CTAS_PER_SM = 4;     // 4 warps x 4 CTAs per SM, 128 registers per thread (tools/quick_bench.py sweep)
+constexpr int CL_CTAS_PER_SM = 3;  // cluster variant (few matrices in flight): 168 registers per thread, no spills
 constexpr int D_LD = 33;        // staging of the 32x32 diagonal block
 constexpr int MI_LD = 40;       // leading dimension of the inverted diagonal block (conflict-free LDS.128)
 constexpr int LT_LD = 34;       // leading dimension of the transposed diagonal factor (even: 16 B pairs)

@@ -1,6 +1,5 @@
 // Covariance build, cross-covariance and batched fused log-likelihood entry points.
 // C-ABI declared in include/gladsgp_b200.h.
-#include <cstdlib>
 #include "ggp_chol.cuh"
 #include "../../include/gladsgp_b200.h"
 
@@ -307,10 +306,10 @@ cross_cov_kernel(const double* __restrict__ X, int m, const double* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------
-// (2) batched fused log-likelihood: one CTA per matrix.
+// (2) batched fused log-likelihood: one CTA (look-ahead schedule) or one thread-block cluster (CL) per matrix.
 // ---------------------------------------------------------------------------------------------
-template <bool CL, bool LA = false, int RA = GGP_RA>
-__global__ void __launch_bounds__(NT, CL ? GGP_CL_CTAS_PER_SM : GGP_CTAS_PER_SM)
+template <bool CL>
+__global__ void __launch_bounds__(NT, CL ? CL_CTAS_PER_SM : CTAS_PER_SM)
 loglik_batched_kernel(const double* __restrict__ X, int m, int Mp, int d, const double* __restrict__ W,
                       long long w_stride, const double* __restrict__ beta, const double* __restrict__ lamz,
                       const double* __restrict__ diag_add, double* __restrict__ Lws, long long l_stride,
@@ -319,17 +318,17 @@ loglik_batched_kernel(const double* __restrict__ X, int m, int Mp, int d, const 
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int b = CL ? blockIdx.x / cluster_nctarank() : blockIdx.x;
     double ll;
-    if constexpr (LA) {
+    if constexpr (CL) {
+        EvalSmem sm = carve_eval_smem(smem_raw, Mp, d);
+        ll = eval_block_loglik<true>(sm, X, m, Mp, d, beta + (size_t)b * d, lamz[b], diag_add[b],
+                                     W + (size_t)b * w_stride, Lws + (size_t)b * l_stride,
+                                     u_out ? u_out + (size_t)b * Mp : nullptr, info ? info + b : nullptr);
+    } else {
         LaSmem sm = carve_la_smem(smem_raw, Mp, d);
         const int rot = cta_role_rotation();
         ll = eval_block_loglik_la(sm, X, m, Mp, d, beta + (size_t)b * d, lamz[b], diag_add[b],
                                   W + (size_t)b * w_stride, Lws + (size_t)b * l_stride,
                                   u_out ? u_out + (size_t)b * Mp : nullptr, info ? info + b : nullptr, rot);
-    } else {
-        EvalSmem sm = carve_eval_smem(smem_raw, Mp, d);
-        ll = eval_block_loglik<CL, RA>(sm, X, m, Mp, d, beta + (size_t)b * d, lamz[b], diag_add[b],
-                                   W + (size_t)b * w_stride, Lws + (size_t)b * l_stride,
-                                   u_out ? u_out + (size_t)b * Mp : nullptr, info ? info + b : nullptr);
     }
     if (threadIdx.x == 0 && (!CL || cluster_ctarank() == 0)) loglik[b] = ll;
 }
@@ -384,9 +383,8 @@ int ggp_cov_build_f64(const double* X, int m, int d, const double* beta, const d
         GGP_CUDA(cudaGetLastError());
         return GGP_OK;
     };
-    // whole 64-row blocks and an aligned output: the row-block kernel (GGP_COVROWS=0 keeps the tile kernel)
-    const char* env_rows = getenv("GGP_COVROWS");
-    if (m % CT == 0 && (reinterpret_cast<uintptr_t>(C_out) & 15) == 0 && !(env_rows && atoi(env_rows) == 0)) {
+    // whole 64-row blocks and a 16-byte aligned output: the row-block kernel
+    if (m % CT == 0 && (reinterpret_cast<uintptr_t>(C_out) & 15) == 0) {
         const size_t smem_r = (size_t)(3 * CT * 4 * cov_ksteps(d) + ETAB + d) * sizeof(double);
         auto run_rows = [&](auto kern) -> int {
             GGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
@@ -445,33 +443,6 @@ int ggp_cross_cov_f64(const double* X, int m, const double* Xp, int n, int d, co
     }
 }
 
-#ifdef GGP_PHASES
-int ggp_debug_phase_cycles(unsigned long long* out_host, int reset)
-{
-    unsigned long long z[32] = {0};
-    GGP_CUDA(cudaDeviceSynchronize());
-    GGP_CUDA(cudaMemcpyFromSymbol(out_host, ggp::g_phase, sizeof(z)));
-    if (reset) GGP_CUDA(cudaMemcpyToSymbol(ggp::g_phase, z, sizeof(z)));
-    return GGP_OK;
-}
-int ggp_debug_stage_cycles(unsigned long long* out_host, int reset)
-{
-    static unsigned long long z[4 * 64 * 2];
-    GGP_CUDA(cudaDeviceSynchronize());
-    GGP_CUDA(cudaMemcpyFromSymbol(out_host, ggp::g_stage, sizeof(z)));
-    if (reset) { memset(z, 0, sizeof(z)); GGP_CUDA(cudaMemcpyToSymbol(ggp::g_stage, z, sizeof(z))); }
-    return GGP_OK;
-}
-int ggp_debug_phase2_cycles(unsigned long long* out_host, int reset)
-{
-    unsigned long long z[128] = {0};
-    GGP_CUDA(cudaDeviceSynchronize());
-    GGP_CUDA(cudaMemcpyFromSymbol(out_host, ggp::g_phase2, sizeof(z)));
-    if (reset) GGP_CUDA(cudaMemcpyToSymbol(ggp::g_phase2, z, sizeof(z)));
-    return GGP_OK;
-}
-#endif
-
 int ggp_debug_exp_neg_f64(const double* y, double* out, int n, void* stream)
 {
     GGP_ARG(y && out && n > 0, "bad argument");
@@ -482,13 +453,6 @@ int ggp_debug_exp_neg_f64(const double* y, double* out, int n, void* stream)
 
 long long ggp_factor_doubles(int m) { return packed_doubles(round_up32(m)); }
 
-int ggp_set_lookahead(int on)
-{
-    const int old = lookahead_flag();
-    lookahead_flag() = on ? 1 : 0;
-    return old;
-}
-
 int ggp_padded_m(int m) { return round_up32(m); }
 
 int ggp_loglik_batched_f64(const double* X, int m, int d, const double* W, long long w_stride,
@@ -498,40 +462,30 @@ int ggp_loglik_batched_f64(const double* X, int m, int d, const double* W, long 
     GGP_ARG(X && W && beta && lamz && diag_add && factor_ws && loglik_out, "null pointer");
     GGP_ARG(m > 0 && d > 0 && B > 0, "m, d, B must be positive");
     const int Mp = round_up32(m);
-    size_t smem = eval_smem_bytes(Mp, d);
+    const size_t smem = eval_smem_bytes(Mp, d);
     if (smem > 227 * 1024) {
         set_error("ggp_loglik_batched_f64: m=%d d=%d needs %zu B of shared memory (> 227 KB)", m, d, smem);
         return GGP_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    int G = choose_cluster(B, round_up32(m));
+    const int G = choose_cluster(B, round_up32(m));
     const long long ls = packed_doubles(Mp);
     if (G > 1) {
-        auto run = [&](auto kern) -> int {
-            GGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const int Gc = checked_cluster(kern, G, smem);
-            GGP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, eval_carveout_pct(smem)));
-            GGP_CUDA(launch_maybe_cluster(kern, dim3(B * Gc), dim3(NT), smem, st, Gc, X, m, Mp, d, W, w_stride,
-                                          beta, lamz, diag_add, factor_ws, ls, u_out, loglik_out, info_out));
-            return GGP_OK;
-        };
-        const int rc = (Mp <= 1024) ? run(loglik_batched_kernel<true, false, 4>) : run(loglik_batched_kernel<true, false, 2>);
-        if (rc != GGP_OK) return rc;
-    } else if (use_lookahead()) {
+        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const int Gc = checked_cluster(loglik_batched_kernel<true>, G, smem);
+        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, eval_carveout_pct(smem)));
+        GGP_CUDA(launch_maybe_cluster(loglik_batched_kernel<true>, dim3(B * Gc), dim3(NT), smem, st, Gc, X, m, Mp, d, W, w_stride,
+                                      beta, lamz, diag_add, factor_ws, ls, u_out, loglik_out, info_out));
+    } else {
         const size_t sla = la_smem_bytes(Mp, d);
         if (sla > 227 * 1024) {
             set_error("ggp_loglik_batched_f64: m=%d d=%d needs %zu B of shared memory (> 227 KB)", m, d, sla);
             return GGP_ERR_UNSUPPORTED;
         }
-        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sla));
-        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, eval_carveout_pct(sla)));
-        loglik_batched_kernel<false, true><<<B, NT, sla, st>>>(X, m, Mp, d, W, w_stride, beta, lamz, diag_add, factor_ws, ls, u_out,
-                                                               loglik_out, info_out);
-    } else {
-        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, eval_carveout_pct(smem)));
-        loglik_batched_kernel<false><<<B, NT, smem, st>>>(X, m, Mp, d, W, w_stride, beta, lamz, diag_add, factor_ws, ls, u_out,
-                                                          loglik_out, info_out);
+        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sla));
+        GGP_CUDA(cudaFuncSetAttribute(loglik_batched_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, eval_carveout_pct(sla)));
+        loglik_batched_kernel<false><<<B, NT, sla, st>>>(X, m, Mp, d, W, w_stride, beta, lamz, diag_add, factor_ws, ls, u_out,
+                                                         loglik_out, info_out);
     }
     GGP_CUDA(cudaGetLastError());
     return GGP_OK;

@@ -156,15 +156,7 @@ __device__ inline void gather_block_params(const ggp_mcmc_args& a, const double*
 // budget with the loop's live state (a dozen pointers and indices) and spilled in the DMMA loops; as a function of its own
 // it gets the whole budget (the caller's few live values are saved once per evaluation), as in the batched log-likelihood
 // kernel.  (The cluster variant, 168 registers, has no spills when inlined and gets them as a function: it stays inline.)
-#ifndef GGP_EVAL_INLINE
-#define GGP_EVAL_INLINE 0
-#endif
-#if GGP_EVAL_INLINE
-#define GGP_EVAL_ATTR __forceinline__
-#else
-#define GGP_EVAL_ATTR __noinline__
-#endif
-static __device__ GGP_EVAL_ATTR double eval_la_call(unsigned char* smem_raw, const double* __restrict__ X, int m, int Mp, int d,
+static __device__ __noinline__ double eval_la_call(unsigned char* smem_raw, const double* __restrict__ X, int m, int Mp, int d,
                                                     const double* beta, double lamz, double diag_add,
                                                     const double* __restrict__ w, double* __restrict__ Lp, int rot)
 {
@@ -172,17 +164,17 @@ static __device__ GGP_EVAL_ATTR double eval_la_call(unsigned char* smem_raw, con
     return eval_block_loglik_la(sm, X, m, Mp, d, beta, lamz, diag_add, w, Lp, nullptr, nullptr, rot);
 }
 
-// one evaluation by the CTA (cluster): CL = cluster variant, LA = look-ahead variant (one CTA per matrix)
-template <bool CL, bool LA, int RA>
+// one evaluation by the CTA (cluster): CL = cluster variant, otherwise the look-ahead variant (one CTA per matrix)
+template <bool CL>
 static __device__ __forceinline__ double eval_dispatch(unsigned char* smem_raw, const double* __restrict__ X, int m, int Mp, int d,
                                                        const double* beta, double lamz, double diag_add,
                                                        const double* __restrict__ w, double* __restrict__ Lp, int rot = 0)
 {
-    if constexpr (LA) {
-        return eval_la_call(smem_raw, X, m, Mp, d, beta, lamz, diag_add, w, Lp, rot);
-    } else {
+    if constexpr (CL) {
         EvalSmem sm = carve_eval_smem(smem_raw, Mp, d);
-        return eval_block_loglik<CL, RA>(sm, X, m, Mp, d, beta, lamz, diag_add, w, Lp, nullptr, nullptr);
+        return eval_block_loglik<true>(sm, X, m, Mp, d, beta, lamz, diag_add, w, Lp, nullptr, nullptr);
+    } else {
+        return eval_la_call(smem_raw, X, m, Mp, d, beta, lamz, diag_add, w, Lp, rot);
     }
 }
 
@@ -236,8 +228,8 @@ __device__ inline void finalize_chain(const ggp_mcmc_args& a, const Plan& pl, co
 }
 
 // One mcmc_step of every chain in one launch (see the header of this file).
-template <bool CL, bool LA = false, int RA = GGP_RA>
-__global__ void __launch_bounds__(NT, CL ? GGP_CL_CTAS_PER_SM : GGP_CTAS_PER_SM)
+template <bool CL>
+__global__ void __launch_bounds__(NT, CL ? CL_CTAS_PER_SM : CTAS_PER_SM)
 sweep_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_stride, double* __restrict__ sig_cand,
              unsigned* __restrict__ arrive, int t)
 {
@@ -252,7 +244,7 @@ sweep_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_str
     double* Lp = Lws + ((size_t)c * pu + j) * l_stride;
     const double* wj = chain_w(a, c, j);
     unsigned char* accd = a.accepted ? a.accepted + ((size_t)t * a.n_chains + c) * P : nullptr;
-    const int rot = LA ? cta_role_rotation() : 0;
+    const int rot = CL ? 0 : cta_role_rotation();
     const bool shard = a.pc_count > 0;                         // PC shard: results leave through a.xchg, no close here
     double* xrow = shard ? a.xchg + ((size_t)j * a.n_chains + c) * (2 * d + 6) : nullptr;
     if (shard && lead) {
@@ -281,7 +273,7 @@ sweep_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_str
         __syncthreads();
         gather_block_params(a, th, c, j, s, cand, beta_sm, lamz, diag_add);
         __syncthreads();
-        const double ll_new = eval_dispatch<CL, LA, RA>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, wj, Lp, rot);
+        const double ll_new = eval_dispatch<CL>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, wj, Lp, rot);
         if (lead) {
             if (a.eval_count) atomicAdd(a.eval_count + (wos ? 1 : 0), 1ULL);
             if (wos) {
@@ -374,8 +366,7 @@ struct SpecWs {
     double* Lws;        // [n_chains][pu][3] factor workspaces
 };
 
-template <int RA>
-__global__ void __launch_bounds__(NT, GGP_CL_CTAS_PER_SM)
+__global__ void __launch_bounds__(NT, CL_CTAS_PER_SM)
 sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, double* __restrict__ sig_cand,
                   unsigned* __restrict__ arrive, int t, unsigned round_base)
 {
@@ -456,7 +447,7 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
             else if (lane_id == 1) gather_spec(a, st, lamwos_cur, c, j, e0, c0, e1, c1, nacc, ncand, e1, beta_sm, lamz, diag_add);
             else gather_spec(a, st, lamwos_cur, c, j, e1, c1, -1, 0.0, nacc, ncand, e1, beta_sm, lamz, diag_add);
             __syncthreads();
-            ll = eval_dispatch<true, false, RA>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, wj, Lp, 0);
+            ll = eval_dispatch<true>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, wj, Lp, 0);
         }
         if (lead) {
             if (work && a.eval_count) atomicAdd(a.eval_count, 1ULL);
@@ -532,8 +523,8 @@ sweep_spec_kernel(ggp_mcmc_args a, Plan pl, SpecWs sw, long long l_stride, doubl
 }
 
 // mode 0: sigwl <- per-PC terms of the current state.  mode 1: sigwl_cand <- terms under candidate lamWOs.
-template <bool CL, bool LA = false, int RA = GGP_RA>
-__global__ void __launch_bounds__(NT, CL ? GGP_CL_CTAS_PER_SM : GGP_CTAS_PER_SM)
+template <bool CL>
+__global__ void __launch_bounds__(NT, CL ? CL_CTAS_PER_SM : CTAS_PER_SM)
 eval_all_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_stride,
                 double* __restrict__ sig_cand, int mode)
 {
@@ -553,10 +544,10 @@ eval_all_kernel(ggp_mcmc_args a, Plan pl, double* __restrict__ Lws, long long l_
         cand = pl.cand[o];
     }
     double lamz, diag_add;
-    const int rot = LA ? cta_role_rotation() : 0;
+    const int rot = CL ? 0 : cta_role_rotation();
     gather_block_params(a, th, c, j, site, cand, beta_sm, lamz, diag_add);
     __syncthreads();
-    const double ll = eval_dispatch<CL, LA, RA>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, chain_w(a, c, j), Lp, rot);
+    const double ll = eval_dispatch<CL>(smem_raw, a.X, a.m, Mp, d, beta_sm, lamz, diag_add, chain_w(a, c, j), Lp, rot);
     if (threadIdx.x == 0 && (!CL || cluster_ctarank() == 0)) {
         if (mode == 0) a.sigwl[(size_t)c * pu + j] = ll;
         else sig_cand[(size_t)c * pu + j] = ll;
@@ -707,15 +698,13 @@ int ggp_mcmc_run_f64(const ggp_mcmc_args* args, void* stream)
     const int Mp = round_up32(a.m);
     int G = choose_cluster((long long)a.pu * a.n_chains, round_up32(a.m));
     int Gs = 0;                                    // cluster size of the speculative step kernel (0: not used)
-    const bool la = (G == 1) && use_lookahead();
-    const size_t smem = la ? la_smem_bytes(Mp, a.d) : eval_smem_bytes(Mp, a.d);
+    const size_t smem = (G > 1) ? eval_smem_bytes(Mp, a.d) : la_smem_bytes(Mp, a.d);
     if (smem > 227 * 1024) {
         set_error("ggp_mcmc_run_f64: m=%d d=%d needs %zu B of shared memory (> 227 KB)", a.m, a.d, smem);
         return GGP_ERR_UNSUPPORTED;
     }
     cudaStream_t st = (cudaStream_t)stream;
     const int cpct = eval_carveout_pct(smem);
-    const bool deep = Mp <= 1024;          // cluster kernels: A-fragment ring depth 4 (see eval_block_loglik)
     if (G > 1) {
         auto prep = [&](auto sweep, auto evall) -> int {
             GGP_CUDA(cudaFuncSetAttribute(sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -726,8 +715,7 @@ int ggp_mcmc_run_f64(const ggp_mcmc_args* args, void* stream)
             G = checked_cluster(evall, G, smem);
             return GGP_OK;
         };
-        const int rc = deep ? prep(sweep_kernel<true, false, 4>, eval_all_kernel<true, false, 4>)
-                            : prep(sweep_kernel<true, false, 2>, eval_all_kernel<true, false, 2>);
+        const int rc = prep(sweep_kernel<true>, eval_all_kernel<true>);
         if (rc != GGP_OK) return rc;
         // speculative step kernel: three clusters per (PC, chain), every one of them resident at the same time
         const int npc = a.pc_count > 0 ? a.pc_count : a.pu;                 // PCs swept by this call
@@ -751,14 +739,9 @@ int ggp_mcmc_run_f64(const ggp_mcmc_args* args, void* stream)
                 }
                 return GGP_OK;
             };
-            const int rs = deep ? prep_spec(sweep_spec_kernel<4>) : prep_spec(sweep_spec_kernel<2>);
+            const int rs = prep_spec(sweep_spec_kernel);
             if (rs != GGP_OK) return rs;
         }
-    } else if (la) {
-        GGP_CUDA(cudaFuncSetAttribute(sweep_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GGP_CUDA(cudaFuncSetAttribute(sweep_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cpct));
-        GGP_CUDA(cudaFuncSetAttribute(eval_all_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        GGP_CUDA(cudaFuncSetAttribute(eval_all_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cpct));
     } else {
         GGP_CUDA(cudaFuncSetAttribute(sweep_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         GGP_CUDA(cudaFuncSetAttribute(sweep_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cpct));
@@ -778,10 +761,8 @@ int ggp_mcmc_run_f64(const ggp_mcmc_args* args, void* stream)
     const int cb = (a.n_chains + 31) / 32;
 
     auto launch_eval_all = [&](int mode) -> cudaError_t {
-        if (G > 1) return deep ? launch_maybe_cluster(eval_all_kernel<true, false, 4>, grid_all, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, mode)
-                               : launch_maybe_cluster(eval_all_kernel<true, false, 2>, grid_all, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, mode);
-        if (la) eval_all_kernel<false, true><<<grid_all, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, mode);
-        else eval_all_kernel<false><<<grid_all, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, mode);
+        if (G > 1) return launch_maybe_cluster(eval_all_kernel<true>, grid_all, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, mode);
+        eval_all_kernel<false><<<grid_all, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, mode);
         return cudaGetLastError();
     };
     const SpecWs specws = wsp.spec;
@@ -790,13 +771,10 @@ int ggp_mcmc_run_f64(const ggp_mcmc_args* args, void* stream)
         if (Gs > 0) {
             const dim3 gs(SPEC_LANES * (a.pc_count > 0 ? a.pc_count : a.pu) * Gs, a.n_chains);
             const unsigned base = (unsigned)(tbase >= 0 ? tbase : t) * (unsigned)rcap;   // rounds since the counters were zeroed
-            return deep ? launch_maybe_cluster(sweep_spec_kernel<4>, gs, dim3(NT), smem, st, Gs, a, pl, specws, l_stride, sig_cand, arrive, t, base)
-                        : launch_maybe_cluster(sweep_spec_kernel<2>, gs, dim3(NT), smem, st, Gs, a, pl, specws, l_stride, sig_cand, arrive, t, base);
+            return launch_maybe_cluster(sweep_spec_kernel, gs, dim3(NT), smem, st, Gs, a, pl, specws, l_stride, sig_cand, arrive, t, base);
         }
-        if (G > 1) return deep ? launch_maybe_cluster(sweep_kernel<true, false, 4>, grid, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, arrive, t)
-                               : launch_maybe_cluster(sweep_kernel<true, false, 2>, grid, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, arrive, t);
-        if (la) sweep_kernel<false, true><<<grid, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, arrive, t);
-        else sweep_kernel<false><<<grid, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, arrive, t);
+        if (G > 1) return launch_maybe_cluster(sweep_kernel<true>, grid, dim3(NT), smem, st, G, a, pl, Lws, l_stride, sig_cand, arrive, t);
+        sweep_kernel<false><<<grid, NT, smem, st>>>(a, pl, Lws, l_stride, sig_cand, arrive, t);
         return cudaGetLastError();
     };
     if (a.init_sigwl) GGP_CUDA(launch_eval_all(0));

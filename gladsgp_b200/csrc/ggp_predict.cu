@@ -509,14 +509,14 @@ static int launch_reconstruct(const float* w, const float* K, const float* sd, i
 // One CTA per block; the factorisation is eval_block_loglik's (DMMA left-looking panels, packed factor as scratch) with
 // the matrix entries read from memory instead of generated, and a product in place of the forward solve.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(NT, GGP_CTAS_PER_SM)
+__global__ void __launch_bounds__(NT, CTAS_PER_SM)
 chol_draw_kernel(const double* __restrict__ Sigma, int n, int Mp, const double* __restrict__ z, double* __restrict__ Lws,
                  long long l_stride, double* __restrict__ dev, int* __restrict__ info, int b0)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const size_t b = (size_t)b0 + blockIdx.x;
     EvalSmem sm = carve_eval_smem(smem_raw, Mp, 0);
-    eval_block_loglik<false, GGP_RA, 1>(sm, Sigma + b * n * n, n, Mp, 0, nullptr, 1.0, 0.0, z + b * n,
+    eval_block_loglik<false, 1>(sm, Sigma + b * n * n, n, Mp, 0, nullptr, 1.0, 0.0, z + b * n,
                                         Lws + (size_t)blockIdx.x * l_stride, dev + b * n, info + b);
 }
 

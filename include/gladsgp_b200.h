@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define GGP_VERSION 201
+#define GGP_VERSION 202
 
 int ggp_version(void);
 const char* ggp_last_error_string(void);
@@ -49,14 +49,12 @@ int ggp_cross_cov_f64(const double* X, int m, const double* Xp, int n, int d, co
  * reference maps a failed Cholesky to -inf the same way).
  * W: vector b starts at W + b*w_stride.  factor_ws[B][ggp_factor_doubles(m)] receives the packed
  * factor (layout in DESIGN.md; unpack with ggp_factor_unpack_f64).  u_out (nullable)
- * [B][ggp_padded_m(m)] receives L^-1 W[b], zero padded.  info_out nullable. */
+ * [B][ggp_padded_m(m)] receives L^-1 W[b], zero padded.  info_out nullable.  A matrix runs on one CTA
+ * (look-ahead schedule) or on a thread-block cluster, chosen from B and m: both give bit-identical results. */
 /* test hook: out[i] = exp(y[i]) for y <= 0 with the kernel-internal exponential (about 1 ulp) */
 int ggp_debug_exp_neg_f64(const double* y, double* out, int n, void* stream);
 long long ggp_factor_doubles(int m);
 int ggp_padded_m(int m);
-/* one-CTA-per-matrix evaluations use the look-ahead schedule (default 1; GGP_LOOKAHEAD=0 in the environment turns it
- * off): both schedules and the cluster variant give bit-identical results.  Returns the previous setting. */
-int ggp_set_lookahead(int on);
 int ggp_loglik_batched_f64(const double* X, int m, int d, const double* W, long long w_stride,
                            const double* beta, const double* lamz, const double* diag_add, int B,
                            double* factor_ws, double* u_out, double* loglik_out, int* info_out, void* stream);

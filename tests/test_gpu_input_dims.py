@@ -71,31 +71,24 @@ def test_cov_build_and_cross_cov_every_distance_path(cuda, d, m):
 
 
 @pytest.mark.parametrize('d', DIMS)
-def test_loglik_every_distance_path_in_every_schedule(cuda, monkeypatch, d):
+def test_loglik_every_distance_path_in_both_schedules(cuda, monkeypatch, d):
     """m = 257 (ragged last panel): log-likelihood against SciPy, u and the factor against the dense solve, and the
-    look-ahead, plain and cluster schedules bit for bit."""
-    from gladsgp_b200 import ops, _lib
-    h = _lib.load()
+    look-ahead and cluster schedules bit for bit."""
+    from gladsgp_b200 import ops
     m, B = 257, 2
     rng = np.random.default_rng(d)
     X = rng.uniform(0, 1, size=(m, d))
     W = rng.standard_normal((B, m))
     beta, lamz, dadd = _hypers(d, B, seed=d + 1)
     res = {}
-    old = h.ggp_set_lookahead(1)
-    try:
-        for key, g, la in (('la', '1', 1), ('plain', '1', 0), ('cluster', '4', 0)):
-            monkeypatch.setenv('GGP_CLUSTER', g)
-            h.ggp_set_lookahead(la)
-            out = ops.loglik_batched(X, W, beta, lamz, dadd, want_factor=True, want_u=True)
-            assert np.all(out['info'].cpu().numpy() == 0), key
-            res[key] = (out['loglik'].cpu().numpy(), ops.factor_unpack(out['factor'], m).cpu().numpy(),
-                        out['u'].cpu().numpy())
-    finally:
-        h.ggp_set_lookahead(old)
-    for key in ('plain', 'cluster'):
-        for a, b in zip(res['la'], res[key]):
-            assert np.array_equal(a, b), key
+    for key, g in (('la', '1'), ('cluster', '4')):
+        monkeypatch.setenv('GGP_CLUSTER', g)
+        out = ops.loglik_batched(X, W, beta, lamz, dadd, want_factor=True, want_u=True)
+        assert np.all(out['info'].cpu().numpy() == 0), key
+        res[key] = (out['loglik'].cpu().numpy(), ops.factor_unpack(out['factor'], m).cpu().numpy(),
+                    out['u'].cpu().numpy())
+    for a, b in zip(res['la'], res['cluster']):
+        assert np.array_equal(a, b)
     ll, Lg, ug = res['la']
     for b in range(B):
         L = scipy.linalg.cholesky(_dense_cov(X, beta[b], lamz[b], dadd[b]), lower=True)

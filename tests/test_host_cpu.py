@@ -152,7 +152,7 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), name
     assert sorted(_lib.SIGNATURES) == declared               # ctypes table mirrors the header one to one
     h = _lib.load()
-    assert h.ggp_version() == 201
+    assert h.ggp_version() == 202
     assert h.ggp_padded_m(100) == 128 and h.ggp_factor_doubles(512) == 139264 + 16 * 1024 + 512 + 64
     # argument validation happens before any CUDA call
     assert h.ggp_cov_build_f64(None, 4, 2, None, None, None, 1, None, None) == -1

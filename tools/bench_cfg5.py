@@ -12,7 +12,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gladsgp_b200 import synthetic, _lib  # noqa: E402
 if os.environ.get('GGP_LIB'):                      # developer A/B runs against a variant library
     _lib.LIB_PATH = os.environ['GGP_LIB']
-    _lib.SIGNATURES.pop('ggp_set_lookahead', None)
 from sepia.SepiaData import SepiaData  # noqa: E402
 from sepia.SepiaModel import SepiaModel  # noqa: E402
 

@@ -1,8 +1,11 @@
-"""Developer timing of the materialised covariance build (592 matrices of 512 x 512, d = 9): tile kernel vs row-block kernel."""
+"""Developer timing of the materialised covariance build (592 matrices of 512 x 512, d = 9): tile kernel vs row-block kernel.
+
+m = 512 is a multiple of the 64-row block, so a 16-byte aligned output takes the row-block kernel; the same call on an output
+offset by 8 bytes takes the tile kernel.  Both results are compared bit for bit."""
 import json, os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from gladsgp_b200 import ops, synthetic
+from gladsgp_b200 import ops, synthetic, _lib
 m, q = 512, 8
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 592
 d = q + 1
@@ -12,6 +15,10 @@ rng = np.random.default_rng(0)
 beta = np.exp(rng.uniform(np.log(0.05), np.log(3.0), size=(B, d)))
 lamz = rng.uniform(0.5, 2.0, B); dadd = rng.uniform(1e-3, 1e-2, B)
 Xd, bd, ld, dd = [torch.as_tensor(a, device='cuda') for a in (X, beta, lamz, dadd)]
+lib = _lib.load()
+def cov_build_into(out):
+    _lib.check(lib.ggp_cov_build_f64(_lib.ptr(Xd), m, d, _lib.ptr(bd), _lib.ptr(ld), _lib.ptr(dd), B, _lib.ptr(out),
+                                     _lib.stream_ptr()), 'ggp_cov_build_f64')
 def ev(fn, reps=7):
     fn(); torch.cuda.synchronize(); best = 1e9
     for _ in range(reps):
@@ -20,10 +27,12 @@ def ev(fn, reps=7):
     return best
 res = {}
 outs = {}
-for mode in ('0', '1'):
-    os.environ['GGP_COVROWS'] = mode
-    outs[mode] = ops.cov_build(Xd, bd, ld, dd)
-    ms = ev(lambda: ops.cov_build(Xd, bd, ld, dd))
+buf = torch.empty(B * m * m + 2, dtype=torch.float64, device='cuda')
+for mode, off in (('0', 1), ('1', 0)):          # covrows0: tile kernel (8-byte offset output), covrows1: row-block kernel
+    out = buf[off:off + B * m * m]
+    assert (out.data_ptr() % 16 == 0) == (mode == '1')
+    ms = ev(lambda: cov_build_into(out))
+    outs[mode] = out.view(B, m, m).clone()
     res['covrows' + mode] = dict(ms=ms, gbs=B * m * m * 8 / ms / 1e6, frac=B * m * m * 8 / ms / 1e6 / 6533.8)
 res['identical'] = bool(torch.equal(outs['0'], outs['1']))
 res['symmetric'] = bool(torch.equal(outs['1'], outs['1'].transpose(1, 2)))

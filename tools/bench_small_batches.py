@@ -6,7 +6,6 @@ import bench
 from gladsgp_b200 import _lib
 if os.environ.get('GGP_LIB'):
     _lib.LIB_PATH = os.environ['GGP_LIB']
-    _lib.SIGNATURES.pop('ggp_set_lookahead', None)      # older variant libraries
 from gladsgp_b200 import svd, model as gmodel
 from sepia.SepiaData import SepiaData
 from sepia.SepiaModel import SepiaModel
