@@ -745,3 +745,37 @@ def main_effects(Z, beta, a, S, pu, grid, mode=0):
     check(_lib.load().ggp_main_effects_f64(ptr(Z), m, q, ptr(beta), ptr(a), S, pu, mode, ptr(g), g.numel(), ptr(out),
                                            ptr(ws), ws.numel(), stream_ptr()), 'ggp_main_effects_f64')
     return out
+
+
+def calib_loglik(mean, var, G, b, c0, want_per_sample=False):
+    """Calibration log-likelihood (csrc/ggp_calib.cu) at n points from the predictive moments mean, var (S*pu, n) of
+    ggp_predict_f64 and the observation terms G (S, pu, pu), b (S, pu), c0 (S,).  Returns ll (n,) [, ll_s (S, n)], float64
+    device tensors."""
+    torch = _lib.require_cuda()
+    mean = _f64(mean, torch, 'cuda'); var = _f64(var, torch, 'cuda')
+    G = _f64(G, torch, 'cuda'); b = _f64(b, torch, 'cuda'); c0 = _f64(c0, torch, 'cuda').reshape(-1)
+    S, pu = c0.numel(), G.shape[-1]
+    n = mean.shape[-1]
+    if G.numel() != S * pu * pu or b.numel() != S * pu:
+        raise ValueError('G, b, c0 must be (S, pu, pu), (S, pu), (S,)')
+    if tuple(mean.shape) != (S * pu, n) or tuple(var.shape) != (S * pu, n):
+        raise ValueError('mean and var must be (S * pu, n)')
+    ll = torch.empty(n, dtype=torch.float64, device='cuda')
+    ll_s = torch.empty((S, n), dtype=torch.float64, device='cuda') if want_per_sample else None
+    check(_lib.load().ggp_calib_loglik_f64(ptr(mean), ptr(var), S, pu, n, ptr(G), ptr(b), ptr(c0), ptr(ll), ptr(ll_s),
+                                           stream_ptr()), 'ggp_calib_loglik_f64')
+    return (ll, ll_s) if want_per_sample else ll
+
+
+def calib_step(mean, var, G, b, c0, Xp, lo, hi, L_prop, z_next, logu, theta, ll, rec_theta, rec_ll, rec_acc):
+    """One Metropolis step of C chains (csrc/ggp_calib.cu): the candidates are the last q columns of Xp (C, d), mean / var
+    (S*pu, C) their predictive moments.  Updates theta (C, q), ll (C) and, unless z_next is None, writes the next
+    candidates theta + L_prop z_next[c] into Xp; rec_theta (C, q), rec_ll (C), rec_acc (C) uint8 receive the step's record.
+    Every tensor argument but G, b, c0 must already be a contiguous CUDA tensor of the right dtype (this runs every step)."""
+    C, d = Xp.shape
+    q = theta.shape[1]
+    pu = G.shape[-1]
+    S = c0.numel()
+    check(_lib.load().ggp_calib_step_f64(ptr(mean), ptr(var), S, pu, C, ptr(G), ptr(b), ptr(c0), ptr(Xp), d, q, ptr(lo),
+                                         ptr(hi), ptr(L_prop), ptr(z_next), ptr(logu), ptr(theta), ptr(ll), ptr(rec_theta),
+                                         ptr(rec_ll), ptr(rec_acc), stream_ptr()), 'ggp_calib_step_f64')

@@ -264,6 +264,30 @@ int ggp_main_effects_f64(const double* Z, int m, int q, const double* beta, cons
                          const double* grid, int ngrid, double* out, void* workspace, long long workspace_bytes,
                          void* stream);
 
+/* ---- Emulator-based calibration (csrc/ggp_calib.cu; DESIGN.md section 2 item 9) ------------------------------------
+ * Log-likelihood of observed outputs at n input points, from the predictive moments of ggp_predict_f64 at the points'
+ * designs: mean, var (S pu, n), block s * pu + j (posterior sample s, PC j), var clamped at 0.  Per-sample observation
+ * terms, precomputed by the caller: G (S, pu, pu) symmetric = K_O D_s^-1 K_O^T, b (S, pu) = K_O D_s^-1 r and
+ * c0 (S) = r^T D_s^-1 r + sum log D_s,ii + n_o log 2 pi.  With A = I + V^1/2 G V^1/2, V = diag(var), h = b - G mu:
+ *   l_s = -1/2 (c0 - 2 mu^T b + mu^T G mu - h^T V^1/2 A^-1 V^1/2 h + log det A),
+ *   ll_out[p] = log((1/S) sum_s exp l_s)   (running maximum, s ascending),   ll_s_out[s][p] = l_s (nullable).
+ * Deterministic (fixed summation orders, no atomics).  GGP_ERR_ARG: a null pointer, S or n < 1, pu outside [1, 32],
+ * S pu >= 2^31. */
+int ggp_calib_loglik_f64(const double* mean, const double* var, int S, int pu, int n, const double* G, const double* b,
+                         const double* c0, double* ll_out, double* ll_s_out, void* stream);
+/* One Metropolis step of C chains on the uniform box [lo, hi] (q inputs, transformed units).  The candidate of chain c is
+ * the last q columns of Xp[c] (C, d), and mean / var are the output of ggp_predict_f64 on Xp issued before this call.
+ * valid = every candidate coordinate in [lo, hi] (inclusive); accept = valid && logu[c] < l' - ll[c] (false for a NaN
+ * l').  theta (C, q) and ll (C) are updated; rec_theta (C, q), rec_ll (C), rec_acc (C) receive the step's state, l and
+ * accepted flag.  If z_next (C, q) is not null, the next candidate theta + L_prop z_next[c] (L_prop (q, q) lower
+ * triangular, sums over k ascending) is written to the last q columns of Xp[c]; an input whose row and column of L_prop
+ * are zero keeps its value.  GGP_ERR_ARG: a null pointer (z_next may be null), S or C < 1, pu or q outside [1, 32],
+ * d < q, S pu >= 2^31. */
+int ggp_calib_step_f64(const double* mean, const double* var, int S, int pu, int C, const double* G, const double* b,
+                       const double* c0, double* Xp, int d, int q, const double* lo, const double* hi,
+                       const double* L_prop, const double* z_next, const double* logu, double* theta, double* ll,
+                       double* rec_theta, double* rec_ll, unsigned char* rec_acc, void* stream);
+
 /* ---- MCMC convergence diagnostics (csrc/ggp_chain_diag.cu; DESIGN.md section 2 "Chain diagnostics") ----------------
  * Rank-normalized split R-hat, bulk ESS and tail ESS of Vehtari et al. (2021), as ArviZ computes rhat(method="rank"),
  * ess(method="bulk") and ess(method="tail"), with the autocovariance as a direct sum.  Draw i of chain c of element e is
