@@ -75,6 +75,10 @@ SIGNATURES = {
     'ggp_main_effects_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _I, _P, _P, _LL, _P]),
     'ggp_calib_loglik_f64': (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
     'ggp_calib_step_f64': (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'ggp_design_workspace_bytes': (_LL, [_I, _I]),
+    'ggp_design_score_f64': (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P, _LL,
+                                  _P]),
+    'ggp_design_condition_f64': (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P]),
     'ggp_rsvd_tc_workspace_bytes': (_LL, [_I]),
     'ggp_rsvd_sketch_tc_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P, _LL, _P]),
     'ggp_rsvd_xty_tc_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P]),

@@ -26,12 +26,17 @@ STEP_CHUNK = 256              # steps whose proposal and acceptance draws are ge
 MAX_DIM = 32                  # pu and q limit of csrc/ggp_calib.cu
 
 
+def _check_t_model(model, what='calibration', verb='calibrate'):
+    """A model whose inputs are all in t (no x_sim) and that has at least one (shared with gladsgp_b200.design)."""
+    if not model.data.dummy_x:
+        raise ValueError('%s needs a model without x_sim (its inputs are all in t)' % what)
+    if model.num.q == 0:
+        raise ValueError('the model has no inputs to %s (q = 0)' % verb)
+
+
 def _check_model(model):
     num = model.num
-    if not model.data.dummy_x:
-        raise ValueError('calibration needs a model without x_sim (its inputs are all in t)')
-    if num.q == 0:
-        raise ValueError('the model has no inputs to calibrate (q = 0)')
+    _check_t_model(model)
     if num.pu > MAX_DIM or num.q > MAX_DIM:
         raise ValueError('calibration supports pu <= %d and q <= %d (got pu = %d, q = %d)' % (MAX_DIM, MAX_DIM, num.pu, num.q))
     return num.q, num.pu

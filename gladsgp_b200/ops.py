@@ -313,25 +313,27 @@ class Predictor:
         self.lamz = _f64(lamz, torch, dev).reshape(-1)
         self.s11 = _f64(s11_diag, torch, dev).reshape(-1)
         self.W = _f64(W, torch, dev).reshape(self.B, self.m)          # training weights: the means of cross-validation
+        self.dadd = _f64(diag_add, torch, dev).reshape(-1)              # the S22 nugget (sequential design's Schur complement)
         out = loglik_batched(self.X, self.W, self.beta, self.lamz, diag_add, want_factor=True, want_u=True)
         self.factor, self.u, self.loglik, self.info = out['factor'], out['u'], out['loglik'], out['info']
         self.Mp = self.u.shape[1]
         self._ws = None
         self._xws = None
 
-    def predict(self, Xp, want_V=False):
-        """Xp (n,d) -> mean (B,n), var (B,n)[, V (B,n,Mp)]."""
+    def predict(self, Xp, want_V=False, b0=0, nb=None):
+        """Xp (n,d) -> mean (nb,n), var (nb,n)[, V (nb,n,Mp)] of blocks [b0, b0+nb) (default: all B)."""
         torch, lib, dev = self.torch, self.lib, 'cuda'
         Xp = _f64(Xp, torch, dev)
         n = Xp.shape[0]
-        need = lib.ggp_predict_workspace_bytes(self.m, n, self.B)
+        nb = self.B - b0 if nb is None else nb
+        need = lib.ggp_predict_workspace_bytes(self.m, n, nb)
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=dev)
-        mean = torch.empty((self.B, n), dtype=torch.float64, device=dev)
-        var = torch.empty((self.B, n), dtype=torch.float64, device=dev)
-        V = torch.empty((self.B, n, self.Mp), dtype=torch.float64, device=dev) if want_V else None
-        check(lib.ggp_predict_f64(ptr(self.X), self.m, self.d, ptr(self.factor), ptr(self.u), ptr(self.beta),
-                                  ptr(self.lamz), ptr(self.s11), ptr(Xp), n, self.B, ptr(mean), ptr(var), ptr(V),
+        mean = torch.empty((nb, n), dtype=torch.float64, device=dev)
+        var = torch.empty((nb, n), dtype=torch.float64, device=dev)
+        V = torch.empty((nb, n, self.Mp), dtype=torch.float64, device=dev) if want_V else None
+        check(lib.ggp_predict_f64(ptr(self.X), self.m, self.d, ptr(self.factor[b0:]), ptr(self.u[b0:]), ptr(self.beta[b0:]),
+                                  ptr(self.lamz[b0:]), ptr(self.s11[b0:]), ptr(Xp), n, nb, ptr(mean), ptr(var), ptr(V),
                                   ptr(self._ws), self._ws.numel(), stream_ptr()), 'ggp_predict_f64')
         return (mean, var, V) if want_V else (mean, var)
 
@@ -779,3 +781,38 @@ def calib_step(mean, var, G, b, c0, Xp, lo, hi, L_prop, z_next, logu, theta, ll,
     check(_lib.load().ggp_calib_step_f64(ptr(mean), ptr(var), S, pu, C, ptr(G), ptr(b), ptr(c0), ptr(Xp), d, q, ptr(lo),
                                          ptr(hi), ptr(L_prop), ptr(z_next), ptr(logu), ptr(theta), ptr(ll), ptr(rec_theta),
                                          ptr(rec_ll), ptr(rec_acc), stream_ptr()), 'ggp_calib_step_f64')
+
+
+def _design_blocks(pred, b0, nb):
+    return (ptr(pred.beta[b0:]), ptr(pred.lamz[b0:]), ptr(pred.dadd[b0:]))
+
+
+def design_score(pred, b0, XR, XC, V_R, V_C, A_R, A_C, t, wgt, score, imse, accumulate, ws=None):
+    """ALC scores of greedy sequential design (csrc/ggp_design.cu) on blocks [b0, b0+nb) of a Predictor, nb = V_C.shape[0]:
+    score (n_cand,) and imse (1,) receive (or, with accumulate, add in block order) sum_b wgt[b] sum_r Sigma_t(r, c)^2 /
+    den_t(c) and sum_b wgt[b] sum_r v_t(r).  XR (n_ref, d), XC (n_cand, d) designs; V_R (nb, n_ref, Mp), V_C (nb, n_cand,
+    Mp) from pred.predict(..., want_V=True, b0=b0, nb=nb); A_R (nb, n_ref, Kp), A_C (nb, n_cand, Kp) with t columns in use;
+    wgt (nb,).  score may be None (imse only).  Every tensor must be a contiguous float64 CUDA tensor.  Returns the
+    workspace (pass it back to reuse it)."""
+    torch, lib = pred.torch, pred.lib
+    nb, n_cand, _ = V_C.shape
+    n_ref = V_R.shape[1]
+    need = lib.ggp_design_workspace_bytes(n_cand, nb)
+    if ws is None or ws.numel() < need:
+        ws = torch.empty(max(need, 1), dtype=torch.uint8, device='cuda')
+    be, lz, da = _design_blocks(pred, b0, nb)
+    check(lib.ggp_design_score_f64(ptr(XR), n_ref, ptr(XC), n_cand, XC.shape[1], be, lz, da, ptr(pred.s11[b0:]), ptr(wgt),
+                                   ptr(V_R), ptr(V_C), pred.m, ptr(A_R), ptr(A_C), A_C.shape[2], int(t), nb, int(accumulate),
+                                   ptr(score), ptr(imse), ptr(ws), ws.numel(), stream_ptr()), 'ggp_design_score_f64')
+    return ws
+
+
+def design_condition(pred, b0, XR, XC, V_R, V_C, A_R, A_C, t, index):
+    """Append column t of A_R and A_C (csrc/ggp_design.cu) after choosing candidate `index`, on the blocks of design_score.
+    The same tensors for XR / XC, V_R / V_C and A_R / A_C mean the reference set is the candidate set."""
+    lib = pred.lib
+    nb, n_cand, _ = V_C.shape
+    be, lz, da = _design_blocks(pred, b0, nb)
+    check(lib.ggp_design_condition_f64(ptr(XR), V_R.shape[1], ptr(XC), n_cand, XC.shape[1], be, lz, da, ptr(V_R), ptr(V_C),
+                                       pred.m, ptr(A_R), ptr(A_C), A_C.shape[2], int(t), nb, int(index), stream_ptr()),
+          'ggp_design_condition_f64')

@@ -288,6 +288,32 @@ int ggp_calib_step_f64(const double* mean, const double* var, int S, int pu, int
                        const double* L_prop, const double* z_next, const double* logu, double* theta, double* ll,
                        double* rec_theta, double* rec_ll, unsigned char* rec_acc, void* stream);
 
+/* ---- Sequential design (csrc/ggp_design.cu; DESIGN.md section 2 item 10) --------------------------------------------
+ * Greedy ALC over B (sample, PC) blocks.  XR (n_ref, d) reference and XC (n_cand, d) candidate designs; beta (B, d),
+ * lamz, dadd (the S22 nugget), s11 (B); V_R (B, n_ref, Mp) and V_C (B, n_cand, Mp) as ggp_predict_f64 writes V
+ * (Mp = ggp_padded_m(m), zero padding); A_R (B, n_ref, Kp), A_C (B, n_cand, Kp): one column per chosen run, columns >= t
+ * zero; Kp a multiple of 8.  With k_b(x, x') = exp(-sum_k beta_bk (x_k - x'_k)^2) / lamz_b,
+ *   Sigma(r, c) = k_b(r, c) - V_r . V_c - A_r . A_c,   den(c) = 1/lamz_b + dadd_b - |V_c|^2 - |A_c|^2,
+ *   score_out[c] = start + sum_b wgt[b] sum_r Sigma(r, c)^2 / den(c),
+ *   imse_out[0]  = start + sum_b wgt[b] sum_r max(s11_b - |V_r|^2 - |A_r|^2, 0),
+ * blocks summed in ascending order; start is 0, or the output's value when accumulate != 0 (so a split of the blocks
+ * over several calls gives the same bits).  score_out may be null (imse only).  The product runs on the FP64 tensor
+ * cores, the n_ref x n_cand matrix is never stored.  workspace: ggp_design_workspace_bytes(n_cand, B).
+ * ggp_design_condition_f64 writes column t of A_R and A_C after choosing candidate `index`:
+ *   A_x[t] = (k_b(x, c*) - V_x . V_c* - A_x[0:t] . A_c*[0:t]) / sqrt(den(c*))   for every reference and candidate x.
+ * Passing the same XR / XC, V_R / V_C and A_R / A_C pointers (reference set = candidate set) conditions each point once.
+ * Deterministic.  GGP_ERR_ARG: a null pointer, a size <= 0, Kp not a multiple of 8, m > 8192, t outside [0, Kp] (score)
+ * or [0, Kp) (condition), index outside [0, n_cand), a short workspace. */
+long long ggp_design_workspace_bytes(int n_cand, int B);
+int ggp_design_score_f64(const double* XR, int n_ref, const double* XC, int n_cand, int d, const double* beta,
+                         const double* lamz, const double* dadd, const double* s11, const double* wgt, const double* V_R,
+                         const double* V_C, int m, const double* A_R, const double* A_C, int Kp, int t, int B,
+                         int accumulate, double* score_out, double* imse_out, void* workspace, long long workspace_bytes,
+                         void* stream);
+int ggp_design_condition_f64(const double* XR, int n_ref, const double* XC, int n_cand, int d, const double* beta,
+                             const double* lamz, const double* dadd, const double* V_R, const double* V_C, int m,
+                             double* A_R, double* A_C, int Kp, int t, int B, int index, void* stream);
+
 /* ---- MCMC convergence diagnostics (csrc/ggp_chain_diag.cu; DESIGN.md section 2 "Chain diagnostics") ----------------
  * Rank-normalized split R-hat, bulk ESS and tail ESS of Vehtari et al. (2021), as ArviZ computes rhat(method="rank"),
  * ess(method="bulk") and ess(method="tail"), with the autocovariance as a direct sum.  Draw i of chain c of element e is
