@@ -79,6 +79,8 @@ SIGNATURES = {
     'ggp_design_score_f64': (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P, _LL,
                                   _P]),
     'ggp_design_condition_f64': (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P]),
+    'ggp_hm_workspace_bytes': (_LL, [_I, _I, _I, _I]),
+    'ggp_hm_impl_f64': (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _I, _I, _D, _P, _P, _P, _LL, _P]),
     'ggp_rsvd_tc_workspace_bytes': (_LL, [_I]),
     'ggp_rsvd_sketch_tc_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P, _LL, _P]),
     'ggp_rsvd_xty_tc_f32': (_I, [_P, _I, _LL, _P, _I, _P, _P]),

@@ -816,3 +816,31 @@ def design_condition(pred, b0, XR, XC, V_R, V_C, A_R, A_C, t, index):
     check(lib.ggp_design_condition_f64(ptr(XR), V_R.shape[1], ptr(XC), n_cand, XC.shape[1], be, lz, da, ptr(V_R), ptr(V_C),
                                        pred.m, ptr(A_R), ptr(A_C), A_C.shape[2], int(t), nb, int(index), stream_ptr()),
           'ggp_design_condition_f64')
+
+
+def hm_impl(mean, var, K_O, r, c, order, cutoff):
+    """History-matching implausibility (csrc/ggp_hm.cu) at n points from the predictive moments mean, var (S*pu, n) of
+    ggp_predict_f64 and the observed outputs' K_O (pu, n_o), r (n_o,) and c (n_o,) = rho + tau^2 + delta^2 (standardized
+    units).  Returns impl (n, order) float64, the `order` largest I_i of each point in descending order, and n_over (n,)
+    int32, the number of outputs with I_i > cutoff, as CUDA tensors."""
+    torch = _lib.require_cuda()
+    mean = _f64(mean, torch, 'cuda'); var = _f64(var, torch, 'cuda')
+    K_O = _f64(K_O, torch, 'cuda'); r = _f64(r, torch, 'cuda').reshape(-1); c = _f64(c, torch, 'cuda').reshape(-1)
+    if K_O.dim() != 2:
+        raise ValueError('K_O must be (pu, n_o)')
+    pu, n_o = K_O.shape
+    if r.numel() != n_o or c.numel() != n_o:
+        raise ValueError('r and c must be (n_o,) = (%d,)' % n_o)
+    if mean.dim() != 2 or mean.shape[0] % pu != 0 or tuple(var.shape) != tuple(mean.shape):
+        raise ValueError('mean and var must be (S * pu, n) with pu = %d' % pu)
+    S, n = mean.shape[0] // pu, mean.shape[1]
+    lib = _lib.load()
+    need = lib.ggp_hm_workspace_bytes(n, n_o, pu, S)
+    if need < 0:
+        raise ValueError('hm_impl needs S, n, n_o >= 1 and 1 <= pu <= 32 (got S=%d, n=%d, n_o=%d, pu=%d)' % (S, n, n_o, pu))
+    ws = torch.empty(need, dtype=torch.uint8, device='cuda')
+    impl = torch.empty((n, int(order)), dtype=torch.float64, device='cuda')
+    n_over = torch.empty(n, dtype=torch.int32, device='cuda')
+    check(lib.ggp_hm_impl_f64(ptr(mean), ptr(var), S, pu, n, ptr(K_O), ptr(r), ptr(c), n_o, int(order), float(cutoff),
+                              ptr(impl), ptr(n_over), ptr(ws), ws.numel(), stream_ptr()), 'ggp_hm_impl_f64')
+    return impl, n_over

@@ -314,6 +314,23 @@ int ggp_design_condition_f64(const double* XR, int n_ref, const double* XC, int 
                              const double* lamz, const double* dadd, const double* V_R, const double* V_C, int m,
                              double* A_R, double* A_C, int Kp, int t, int B, int index, void* stream);
 
+/* ---- History matching (csrc/ggp_hm.cu; DESIGN.md section 2 item 11) -------------------------------------------------
+ * Implausibility of n input points against n_o observed outputs.  mean, var (S pu, n): block s * pu + j as
+ * ggp_predict_f64 writes them, var clamped at 0.  Over the samples, m_j = (1/S) sum_s mean_sj and
+ * M_jk = (1/S) sum_s [delta_jk var_sj + (mean_sj - m_j)(mean_sk - m_k)].  K_O (pu, n_o), r and c (n_o) in standardized
+ * units, c_i = rho + tau_i^2 + delta_i^2 (truncation residual, observation and discrepancy variances).  Per output
+ *   e_i = r_i - sum_j K_ji m_j,   V_i = sum_jk K_ji M_jk K_ki + c_i,   I_i = |e_i| / sqrt(V_i)
+ * (V_i = 0: +inf for e_i != 0, 0 for e_i = 0; a NaN counts as +inf).  impl_out (n, order) receives each point's `order`
+ * largest I_i in descending order, nover_out (n) the number of outputs with I_i > cutoff.  The two products run on the
+ * FP64 tensor cores; the n x n_o matrices are never stored.  Deterministic (the outputs' split over CTAs does not change
+ * a result).  workspace: ggp_hm_workspace_bytes(n, n_o, pu, S) (-1 for arguments the call refuses).  GGP_ERR_ARG: a null
+ * pointer, S, n or n_o < 1, pu outside [1, 32], order outside [1, min(8, n_o)], a non-finite or non-positive cutoff,
+ * S pu >= 2^31, a short workspace. */
+long long ggp_hm_workspace_bytes(int n, int n_o, int pu, int S);
+int ggp_hm_impl_f64(const double* mean, const double* var, int S, int pu, int n, const double* K_O, const double* r,
+                    const double* c, int n_o, int order, double cutoff, double* impl_out, int* nover_out,
+                    void* workspace, long long workspace_bytes, void* stream);
+
 /* ---- MCMC convergence diagnostics (csrc/ggp_chain_diag.cu; DESIGN.md section 2 "Chain diagnostics") ----------------
  * Rank-normalized split R-hat, bulk ESS and tail ESS of Vehtari et al. (2021), as ArviZ computes rhat(method="rank"),
  * ess(method="bulk") and ess(method="tail"), with the autocovariance as a direct sum.  Draw i of chain c of element e is
