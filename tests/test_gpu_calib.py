@@ -4,9 +4,10 @@ posterior of a two-input problem and a full-field precompute."""
 import numpy as np
 import pytest
 
-from helpers import make_problem, make_scalar_problem, synthetic
+from helpers import synthetic
 from oracle import calib_oracle as co
-from oracle import sepia_oracle as so
+from posterior_helpers import basis, at, calib_obs as _obs, emulator as _oracle, native as _native, \
+    scalar_model as _scalar_model, sepia_model as _model
 
 pytestmark = pytest.mark.gpu
 
@@ -14,63 +15,13 @@ LL_RTOL = 1e-9
 TIE = 1e-6
 
 
-def _model(m=64, q=3, pu=2, seed=5, n_x=20, n_t=10, K=None):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_problem(m=m, q=q, pu=min(pu, 25), n_x=n_x, n_t=n_t, seed=seed)
-    if K is None:
-        K = pr['K']
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'], y_ind_sim=np.arange(pr['y'].shape[1], dtype=float))
-    data.transform_xt(); data.standardize_y(y_mean=pr['mu'], y_sd=pr['sd']); data.create_K_basis(K=K)
-    return SepiaModel(data)
-
-
-def _scalar_model(m=200):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_scalar_problem(m=m)
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'])
-    data.transform_xt(); data.standardize_y()
-    return SepiaModel(data)
-
-
-def _oracle(model, samples):
-    """Oracle emulator on exactly the model's design, PC weights and LamSim."""
-    sd = model.data.sim_data
-    K = None if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
-    num = so.OracleNum(model.num.zt[:, 1:], np.asarray(sd.y_std, dtype=np.float64), K)
-    num.w = model._w_pcs.T.copy()
-    num.wv = num.w.reshape((-1, 1), order='F')
-    num.LamSim = np.asarray(model.num.LamSim, dtype=np.float64)
-    return co.Emulator(num, samples)
-
-
-def _obs(model, O, y_obs, obs_sd, samples):
-    """Oracle G, b, c0 of native observations at outputs O."""
-    sd = model.data.sim_data
-    K = np.ones((1, 1)) if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
-
-    def at(v):
-        v = np.asarray(v, dtype=np.float64).reshape(-1)
-        return np.broadcast_to(v, (O.size,)) if v.size == 1 else v[O]
-    r, tau = co.standardized_obs(y_obs, obs_sd, at(sd.orig_y_mean), at(sd.orig_y_sd))
-    return co.obs_terms(K[:, O], r, tau, np.asarray(samples['lamWOs'], dtype=np.float64).reshape(-1))
-
-
-def _native(model, tt):
-    sd = model.data.sim_data
-    return tt * (sd.orig_t_max - sd.orig_t_min) + sd.orig_t_min
-
-
 def _synthetic_obs(model, em, O, theta_star, obs_sd, seed):
     """y_obs at outputs O: the oracle's posterior-mean prediction at theta_star (transformed) plus N(0, obs_sd^2)."""
     sd = model.data.sim_data
-    K = np.ones((1, 1)) if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
     mu, _ = em.moments(np.asarray(theta_star, dtype=np.float64)[None])
-    ystd = mu[:, :, 0].mean(0) @ K[:, O]
-    ysd = np.broadcast_to(np.asarray(sd.orig_y_sd, dtype=np.float64).reshape(-1), (K.shape[1],))[O]
-    ym = np.broadcast_to(np.asarray(sd.orig_y_mean, dtype=np.float64).reshape(-1), (K.shape[1],))[O]
-    return ystd * ysd + ym + obs_sd * np.random.default_rng(seed).standard_normal(O.size)
+    ystd = mu[:, :, 0].mean(0) @ basis(model)[:, O]
+    return ystd * at(model, sd.orig_y_sd, O) + at(model, sd.orig_y_mean, O) + \
+        obs_sd * np.random.default_rng(seed).standard_normal(O.size)
 
 
 @pytest.mark.parametrize('m,q,pu,S', [(64, 1, 1, 1), (100, 3, 2, 7), (64, 8, 10, 7), (100, 3, 32, 7), (512, 8, 10, 64),

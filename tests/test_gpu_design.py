@@ -4,22 +4,14 @@ blocks, prefixes of a longer design and a one-input model with an empty half."""
 import numpy as np
 import pytest
 
-from helpers import make_problem, make_scalar_problem, synthetic
+from helpers import make_scalar_problem, synthetic
 from oracle import design_oracle as do
+from posterior_helpers import sepia_model as _model
 
 pytestmark = pytest.mark.gpu
 
 SCORE_RTOL = 1e-9
 CANCEL_TOL = 1e-11
-
-
-def _model(m=64, q=3, pu=2, seed=5):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_problem(m=m, q=q, pu=pu, n_x=20, n_t=10, seed=seed)
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'], y_ind_sim=np.arange(pr['y'].shape[1], dtype=float))
-    data.transform_xt(); data.standardize_y(y_mean=pr['mu'], y_sd=pr['sd']); data.create_K_basis(K=pr['K'])
-    return SepiaModel(data)
 
 
 def _scalar_model(t=None, m=200):

@@ -6,6 +6,7 @@ import pytest
 from helpers import synthetic, make_problem, make_scalar_problem, random_hypers
 from oracle import gp_sens_oracle as gso
 from oracle import sobol_oracle as sob
+from posterior_helpers import sepia_model_of
 
 pytestmark = pytest.mark.gpu
 
@@ -44,10 +45,12 @@ def _device(Zin, beta, a, option, grid=None):
 
 
 def _check(Zin, beta, a, option, which=None, grid=np.linspace(0.0, 1.0, 5)):
+    """Returns the largest index error over its tolerance."""
     q = Zin.shape[1]
     M, E0, me = _device(Zin, beta, a, option, grid)
     M, E0, me = M.cpu().numpy(), E0.cpu().numpy(), me.cpu().numpy()
     funcs = gso.block_terms(Zin, beta, a, option)
+    worst = 0.0
     for f in (range(len(funcs)) if which is None else which):
         fa, fb, fz = funcs[f]
         ref = gso.moments(fa, fb, fz)
@@ -59,8 +62,11 @@ def _check(Zin, beta, a, option, which=None, grid=np.linspace(0.0, 1.0, 5)):
         itol = IDX_ATOL + IDX_COND * scale / abs(ref['V'])
         np.testing.assert_allclose(got['first'], ref['first'], rtol=0, atol=itol, err_msg='first f=%d' % f)
         np.testing.assert_allclose(got['total'], ref['total'], rtol=0, atol=itol, err_msg='total f=%d' % f)
+        worst = max(worst, float(np.max(np.abs(got['first'] - ref['first']) / itol)),
+                    float(np.max(np.abs(got['total'] - ref['total']) / itol)))
         np.testing.assert_allclose(me[f], gso.main_effects(fa, fb, fz, grid), rtol=M_RTOL,
                                    atol=M_RTOL * np.sum(np.abs(fa)), err_msg='main effect f=%d' % f)
+    return worst
 
 
 @pytest.mark.parametrize('m,q,pu,S', [(64, 1, 1, 4), (100, 3, 3, 3), (64, 8, 10, 2), (100, 16, 3, 2), (512, 8, 2, 2),
@@ -98,12 +104,7 @@ def test_identical_calls_give_identical_bits(cuda):
 
 
 def _model(m=64, q=3, pu=2, seed=5):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_problem(m=m, q=q, pu=pu, n_x=40, n_t=30, seed=seed)
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'], y_ind_sim=np.arange(pr['y'].shape[1], dtype=float))
-    data.transform_xt(t_notrans=np.arange(q)); data.standardize_y(y_mean=pr['mu'], y_sd=pr['sd']); data.create_K_basis(K=pr['K'])
-    return SepiaModel(data)
+    return sepia_model_of(make_problem(m=m, q=q, pu=pu, n_x=40, n_t=30, seed=seed), t_notrans=True)
 
 
 def test_weights_reproduce_predictive_means(cuda):

@@ -11,76 +11,15 @@ distance to the cutoff exceeds that tolerance."""
 import numpy as np
 import pytest
 
-from helpers import make_problem, make_scalar_problem, synthetic
-from oracle import calib_oracle as co
+from helpers import synthetic
 from oracle import hm_oracle as ho
-from oracle import sepia_oracle as so
+from posterior_helpers import at as _at, emulator as _emulator, hm_obs as _obs_terms, mean_field as _mean_field, \
+    native as _native, scalar_model as _scalar_model, sepia_model as _model
 
 pytestmark = pytest.mark.gpu
 
 IMPL_RTOL = 1e-10
 SCALE_TOL = 1e-12
-
-
-def _model(m=64, q=3, pu=2, seed=5, n_x=20, n_t=10, K=None):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_problem(m=m, q=q, pu=min(pu, 25), n_x=n_x, n_t=n_t, seed=seed)
-    if K is None:
-        K = pr['K']
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'], y_ind_sim=np.arange(pr['y'].shape[1], dtype=float))
-    data.transform_xt(); data.standardize_y(y_mean=pr['mu'], y_sd=pr['sd']); data.create_K_basis(K=K)
-    return SepiaModel(data)
-
-
-def _scalar_model(m=200):
-    from sepia.SepiaData import SepiaData
-    from sepia.SepiaModel import SepiaModel
-    pr = make_scalar_problem(m=m)
-    data = SepiaData(t_sim=pr['t'], y_sim=pr['y'])
-    data.transform_xt(); data.standardize_y()
-    return SepiaModel(data)
-
-
-def _emulator(model, samples):
-    """Oracle emulator on exactly the model's design, PC weights and LamSim."""
-    sd = model.data.sim_data
-    K = None if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
-    num = so.OracleNum(model.num.zt[:, 1:], np.asarray(sd.y_std, dtype=np.float64), K)
-    num.w = model._w_pcs.T.copy()
-    num.wv = num.w.reshape((-1, 1), order='F')
-    num.LamSim = np.asarray(model.num.LamSim, dtype=np.float64)
-    return co.Emulator(num, samples)
-
-
-def _at(model, v, O):
-    n_y = 1 if model.data.scalar_out else np.asarray(model.data.sim_data.K).shape[1]
-    v = np.asarray(v, dtype=np.float64).reshape(-1)
-    return np.broadcast_to(v, (n_y,))[O]
-
-
-def _obs_terms(model, samples, O, y, obs_sd, disc_sd):
-    """K_O, r, c of the oracle for native observations y at outputs O."""
-    sd = model.data.sim_data
-    K = np.ones((1, 1)) if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
-    ysd = _at(model, sd.orig_y_sd, O)
-    r, tau = co.standardized_obs(y, obs_sd, _at(model, sd.orig_y_mean, O), ysd)
-    delta = np.broadcast_to(np.asarray(disc_sd, dtype=np.float64), (O.size,)) / ysd
-    rho = np.mean(1.0 / np.asarray(samples['lamWOs'], dtype=np.float64).reshape(-1))
-    return K[:, O], r, rho + tau ** 2 + delta ** 2
-
-
-def _native(model, tt):
-    sd = model.data.sim_data
-    return tt * (sd.orig_t_max - sd.orig_t_min) + sd.orig_t_min
-
-
-def _mean_field(model, em, O, theta_star):
-    """Native outputs O of the oracle's mixture mean at theta_star (transformed)."""
-    sd = model.data.sim_data
-    K = np.ones((1, 1)) if model.data.scalar_out else np.asarray(sd.K, dtype=np.float64)
-    mu, _ = em.moments(np.asarray(theta_star, dtype=np.float64)[None])
-    return (mu[:, :, 0].mean(0) @ K[:, O]) * _at(model, sd.orig_y_sd, O) + _at(model, sd.orig_y_mean, O)
 
 
 def _check(out, ref, cutoff):
