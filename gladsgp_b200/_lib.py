@@ -72,6 +72,8 @@ SIGNATURES = {
     'ggp_sobol_stats_f64': (_I, [_P, _P, _P, _I, _I, _I, _P, _LL, _I, _I, _I, _P, _P, _P]),
     'ggp_gp_sens_workspace_bytes': (_LL, [_I, _I, _I, _I, _I]),
     'ggp_gp_sens_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _P, _P, _LL, _P]),
+    'ggp_grad_sens_workspace_bytes': (_LL, [_I, _I, _I, _I, _I]),
+    'ggp_grad_sens_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _P, _P, _LL, _P]),
     'ggp_main_effects_f64': (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _P, _I, _P, _P, _LL, _P]),
     'ggp_calib_loglik_f64': (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
     'ggp_calib_step_f64': (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

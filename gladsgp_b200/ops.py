@@ -749,6 +749,44 @@ def main_effects(Z, beta, a, S, pu, grid, mode=0):
     return out
 
 
+def grad_sens(Z, beta, a, S, pu, mode, omega=None):
+    """Gradient outer-product matrices C = E[grad g grad g^T] on [0,1]^q (csrc/ggp_grad_sens.cu) of the functions
+    g = sum over terms of a_n Omega-weighted products of squared-exponential kernels.  Z (m, q), beta (S*pu, q), a (S*pu, m)
+    per block b = s*pu + j, as gp_sens takes them.  mode 0: one function per block; 1: one per PC over every sample's
+    terms; 2: one per sample over every PC's terms, weighted by omega (pu, pu); 3: one function over every block, omega.
+    The weights are used as given (scale by 1/S for the posterior mean).  Returns C (F, q, q), a float64 device tensor."""
+    torch = _lib.require_cuda()
+    Z = _f64(Z, torch, 'cuda')
+    if Z.dim() != 2:
+        raise ValueError('Z must be (m, q)')
+    m, q = Z.shape
+    beta = _f64(beta, torch, 'cuda').reshape(-1)
+    a = _f64(a, torch, 'cuda').reshape(-1)
+    if beta.numel() != S * pu * q or a.numel() != S * pu * m:
+        raise ValueError('beta must hold (S * pu, q) and a (S * pu, m) values')
+    if mode not in (0, 1, 2, 3):
+        raise ValueError('mode must be 0 (per block), 1 (per PC), 2 (per sample) or 3 (one function)')
+    if mode < 2:
+        omega = None
+    else:
+        if omega is None:
+            raise ValueError('modes 2 and 3 need omega (pu, pu)')
+        omega = _f64(omega, torch, 'cuda')
+        if tuple(omega.shape) != (pu, pu):
+            raise ValueError('omega must be (pu, pu) = (%d, %d)' % (pu, pu))
+    nb = _lib.load().ggp_grad_sens_workspace_bytes(m, q, S, pu, mode)
+    if nb < 0:
+        raise ValueError('grad_sens needs m, S, pu >= 1, 1 <= q <= 32 and fewer than 2^31 terms per function '
+                         '(got m=%d, q=%d, S=%d, pu=%d, mode=%d)' % (m, q, S, pu, mode))
+    ws = torch.empty(nb, dtype=torch.uint8, device='cuda')
+    F = (S * pu, pu, S, 1)[mode]
+    out = torch.empty((F, q, q), dtype=torch.float64, device='cuda')
+    check(_lib.load().ggp_grad_sens_f64(ptr(Z), m, q, ptr(beta), ptr(a), S, pu, mode,
+                                        None if omega is None else ptr(omega), ptr(out), ptr(ws), ws.numel(),
+                                        stream_ptr()), 'ggp_grad_sens_f64')
+    return out
+
+
 def calib_loglik(mean, var, G, b, c0, want_per_sample=False):
     """Calibration log-likelihood (csrc/ggp_calib.cu) at n points from the predictive moments mean, var (S*pu, n) of
     ggp_predict_f64 and the observation terms G (S, pu, pu), b (S, pu), c0 (S,).  Returns ll (n,) [, ll_s (S, n)], float64

@@ -16,6 +16,11 @@ predictor: posterior-sample average of the emulator's PC weights at N designs pe
 `gp_sensitivity_indices(model, samples, option, pcvar, ngrid)` computes the indices of that function (and of each
 posterior sample's mean function) exactly instead: the mean is a sum of product squared-exponential kernels, so every
 Sobol' integral over uniform inputs is a closed form in erf and exp (csrc/ggp_gp_sens.cu).
+
+`gp_active_subspace(model, samples, option, target, outputs)` computes the gradient outer-product matrix
+C = E[grad f grad f^T] of the same functions, of a linear combination of the PCs or of the native-unit output field, in
+closed form too (csrc/ggp_grad_sens.cu): its eigenvectors span the active subspace, its diagonal is the derivative-based
+sensitivity (DGSM) of every input.
 """
 from collections import namedtuple
 from dataclasses import dataclass
@@ -24,7 +29,7 @@ import numpy as np
 from scipy import special, stats
 from scipy._lib._util import check_random_state, rng_integers
 
-from . import ops
+from . import _lib, ops
 
 ConfidenceInterval = namedtuple('ConfidenceInterval', ['low', 'high'])
 
@@ -233,4 +238,109 @@ def gp_sensitivity_indices(model, samples, option='samples', pcvar=None, ngrid=2
         sd = model.data.sim_data
         out['main_effect_native'] = (out['main_effect'] * float(np.asarray(sd.orig_y_sd).reshape(-1)[0]) +
                                      float(np.asarray(sd.orig_y_mean).reshape(-1)[0]))
+    return out
+
+
+def _field_omega(model, outputs):
+    """Omega = (K_O diag(sd_O)) (K_O diag(sd_O))^T (pu, pu) over the outputs O, in FP64 on the device (K = [[1]] for a
+    scalar-output model); with every output its diagonal is design.field_weights(model)."""
+    torch = _lib.require_cuda()
+    sd = model.data.sim_data
+    K = np.ones((1, 1)) if model.data.scalar_out else sd.K
+    Kd = torch.as_tensor(np.asarray(K), device='cuda').to(torch.float64)
+    ny = Kd.shape[1]
+    ysd = torch.as_tensor(np.broadcast_to(np.asarray(sd.orig_y_sd, dtype=np.float64).reshape(-1), (ny,)).copy(),
+                          device='cuda')
+    if outputs is not None:
+        O = np.asarray(outputs).reshape(-1)
+        if O.size == 0 or O.dtype.kind not in 'iu' or O.min() < 0 or O.max() >= ny:
+            raise ValueError('outputs must be a non-empty list of output indices in [0, %d)' % ny)
+        O = torch.as_tensor(O.astype(np.int64), device='cuda')
+        Kd, ysd = Kd[:, O], ysd[O]
+    KS = Kd * ysd[None, :]
+    return KS @ KS.T
+
+
+def _input_span(model):
+    """Native range of every input column emulator_expansion keeps (x columns unless x is a dummy, then t): 1 for a
+    column the transform leaves untouched."""
+    sd = model.data.sim_data
+    parts = []
+    if not model.data.dummy_x:
+        parts.append(np.asarray(sd.orig_x_max - sd.orig_x_min, dtype=np.float64).reshape(-1))
+    if model.num.q:
+        parts.append(np.asarray(sd.orig_t_max - sd.orig_t_min, dtype=np.float64).reshape(-1))
+    return np.concatenate(parts)
+
+
+def _eig(C):
+    """Eigen-pairs of symmetric (..., q, q): eigenvalues descending, eigenvectors as columns with their largest-magnitude
+    component positive."""
+    torch = _lib.require_cuda()
+    lam, V = torch.linalg.eigh(torch.as_tensor(C, device='cuda'))
+    lam, V = lam.flip(-1), V.flip(-1)
+    big = torch.gather(V, -2, V.abs().argmax(dim=-2, keepdim=True))
+    V = torch.where(big < 0, -V, V)
+    return lam.cpu().numpy(), V.cpu().numpy()
+
+
+def gp_active_subspace(model, samples, option='samples', target='pc', outputs=None):
+    """Active subspaces and derivative-based sensitivity of the emulator's predictive mean in closed form
+    (csrc/ggp_grad_sens.cu; DESIGN.md section 2 item 12): C = E[grad f grad f^T] with the inputs independent and uniform
+    on [0, 1] in the transformed scale.
+
+    target='pc': f = mu_sj, every PC on its own (C (ns, pu, q, q) for option='samples', (pu, q, q) of the posterior-mean
+    function for 'mean').  target='field': f = the native-unit field over `outputs` (default: every output),
+    E||grad y||^2-type sums through Omega = (K_O diag(sd_O))(K_O diag(sd_O))^T (C (ns, q, q) or (q, q)).  target=c, an
+    array (pu,): the linear quantity sum_j c_j mu_j, Omega = c c^T.
+    Returns a dict of NumPy arrays: C, eigenvalues (descending), eigenvectors (columns, largest-magnitude component
+    positive), dgsm = diag C, dgsm_native = dgsm / span^2 in native input units; for 'samples' also C_avg (the posterior
+    average over samples: the expected active subspace) with eigenvalues_avg, eigenvectors_avg, dgsm_avg; for 'pc' also
+    total_bound = min(1, dgsm / (pi^2 V)), an upper bound on the total Sobol' index (V from ops.gp_sens)."""
+    if option not in ('samples', 'mean'):
+        raise ValueError("option must be 'samples' or 'mean'")
+    pu = model.num.pu
+    omega = None
+    if isinstance(target, str):
+        if target not in ('pc', 'field'):
+            raise ValueError("target must be 'pc', 'field' or an array of pu coefficients")
+        if target == 'pc' and outputs is not None:
+            raise ValueError("outputs applies to target='field' only")
+    else:
+        c = np.asarray(target, dtype=np.float64).reshape(-1)
+        if c.size != pu or not np.all(np.isfinite(c)):
+            raise ValueError('target coefficients must be %d finite values (one per PC)' % pu)
+        if outputs is not None:
+            raise ValueError("outputs applies to target='field' only")
+        omega = np.outer(c, c)
+        target = 'linear'
+    if target == 'field':
+        omega = _field_omega(model, outputs)
+    Z, beta, a, ns = emulator_expansion(model, samples)
+    q = Z.shape[1]
+    if target == 'pc':
+        mode = 0 if option == 'samples' else 1
+    else:
+        mode = 2 if option == 'samples' else 3
+    if mode in (1, 3):
+        a = a / ns
+    C = ops.grad_sens(Z, beta, a, ns, pu, mode, omega)
+    lead = {0: (ns, pu), 1: (pu,), 2: (ns,), 3: ()}[mode]
+    C = C.reshape(lead + (q, q))
+    span = _input_span(model)
+    out = dict(C=C.cpu().numpy())
+    out['eigenvalues'], out['eigenvectors'] = _eig(C)
+    out['dgsm'] = np.diagonal(out['C'], axis1=-2, axis2=-1).copy()
+    out['dgsm_native'] = out['dgsm'] / (span * span)
+    if option == 'samples':
+        Cavg = C.mean(dim=0)
+        out['C_avg'] = Cavg.cpu().numpy()
+        out['eigenvalues_avg'], out['eigenvectors_avg'] = _eig(Cavg)
+        out['dgsm_avg'] = np.diagonal(out['C_avg'], axis1=-2, axis2=-1).copy()
+    if target == 'pc':
+        M, E0 = ops.gp_sens(Z, beta, a, ns, pu, mode)
+        V = (M[:, 2 * q] - E0 * E0).cpu().numpy().reshape(lead)
+        with np.errstate(divide='ignore', invalid='ignore'):
+            bound = out['dgsm'] / (np.pi ** 2 * V[..., None])
+        out['total_bound'] = np.where(out['dgsm'] == 0.0, 0.0, np.minimum(1.0, np.where(V[..., None] > 0, bound, 1.0)))
     return out

@@ -264,6 +264,23 @@ int ggp_main_effects_f64(const double* Z, int m, int q, const double* beta, cons
                          const double* grid, int ngrid, double* out, void* workspace, long long workspace_bytes,
                          void* stream);
 
+/* ---- Closed-form gradient outer products (csrc/ggp_grad_sens.cu; DESIGN.md section 2 item 12) ----------------------
+ * C = E[grad g grad g^T] over independent inputs uniform on [0,1]^q, for g a weighted combination of the functions
+ * mu_b(x) = sum_i a[b][i] prod_k exp(-beta[b][k] (x_k - Z[i][k])^2) of blocks b = s * pu + j (the layout of
+ * ggp_gp_sens_f64): C = sum over pairs of terms (n, n') of a_n a_n' Omega_{j(n) j(n')} int grad phi_n grad phi_n'^T.
+ *   mode 0: one function per block (F = S pu, Omega = 1);   mode 1: one per PC j over every sample's terms (F = pu,
+ *   Omega = 1; scale a by 1/S for the posterior mean);   mode 2: one per sample s over every PC's terms (F = S,
+ *   Omega = omega[pu][pu], symmetric);   mode 3: one function over every (s, j) (F = 1, omega; a scaled by 1/S).
+ * C_out[f][k][l] (F x q x q, exactly symmetric): the active-subspace matrix; its diagonal is the derivative-based
+ * sensitivity E[(d_k g)^2].  An input whose beta is 0 in every term gets row and column k exactly 0.  FP64 libdevice
+ * erf / exp, the off-diagonal pair sums on DMMA m8n8k4; every sum in a fixed order (bit-identical between identical
+ * calls).  workspace_bytes >= ggp_grad_sens_workspace_bytes(m, q, S, pu, mode) (-1 for arguments the call refuses), else
+ * GGP_ERR_WORKSPACE.  GGP_ERR_ARG: a null pointer (omega in modes 2 and 3), m, S or pu < 1, q outside [1, 32], mode
+ * outside 0-3, S pu or a function's term count (m, S m, pu m or S pu m) >= 2^31. */
+long long ggp_grad_sens_workspace_bytes(int m, int q, int S, int pu, int mode);
+int ggp_grad_sens_f64(const double* Z, int m, int q, const double* beta, const double* a, int S, int pu, int mode,
+                      const double* omega, double* C_out, void* workspace, long long workspace_bytes, void* stream);
+
 /* ---- Emulator-based calibration (csrc/ggp_calib.cu; DESIGN.md section 2 item 9) ------------------------------------
  * Log-likelihood of observed outputs at n input points, from the predictive moments of ggp_predict_f64 at the points'
  * designs: mean, var (S pu, n), block s * pu + j (posterior sample s, PC j), var clamped at 0.  Per-sample observation
