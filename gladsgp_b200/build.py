@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libgladsgp_b200.so')
-SOURCES = ['ggp_api.cu', 'ggp_loglik.cu', 'ggp_mcmc.cu', 'ggp_predict.cu', 'ggp_quantile.cu', 'ggp_xval.cu', 'ggp_chain_diag.cu', 'ggp_rsvd_tc.cu', 'ggp_ingest.cu', 'ggp_sobol.cu', 'ggp_gp_sens.cu', 'ggp_calib.cu', 'ggp_design.cu', 'ggp_hm.cu', 'ggp_grad_sens.cu']
+SOURCES = ['ggp_api.cu', 'ggp_loglik.cu', 'ggp_mcmc.cu', 'ggp_predict.cu', 'ggp_quantile.cu', 'ggp_xval.cu', 'ggp_chain_diag.cu', 'ggp_rsvd_tc.cu', 'ggp_ingest.cu', 'ggp_sobol.cu', 'ggp_gp_sens.cu', 'ggp_calib.cu', 'ggp_design.cu', 'ggp_hm.cu', 'ggp_grad_sens.cu', 'ggp_jacobian.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-fmad=false', '-Xcompiler', '-fPIC', '-Xptxas', '-v']
 

@@ -337,6 +337,30 @@ class Predictor:
                                   ptr(self._ws), self._ws.numel(), stream_ptr()), 'ggp_predict_f64')
         return (mean, var, V) if want_V else (mean, var)
 
+    def jacobian(self, Xp, col0, full=True, b0=0, nb=None):
+        """Gradients of the predictive moments at Xp (n,d) with respect to inputs col0 .. d-1 (q = d - col0 in [1, 31]) on
+        blocks [b0, b0+nb) (csrc/ggp_jacobian.cu).  Returns (mean (nb,n,q+1) = [mu, grad mu], cov): with full, cov
+        (nb,n,q+1,q+1) is the joint posterior covariance of [f, grad f]; otherwise (nb,n,2q+1) = [v, Cov(f, d_k f),
+        Var(d_k f)].  mu and v equal predict's bit for bit; nothing is clamped."""
+        torch, lib, dev = self.torch, self.lib, 'cuda'
+        Xp = _f64(Xp, torch, dev)
+        n = Xp.shape[0]
+        nb = self.B - b0 if nb is None else nb
+        q = self.d - int(col0)
+        need = lib.ggp_jacobian_workspace_bytes(self.m, self.d, int(col0), n, nb)
+        if need < 0:
+            raise ValueError('jacobian needs 1 <= q = d - col0 <= 31 differentiated inputs and m <= 8192 (got q=%d, m=%d)'
+                             % (q, self.m))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        mean = torch.empty((nb, n, q + 1), dtype=torch.float64, device=dev)
+        cov = torch.empty((nb, n, q + 1, q + 1) if full else (nb, n, 2 * q + 1), dtype=torch.float64, device=dev)
+        check(lib.ggp_jacobian_f64(ptr(self.X), self.m, self.d, ptr(self.factor[b0:]), ptr(self.u[b0:]),
+                                   ptr(self.beta[b0:]), ptr(self.lamz[b0:]), ptr(self.s11[b0:]), ptr(Xp), n, nb, int(col0),
+                                   1 if full else 0, ptr(mean), ptr(cov), ptr(self._ws), self._ws.numel(), stream_ptr()),
+              'ggp_jacobian_f64')
+        return mean, cov
+
     def pred_cov(self, Xp, V):
         """Joint covariance Sigma (B,n,n) = S11 - V V^T."""
         torch, lib, dev = self.torch, self.lib, 'cuda'

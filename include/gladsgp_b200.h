@@ -281,6 +281,21 @@ long long ggp_grad_sens_workspace_bytes(int m, int q, int S, int pu, int mode);
 int ggp_grad_sens_f64(const double* Z, int m, int q, const double* beta, const double* a, int S, int pu, int mode,
                       const double* omega, double* C_out, void* workspace, long long workspace_bytes, void* stream);
 
+/* ---- Emulator Jacobians (csrc/ggp_jacobian.cu; DESIGN.md section 2 item 13) ---------------------------------------
+ * The inputs of ggp_predict_f64, plus col0: inputs col0 .. d-1 (q = d - col0 of them, 1 <= q <= 31) are differentiated.
+ * Per block b and design t, with g_k = d k(x, Z) / d x_{col0+k-1} and R = L^-1 [k(x, Z); g_1; ...; g_q]:
+ *   mean_out (B, n, q+1) = R u = [mu, d mu / d x_k];
+ *   full = 1: cov_out (B, n, q+1, q+1) = P - R R^T, P = diag(s11[b], 2 beta_bk / lamz_b), exactly symmetric: the joint
+ *             posterior covariance of [f, grad f] (without clamping);
+ *   full = 0: cov_out (B, n, 2q+1) = [v, Cov(f, d_k f) (k = 1..q), Var(d_k f) (k = 1..q)]; d v / d x_k = 2 Cov(f, d_k f).
+ * mu and v equal ggp_predict_f64's bit for bit; an input with beta_bk = 0 gets exact zeros.  Deterministic.
+ * workspace_bytes >= ggp_jacobian_workspace_bytes(m, d, col0, n, B) (-1 for arguments the call refuses), else
+ * GGP_ERR_WORKSPACE.  GGP_ERR_ARG: a null pointer, m, d, n or B < 1, m > 8192, q outside [1, 31], full not 0 or 1. */
+long long ggp_jacobian_workspace_bytes(int m, int d, int col0, int n, int B);
+int ggp_jacobian_f64(const double* X, int m, int d, const double* factor, const double* u, const double* beta,
+                     const double* lamz, const double* s11_diag, const double* Xp, int n, int B, int col0, int full,
+                     double* mean_out, double* cov_out, void* workspace, long long workspace_bytes, void* stream);
+
 /* ---- Emulator-based calibration (csrc/ggp_calib.cu; DESIGN.md section 2 item 9) ------------------------------------
  * Log-likelihood of observed outputs at n input points, from the predictive moments of ggp_predict_f64 at the points'
  * designs: mean, var (S pu, n), block s * pu + j (posterior sample s, PC j), var clamped at 0.  Per-sample observation
